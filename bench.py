@@ -317,6 +317,29 @@ def timed_steps(smp, dist, device, steps, iters, proposals):
     return ms, eik_ms, eik_n, solves_per_launch, smp.profile_kernels()
 
 
+DUMP_LIMIT_BYTES = 60 * 10**6
+
+
+def dump_outputs(smp, stats, out_dir, seed=0):
+    """What the timed steps left for a caller of mq_step, written as out_dir/<name>.npy: the chain states (mq_get_models),
+    the per-chain statistics `stats` = smp.stats() and the tempering betas.  Integers are written as float64; nucleus slots past a
+    chain's dimension are not part of its model and are written as 0.  When all chains would take more than
+    DUMP_LIMIT_BYTES, a seeded sample of chains is written, the same for every run; chain.npy holds their indices."""
+    m = smp.get_models()
+    counts, ll, rms = stats
+    live = np.arange(m.md)[None, :] < m.dim[:, None]
+    out = {"dim": m.dim.astype(np.float64), "z": np.where(live, m.z, np.float32(0)), "vp": np.where(live, m.vp, np.float32(0)),
+           "vpvs": np.where(live, m.vpvs, np.float32(0)), "eq": m.eq, "origin": m.origin, "pres": m.pres, "sres": m.sres,
+           "noise": m.noise, "counts": counts.astype(np.float64), "loglik": ll, "rms": rms, "beta": smp.get_beta()}
+    per_chain = 8 + sum(a.nbytes for a in out.values()) // smp.n
+    keep = min(smp.n, DUMP_LIMIT_BYTES // per_chain)
+    idx = np.arange(smp.n) if keep == smp.n else np.sort(np.random.default_rng(seed).choice(smp.n, keep, replace=False))
+    out["chain"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a if name == "chain" else a[idx])
+
+
 def roofline_block(cfg, smp, ms, eik_ms, eik_n, solves_per_launch, kernels, clk, device, n_rows):
     """Roofline of the dominant kernel (eikonal) from the live CUDA-event time of its launches."""
     nz, nxmod = cfg.grid.nz, smp.nxmod
@@ -546,7 +569,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="headline, roofline, e2e and parity check only (profiling runs)")
     ap.add_argument("--parity-chains", type=int, default=8)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the chain states and statistics they computed as DIR/<name>.npy "
+                         "(rank 0's chains when several GPUs run)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what this library computed: it needs --impl ours")
     W = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     if args.impl == "reference":
@@ -623,6 +651,8 @@ def main():
     launches = mq.lib().mq_launch_count() - launches0
     clk = clocks.stop()
     counts, ll, rms = smp.stats()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(smp, (counts, ll, rms), args.dump_outputs)
     proposals = chains * n_gpus * args.steps * args.iters_per_step
     value = proposals / (ms / 1000.0)
 

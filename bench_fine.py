@@ -88,6 +88,8 @@ def main(args, rank, world, local, dist):
     kernels = smp.profile_kernels()
     clk = clocks.stop()
     counts, ll, rms = smp.stats()
+    if args.dump_outputs and rank == 0:
+        B.dump_outputs(smp, (counts, ll, rms), args.dump_outputs)
     value = chains * n_gpus * args.steps / (ms / 1000.0)
     n_rows = mq.lib().mq_get_rows(smp.h, 0, 1, None, None)
     roofline = B.roofline_block(cfg, smp, ms, eik_ms, eik_n, spl, kernels, clk, device, n_rows) if eik_n else None

@@ -2,15 +2,11 @@
 from __future__ import annotations
 
 import ctypes as C
-import os
 
 import numpy as np
 
 from tests import util
 from tests.util import FmGrid, FmPicks, f32, ptr, ip
-
-REF_ROOT = "/root/reference"
-DATA = os.path.join(util.ROOT, "tests", "data")
 
 
 def fm_grid(cfg) -> FmGrid:
@@ -96,12 +92,3 @@ def fill_models(m, states):
         m.z[c, :d], m.vp[c, :d], m.vpvs[c, :d] = s["z"], s["vp"], s["vpvs"]
         m.eq[c], m.pres[c], m.sres[c], m.noise[c] = s["eq"], s["pres"], s["sres"], s["noise"]
     return m
-
-
-def example_paths(name):
-    """(config, picks) of a shipped example; tests/data holds copies of the two small input files
-    so that the GPU box (no /root/reference) can run them."""
-    d = os.path.join(DATA, name)
-    cfgp = os.path.join(d, "config_eqx.dat")
-    pk = os.path.join(d, "picks_synth" if name == "Example" else "picks.mcmc")
-    return cfgp, pk

@@ -1,6 +1,5 @@
 """Parity of the CUDA eikonal path (through the C ABI) with the oracle and the reference fixtures.
 Tolerance: |dT| <= max(1e-4 s, 2e-6 T) -- FP32 restatement bound, SURVEY.md Appendix A.5."""
-import os
 
 import numpy as np
 import pytest
@@ -12,11 +11,11 @@ pytestmark = pytest.mark.gpu
 
 def test_batch_matches_golden_reference_fields():
     import mcmc_eq_b200 as mq
-    d = np.load(os.path.join(util.GOLDEN, "eikonal_ref.npz"))
+    d, meta = util.golden_eikonal()
     groups = {}
-    for i, m in enumerate(d["meta"]):
+    for i, m in enumerate(meta):
         tref = d[f"t_{i}"]
-        groups.setdefault(tref.shape, []).append((d[f"s_{i}"], int(m.split("|")[2]), tref))
+        groups.setdefault(tref.shape, []).append((d[f"s_{i}"], int(m[2]), tref))
     worst = 0.0
     for (nx, nz), items in groups.items():
         t = mq.eikonal_batch(np.array([s for s, _, _ in items]), [iz for _, iz, _ in items], nx)

@@ -2,7 +2,6 @@
 algorithm the GPU runs, checked against the oracle on CPU.  Tolerance: |dT| <= max(1e-4 s, 2e-6 T)
 (SURVEY.md Appendix A.5).  This is a test of the algorithm, not a product path."""
 import ctypes as C
-import os
 
 import numpy as np
 import pytest
@@ -40,12 +39,12 @@ def _run(emu, s, nx, iz):
 
 
 def test_core_matches_golden(emu):
-    d = np.load(os.path.join(util.GOLDEN, "eikonal_ref.npz"))
+    d, meta = util.golden_eikonal()
     worst = 0.0
     tot = np.zeros(7, np.int64)
-    for i, m in enumerate(d["meta"]):
+    for i, m in enumerate(meta):
         s, tref = d[f"s_{i}"], d[f"t_{i}"]
-        t, rc, cnt = _run(emu, s, tref.shape[0], int(m.split("|")[2]))
+        t, rc, cnt = _run(emu, s, tref.shape[0], int(m[2]))
         assert rc == 0
         err = np.abs(t - tref)
         assert (err <= util.eikonal_tol(tref)).all(), (m, err.max())

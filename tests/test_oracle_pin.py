@@ -11,13 +11,8 @@ from tests import util, inputs
 from tests.util import f32, ptr
 
 
-def _golden_eikonal():
-    d = np.load(os.path.join(util.GOLDEN, "eikonal_ref.npz"))
-    return d, [m.split("|") for m in d["meta"]]
-
-
 def test_eikonal_oracle_matches_golden_bitwise(oracle):
-    d, meta = _golden_eikonal()
+    d, meta = util.golden_eikonal()
     st = util.PlStats()
     for i, (gname, kind, iz) in enumerate(meta):
         s, tref = d[f"s_{i}"], d[f"t_{i}"]

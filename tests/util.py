@@ -90,6 +90,15 @@ def reflib():
     return _ref
 
 
+def golden_eikonal():
+    """time_2d fields of the compiled reference for seeded models (tools/make_golden.py): ({"s_i", "t_i"}, meta), where
+    meta[i] = [grid, kind, source iz].  The fields are stored in two files to keep each under 1 MB."""
+    d = {}
+    for part in (1, 2):
+        d.update(np.load(os.path.join(GOLDEN, f"eikonal_ref_{part}.npz")))
+    return d, [m.split("|") for m in d["meta"]]
+
+
 def f32(a):
     return np.ascontiguousarray(a, dtype=np.float32)
 

@@ -2,7 +2,7 @@
 """Generate tests/golden/* from the UNMODIFIED reference (run in the build container only).
 
   inputs_example{,2}.json/.npz : the two shipped data sets, parsed (configs 1 and 2 of BASELINE.json)
-  eikonal_ref.npz              : time_2d fields of the compiled reference (oracle/_ref) for seeded models
+  eikonal_ref_{1,2}.npz        : time_2d fields of the compiled reference (oracle/_ref) for seeded models
   forward_ref.npz              : cal_fit_newx class sums / origin times of the compiled reference
   chain_ref_example2.out       : a short fixed-seed chain of the reference mcmc_eq binary
   replay_example2.npz          : the proposal stream of that same chain (every proposed model, the uniform deviate of
@@ -100,7 +100,10 @@ def eikonal_fields():
             out[f"s_{len(cases) - 1}"] = s
             out[f"t_{len(cases) - 1}"] = t
     out["meta"] = np.array([f"{a}|{b}|{c}" for a, b, c in cases])
-    np.savez_compressed(os.path.join(G, "eikonal_ref.npz"), **out)
+    # two files of under 1 MB each (tests/util.golden_eikonal): the Example2-grid fields with meta, then the rest
+    first = {k: v for k, v in out.items() if k == "meta" or cases[int(k.split("_")[1])][0] == "ex2"}
+    np.savez_compressed(os.path.join(G, "eikonal_ref_1.npz"), **first)
+    np.savez_compressed(os.path.join(G, "eikonal_ref_2.npz"), **{k: v for k, v in out.items() if k not in first})
     print("eikonal_ref:", len(cases), "fields")
 
 
