@@ -279,7 +279,7 @@ extern "C" int mq_create(const mq_config* cfg, const mq_picks* pk, int n_chains,
             TRY(cudaMalloc(&h->eik_order_work, h->eik_order_bytes));
             TRY(cudaMalloc((void**)&h->eik_order, (((size_t)max_solves + 31) / 32 * 32) * sizeof(int32_t)));
         }
-        if (eik_pipe_supported(h->nxmod, h->nz)) { TRY(dalloc(&h->eik_task_counter, 1)); TRY(dalloc(&h->eik_tie_scratch, eik_pipe_tie_floats())); }
+        if (eik_pipe_supported(h->nxmod, h->nz)) { TRY(dalloc(&h->eik_task_counter, 1)); TRY(dalloc(&h->eik_tie_scratch, eik_pipe_tie_floats(h->nz))); }
     }
     TRY(cudaStreamSynchronize(s));
 #undef TRY

@@ -6,10 +6,12 @@
 // writes 32 bits of TMEM lane (32*(warp%4) + i) at a column address common to the warp.  So the past column, the current
 // column and the slowness column of a marching warp live in tensor memory, node k of a lane at column k+1 of that lane:
 //   * a marching warp needs no shared memory, which goes to the warps that are in their box phase (per-lane indices):
-//     eik_pipe_kernel (eikonal.cu) runs 12 warps per SM on 7 - 9 shared-memory slices + 8 TMEM sets instead of 9 warps;
+//     eik_pipe_kernel (eikonal.cu) runs 12 warps per SM on 7 - 9 shared-memory slices + 8 TMEM sets instead of 9 warps
+//     on the Example plane;
 //   * four consecutive nodes move per instruction (.x4);
 //   * TMEM load latency is 12 cycles against 29 for shared memory.
-// A column array holds the nodes -1 .. CA-2 (CA = 64 for nz <= 62): nodes -1 and ke+1.. carry sentinels larger than any
+// A column array holds the nodes -1 .. CA-2 (CA = 64 for nz <= 62, CA = 128 for 88 <= nz <= 126; eikonal.cu: pipe_shape):
+// nodes -1 and ke+1.. carry sentinels larger than any
 // time (strictly increasing, so they never tie), which end the chains exactly where march_sweep3's kEdge slots do.
 // Arithmetic: chain_a_node / chain_b_node of eik_fast.cuh, unchanged -- results are bit-identical to the fused kernel's.
 #pragma once

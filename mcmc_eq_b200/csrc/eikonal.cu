@@ -264,13 +264,36 @@ cudaError_t eik_order_tasks(const EikBatch& b, int32_t* order, void* work, size_
 // are in the latency-bound box phase and half in the issue-bound march, and there are 12 of them instead of 9 (146 registers each: no spills).
 // Resources are taken in a fixed order (slice, then TMEM set; the tie scratch last and never while waiting for anything
 // else), holders of a TMEM set never wait for a slice: no cycle, no deadlock.
+// Two instantiations, chosen by the depth of the plane (pipe_shape): column arrays of CA = 64 nodes for nz <= 62 (the Example
+// plane), and CA = 128 for 88 <= nz <= 126, which holds the planes of the example grids refined by halving the spacing.  A CA = 128 set is 384
+// columns, so a lane quarter holds one and 4 marches are in flight per SM; slices are 48 - 64 KB at those depths (3 - 4 per
+// SM), so fewer warps per CTA (profiles/README.md, deep planes).
 #ifndef MCMCEQ_PIPE_WARPS
 #define MCMCEQ_PIPE_WARPS 12
 #endif
-constexpr int kPipeWarps = MCMCEQ_PIPE_WARPS;     // measured 10 .. 20: 12 - 13 are best at 1024 chains, 12 - 16 equal at 8192 (profiles/README.md)
-constexpr int kPipeCA = 64;          // nodes -1 .. 62 per TMEM column array: nz <= 62
+#ifndef MCMCEQ_PIPE_WARPS_DEEP
+#define MCMCEQ_PIPE_WARPS_DEEP 8
+#endif
+constexpr int kPipeWarps = MCMCEQ_PIPE_WARPS;     // CA = 64.  Measured 10 .. 20: 12 - 13 are best at 1024 chains, 12 - 16 equal at 8192 (profiles/README.md)
+constexpr int kPipeWarpsDeep = MCMCEQ_PIPE_WARPS_DEEP;   // CA = 128.  Measured 6, 8, 12: 8 is best or level (profiles/README.md)
 constexpr int kPipeMaxCtas = 256;    // one CTA per SM; the tie scratch is sized for this many
-constexpr size_t kPipeTieFloats = (size_t)(3 * kPipeCA + 2) * 32;   // two time columns + slowness column of the tie scratch
+// two time columns + slowness column of the tie scratch of a CTA
+template <int CA>
+constexpr size_t kPipeTieFloats = (size_t)(3 * CA + 2) * 32;
+// The instantiation a plane of nz depth nodes takes (ca = 0: none), its warps per CTA and its default box-phase variant
+// (Dims::lock_cols; MCMCEQ_PIPE_LC overrides it).
+struct PipeShape {
+    int ca, warps, lock_cols;
+};
+// Lowest nz for CA = 128: a shallower plane fills too little of the column arrays, and the fused kernel is faster (B200,
+// 1024 chains: 21.3 against 22.7 ms per launch at nz = 80, 33.4 against 27.5 at nz = 88; DESIGN.md section 3).
+constexpr int kPipeDeepMinNz = 88;
+static PipeShape pipe_shape(int nz)
+{
+    if (nz + 2 <= 64) return {64, kPipeWarps, 1};
+    if (nz >= kPipeDeepMinNz && nz + 2 <= 128) return {128, kPipeWarpsDeep, 1};
+    return {0, 0, 0};
+}
 
 // The box phase of a task.  Until round 2 it had to be compiled as a function of its own: inlined next to the tensor-memory
 // march, nvcc 12.9 produced a kernel whose box-region output was wrong (bisected on the GPU in round 1: any variant with the
@@ -326,16 +349,19 @@ __device__ __forceinline__ void pipe_release(unsigned* mask, int bit, int lane)
     if (lane == 0) { __threadfence_block(); atomicOr(mask, 1u << bit); }
 }
 
-__global__ void __launch_bounds__(kPipeWarps * 32, 1) eik_pipe_kernel(EikBatch b, eikf::Dims D, int n_slices, int* task_counter)
+// CA: nodes -1 .. CA-2 per TMEM column array (nz <= CA - 2); WARPS: warps per CTA
+template <int CA, int WARPS>
+__global__ void __launch_bounds__(WARPS * 32, 1) eik_pipe_kernel(EikBatch b, eikf::Dims D, int n_slices, int* task_counter)
 {
-    constexpr int CA = kPipeCA, NB = CA / 4;
+    constexpr int NB = CA / 4;
+    constexpr int kSets = 512 / (3 * CA);        // TMEM sets per lane quarter: 2 at CA = 64, 1 at CA = 128
     extern __shared__ float smem_p[];
     __shared__ PipeCtl ctl;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, quarter = warp & 3;
     if (warp == 0) eikm::tmem_alloc<512>(&ctl.tmem);
     if (threadIdx.x == 0) {
         ctl.slice_free = (1u << n_slices) - 1u;
-        for (int q = 0; q < 4; q++) ctl.tset_free[q] = 3u;
+        for (int q = 0; q < 4; q++) ctl.tset_free[q] = (1u << kSets) - 1u;
         ctl.tie_lock = 0;
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
@@ -343,7 +369,7 @@ __global__ void __launch_bounds__(kPipeWarps * 32, 1) eik_pipe_kernel(EikBatch b
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const size_t slice_floats = (size_t)eikf::smem_floats_per_lane(D) * 32;
     // scratch of the literal walk for a column with an exact tie (4 in 100 000): global memory, one per CTA, under a lock
-    float* tieP = b.tie_scratch + (size_t)blockIdx.x * kPipeTieFloats + 32 + lane;   // node k at tieP[k*32], k = -1 .. CA-2
+    float* tieP = b.tie_scratch + (size_t)blockIdx.x * kPipeTieFloats<CA> + 32 + lane;   // node k at tieP[k*32], k = -1 .. CA-2
     float* tieC = tieP + (size_t)CA * 32;
     float* tieS = tieC + (size_t)CA * 32 + 32;                             // cell k at tieS[k*32], k = -2 .. CA-1
     const int nz = b.nz, ke = nz - 1, mx = b.nxmod - 1;
@@ -351,7 +377,7 @@ __global__ void __launch_bounds__(kPipeWarps * 32, 1) eik_pipe_kernel(EikBatch b
     const int n_solves = n_items * nz;
     const int n_tasks = (n_solves + 31) >> 5;
     const size_t wfloats = ((size_t)D.wx * D.nz + kFineNodes) * 32;
-    float* Wbase = b.scratch + (size_t)(blockIdx.x * kPipeWarps + warp) * wfloats + lane;
+    float* Wbase = b.scratch + (size_t)(blockIdx.x * WARPS + warp) * wfloats + lane;
 
     for (;;) {
         int task = 0;
@@ -389,8 +415,9 @@ __global__ void __launch_bounds__(kPipeWarps * 32, 1) eik_pipe_kernel(EikBatch b
         if (!__any_sync(0xffffffffu, live)) { pipe_release(&ctl.slice_free, sl, lane); continue; }
         // ---- move the task into a TMEM set of this warp's lane quarter, give the slice back
         const int ts = pipe_acquire(&ctl.tset_free[quarter], lane);
-        // sets 0 and 1 of the quarter: columns [0,192) and [192,384) = past | current | slowness (columns [384,512) stay unused:
-        // a third set with its slowness column in shared memory costs two slices and was slower, profiles/README.md)
+        // set ts of the quarter: columns [3 CA ts, 3 CA (ts + 1)) = past | current | slowness.  Columns [3 CA kSets, 512) stay
+        // unused (at CA = 64: a third set with its slowness column in shared memory costs two slices and was slower,
+        // profiles/README.md)
         const uint32_t tset = ctl.tmem + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(ts * 3 * CA);
         const uint32_t tS = tset + 2 * CA;
         for (int q = 0; q < NB; q++) {
@@ -447,7 +474,17 @@ __global__ void __launch_bounds__(kPipeWarps * 32, 1) eik_pipe_kernel(EikBatch b
                 if (lane == 0) { __threadfence_block(); atomicExch(&ctl.tie_lock, 0); }
             }
             eikm::tmem_st1(tc, eikf::kEdge);
-            for (int k = ke + 1; k <= CA - 2; k++) eikm::tmem_st1(tc + k + 1, eikm::sentinel(k, ke));
+            if (CA == 64) {
+                for (int k = ke + 1; k <= CA - 2; k++) eikm::tmem_st1(tc + k + 1, eikm::sentinel(k, ke));
+            } else {
+                // up to 64 nodes at CA = 128: single stores up to the next group of four columns, .x4 stores from there
+                int k = ke + 1;
+                for (; k <= CA - 2 && ((k + 1) & 3); k++) eikm::tmem_st1(tc + k + 1, eikm::sentinel(k, ke));
+                for (; k <= CA - 2; k += 4) {
+                    const float v[4] = {eikm::sentinel(k, ke), eikm::sentinel(k + 1, ke), eikm::sentinel(k + 2, ke), eikm::sentinel(k + 3, ke)};
+                    eikm::tmem_st4(tc + k + 1, v);
+                }
+            }
             eikm::tmem_wait_st();
             for (int r = 0; r < b.n_rows; r++) {
                 float v = eikm::tmem_ld1(tc + b.rows[r] + 1);
@@ -470,12 +507,15 @@ bool eik_pipe_supported(int nxmod, int nz)
         const char* e = getenv("MCMCEQ_EIKONAL_PIPE");
         enabled = (e && e[0] == '0') ? 0 : 1;     // on unless MCMCEQ_EIKONAL_PIPE=0
     }
-    return enabled && eik_fast_supported(nxmod, nz) && nz + 2 <= kPipeCA;
+    return enabled && eik_fast_supported(nxmod, nz) && pipe_shape(nz).ca > 0;
 }
 
 cudaError_t eik_launch_pipe(const EikBatch& b, int* task_counter, cudaStream_t stream)
 {
     if (b.src_iz || b.full_out || !task_counter || !b.tie_scratch) return cudaErrorInvalidValue;
+    const PipeShape sh = pipe_shape(b.nz);
+    if (!sh.ca) return cudaErrorInvalidValue;
+    void (*const kernel)(EikBatch, eikf::Dims, int, int*) = sh.ca == 64 ? eik_pipe_kernel<64, kPipeWarps> : eik_pipe_kernel<128, kPipeWarpsDeep>;
     eikf::Dims D = fast_dims(b.nxmod, b.nz);
     {
         // Lock-step columns in the box phase (a second column buffer per slice: 7 slices instead of 9 on the Example plane).
@@ -484,7 +524,7 @@ cudaError_t eik_launch_pipe(const EikBatch& b, int* task_counter, cudaStream_t s
         // selects the in-place walk.
         static int lc_env = -2;
         if (lc_env == -2) { const char* e = getenv("MCMCEQ_PIPE_LC"); lc_env = e ? atoi(e) : -1; }
-        D.lock_cols = (lc_env >= 0) ? (lc_env != 0) : 1;
+        D.lock_cols = (lc_env >= 0) ? (lc_env != 0) : sh.lock_cols;
     }
     const size_t slice = fast_smem_floats_per_warp(D) * sizeof(float);
     const size_t tie = 0;      // the tie scratch lives in global memory (b.tie_scratch)
@@ -493,7 +533,7 @@ cudaError_t eik_launch_pipe(const EikBatch& b, int* task_counter, cudaStream_t s
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
     int n_slices = (int)(((size_t)smem_max - tie - 256) / slice);
-    if (n_slices > 12) n_slices = 12;
+    if (n_slices > sh.warps) n_slices = sh.warps;
     {
         static int env_slices = -1;      // experiment: fewer slices than fit (profiles/README.md)
         if (env_slices < 0) { const char* e = getenv("MCMCEQ_PIPE_SLICES"); env_slices = e ? atoi(e) : 0; }
@@ -501,28 +541,33 @@ cudaError_t eik_launch_pipe(const EikBatch& b, int* task_counter, cudaStream_t s
     }
     if (n_slices < 2) return cudaErrorInvalidValue;
     const size_t smem = (size_t)n_slices * slice + tie;
-    static size_t configured[64] = {0};     // per device: largest dynamic shared-memory size the kernel has been opted in for
-    if (dev < 0 || dev >= 64 || smem > configured[dev]) {
-        cudaFuncSetAttribute(eik_pipe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        cudaFuncSetAttribute(eik_pipe_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-        if (dev >= 0 && dev < 64) configured[dev] = smem;
+    // per instantiation and device: largest dynamic shared-memory size the kernel has been opted in for
+    static size_t configured[2][64] = {};
+    size_t* conf = (dev >= 0 && dev < 64) ? &configured[sh.ca == 128][dev] : nullptr;
+    if (!conf || smem > *conf) {
+        cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+        if (conf) *conf = smem;
     }
     const int n_tasks = (b.n_items * b.nz + 31) / 32;
     // per-warp global window: the scratch was sized for max_warps warps of the generic kernel
     const size_t have = (size_t)b.max_warps * eik_scratch_floats_per_warp(b.nxmod, b.nz);
     const long warps_by_scratch = (long)(have / fast_scratch_floats_per_warp(D));
-    int blocks = (n_tasks + kPipeWarps - 1) / kPipeWarps;
+    int blocks = (n_tasks + sh.warps - 1) / sh.warps;
     if (blocks > sms) blocks = sms;
-    if ((long)blocks * kPipeWarps > warps_by_scratch) blocks = (int)(warps_by_scratch / kPipeWarps);
+    if ((long)blocks * sh.warps > warps_by_scratch) blocks = (int)(warps_by_scratch / sh.warps);
     if (blocks < 1) return cudaErrorInvalidValue;
     cudaError_t e = cudaMemsetAsync(task_counter, 0, sizeof(int), stream);
     if (e != cudaSuccess) return e;
-    eik_pipe_kernel<<<blocks, kPipeWarps * 32, smem, stream>>>(b, D, n_slices, task_counter);
+    kernel<<<blocks, sh.warps * 32, smem, stream>>>(b, D, n_slices, task_counter);
     count_launch();
     return cudaGetLastError();
 }
 
-size_t eik_pipe_tie_floats() { return (size_t)kPipeMaxCtas * kPipeTieFloats; }
+size_t eik_pipe_tie_floats(int nz)
+{
+    return (size_t)kPipeMaxCtas * (pipe_shape(nz).ca == 128 ? kPipeTieFloats<128> : kPipeTieFloats<64>);
+}
 
 int eik_fast_max_warps(int nxmod, int nz, int device)
 {
@@ -627,7 +672,8 @@ cudaError_t eik_launch(const EikBatch& b, cudaStream_t stream, int* which)
         int dev = 0, sms = 148;
         cudaGetDevice(&dev);
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        if ((long)(have / fast_scratch_floats_per_warp(D)) >= (long)sms * kPipeWarps && n_tasks >= (long)sms * kPipeWarps &&
+        const int warps = pipe_shape(b.nz).warps;
+        if ((long)(have / fast_scratch_floats_per_warp(D)) >= (long)sms * warps && n_tasks >= (long)sms * warps &&
             sms <= kPipeMaxCtas) {
             EikBatch piped = b;
             *which = kEikPipe;

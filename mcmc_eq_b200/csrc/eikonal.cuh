@@ -27,7 +27,7 @@ struct EikBatch {
     int lanes_per_task;       // fused kernel: solves per warp-task (32, 16, 8 or 4; 0 = chosen by eik_launch_fast: fewer when
                               // the launch has fewer tasks than resident warps, so that a small launch spreads over the SMs)
     int32_t* task_counter;    // [1] device: work counter of the pipelined kernel (eik_launch_pipe), or nullptr
-    float* tie_scratch;       // device, eik_pipe_tie_floats() floats: per-CTA scratch of the pipelined kernel's tie fallback
+    float* tie_scratch;       // device, eik_pipe_tie_floats(nz) floats: per-CTA scratch of the pipelined kernel's tie fallback
     // Outputs (device).  full_out: [n_solves][nxmod*nz] in the reference layout (x*nz+y).
     float* full_out;
     // Receiver-row tables: table of item i starts at row_out[i] (or row_out_base + i*row_item_stride
@@ -59,9 +59,10 @@ cudaError_t eik_launch_fast(const EikBatch& b, cudaStream_t stream);
 // The same warp-synchronous solver with its per-lane arrays in global memory, for planes of any size (the fine grid).
 size_t eik_fine_slice_floats_per_warp(int nxmod, int nz);
 cudaError_t eik_launch_fine(const EikBatch& b, cudaStream_t stream);
-// One persistent CTA per SM, 16 warps: box phases on a pool of shared-memory slices, marches on a pool of TMEM sets.
+// One persistent CTA per SM: box phases on a pool of shared-memory slices, marches on a pool of TMEM sets; planes of up to
+// 126 depth nodes.  eik_pipe_tie_floats(nz): size of EikBatch::tie_scratch for a plane of nz depth nodes.
 bool eik_pipe_supported(int nxmod, int nz);
-size_t eik_pipe_tie_floats();
+size_t eik_pipe_tie_floats(int nz);
 cudaError_t eik_launch_pipe(const EikBatch& b, int* task_counter, cudaStream_t stream);
 // Picks the kernel: pipelined when the launch fills the GPU and the plane fits a shared-memory slice, fused for smaller
 // launches of such planes, generic otherwise (MCMCEQ_EIKONAL=generic forces the generic one).  *which (may be nullptr)
