@@ -307,6 +307,67 @@ int mq_set_beta(mq_handle* h, const float* beta);
 int mq_get_beta(mq_handle* h, float* beta);
 int mq_temper_swap(mq_handle* h, int64_t round, int32_t* n_swapped);
 
+/* ===== checkpoint and resume =================================================================================
+ * Sampler state of every chain of the handle: what mq_step needs to continue each chain exactly where it is -- the
+ * current model, hypocentres, origin times, station corrections, sigmas, per-event class sums, likelihood, counters, the
+ * random-stream position (Philox counter) and LVZ switch of every chain, its best model so far, the posterior
+ * accumulators and temperatures when they are on, the seed and the chain offset.  A handle that loads a state continues
+ * every chain with the same proposals, decisions and records as the handle that saved it, bit for bit.
+ *
+ * mq_state_size: *bytes = the size of a state of this handle as it is now (the posterior and temperatures count only when
+ *   they are on).
+ * mq_state_save: writes the state into buf[0, cap), *bytes (may be NULL) = its size.  It first reports a pending error of
+ *   an earlier asynchronous call.  MQ_ERR_STATE before there is a sampler state (mq_init_chains, or mq_set_models and a
+ *   first mq_step) and while decimated records wait in the ring (records are not state: drain first, so that a resumed run
+ *   never delivers a record twice); MQ_ERR_BUSY while a drain batch is in flight (mq_drain_begin .. mq_batch_release);
+ *   MQ_ERR_ARG when cap is too small.
+ * mq_state_load: replaces the sampler state of the handle -- fresh (no mq_init_chains) or one that has stepped -- by a saved
+ *   one.  The state's seed, chain offset, posterior setting and temperatures replace the handle's; records still in the
+ *   handle's ring are discarded.  A state that does not fit the handle -- other chain count or sizes, a configuration or
+ *   pick set with another checksum (mq_create's inputs), another format version, a bad trailing checksum (truncated or
+ *   damaged) -- is refused with MQ_ERR_ARG before anything on the device changes: the handle stays as it was.  The
+ *   travel-time tables are not in the state; they are rebuilt, and their hashes compared with the saved ones: a table
+ *   that differs (a library whose eikonal results differ) gives MQ_ERR_STATE, mq_last_error() names the first chain and
+ *   phase, and the handle has no usable state until the next mq_state_load / mq_init_chains / mq_set_models.
+ *
+ * Layout (native little-endian): an mq_state_header, n_sections mq_state_section entries, the sections at their offsets
+ * (8-byte aligned, zero padding), and a trailing uint64 checksum of every byte before it.  Checksums are sum64: starting
+ * from h = 0x9E3779B97F4A7C15, for every 64-bit little-endian word w of the data (the last one zero-padded),
+ * h = (h ^ w) * 0x100000001B3 and then h ^= h >> 32.  config_sum is sum64 of the mq_config with the bytes after each
+ * string's NUL zeroed; picks_sum chains sum64 over (n_events, n_picks, n_stations), ev_off, n_p, st_id, x, y, z, t, cls,
+ * (reftime != NULL, fix != NULL) and the arrays reftime and fix when present.  Sections: MQ_STATE_SEC_CHAINS = one record
+ * per chain (layout given by the format version), MQ_STATE_SEC_TABLES = uint64 hash per (chain, phase P/S) of the stored
+ * receiver rows, MQ_STATE_SEC_POSTERIOR = the int32 then (8-byte aligned) double accumulators of mq_posterior_begin,
+ * MQ_STATE_SEC_BETA = float beta per chain. */
+#define MQ_STATE_MAGIC "MQSTATE"
+#define MQ_STATE_FORMAT 1
+#define MQ_STATE_POSTERIOR 1u    /* flags */
+#define MQ_STATE_BETA 2u
+#define MQ_STATE_TABLES 4u       /* table hashes present (no tables exist with eikonal == 0 or aflag == 1) */
+#define MQ_STATE_SEC_CHAINS 1u
+#define MQ_STATE_SEC_TABLES 2u
+#define MQ_STATE_SEC_POSTERIOR 3u
+#define MQ_STATE_SEC_BETA 4u
+typedef struct mq_state_header {
+    char magic[8];             /* MQ_STATE_MAGIC */
+    uint32_t format;           /* MQ_STATE_FORMAT */
+    uint32_t header_bytes;     /* sizeof(mq_state_header) */
+    char version[48];          /* mq_version() of the library that saved it */
+    int32_t n_chains, max_dim, n_events, n_stations, n_picks, nz, nxmod, n_rows;
+    uint64_t seed;
+    int64_t chain_offset;
+    uint32_t flags;            /* MQ_STATE_POSTERIOR | MQ_STATE_BETA | MQ_STATE_TABLES */
+    uint32_t n_sections;
+    float post_dv, post_dvpvs; /* mq_posterior_begin's arguments and the histogram sizes (0 when off) */
+    int32_t post_ndv, post_ndvpvs;
+    int64_t post_burn_in;
+    uint64_t config_sum, picks_sum;
+} mq_state_header;
+typedef struct mq_state_section { uint32_t id, reserved; uint64_t offset, bytes; } mq_state_section;   /* offset from the blob's start */
+int mq_state_size(mq_handle* h, uint64_t* bytes);
+int mq_state_save(mq_handle* h, void* buf, uint64_t cap, uint64_t* bytes);
+int mq_state_load(mq_handle* h, const void* buf, uint64_t bytes);
+
 /* Measurement aid for bench.py: with enable != 0 every eikonal launch is bracketed by CUDA events on
  * the handle's stream.  Returns the time and number of launches accumulated since the previous call
  * (and restarts the accumulation); solves_per_full_launch = 2 * n_chains * nz, the number of solves one

@@ -81,6 +81,23 @@ class MqPosteriorDims(C.Structure):
     _fields_ = [("ndv", C.c_int32), ("ndvpvs", C.c_int32), ("nz", C.c_int32), ("n_events", C.c_int32), ("n_stations", C.c_int32)]
 
 
+class MqStateHeader(C.Structure):
+    """Start of a saved sampler state (include/mcmceq_b200.h: mq_state_header)."""
+    _fields_ = [("magic", C.c_char * 8), ("format", C.c_uint32), ("header_bytes", C.c_uint32), ("version", C.c_char * 48),
+                ("n_chains", C.c_int32), ("max_dim", C.c_int32), ("n_events", C.c_int32), ("n_stations", C.c_int32),
+                ("n_picks", C.c_int32), ("nz", C.c_int32), ("nxmod", C.c_int32), ("n_rows", C.c_int32),
+                ("seed", C.c_uint64), ("chain_offset", C.c_int64), ("flags", C.c_uint32), ("n_sections", C.c_uint32),
+                ("post_dv", C.c_float), ("post_dvpvs", C.c_float), ("post_ndv", C.c_int32), ("post_ndvpvs", C.c_int32),
+                ("post_burn_in", C.c_int64), ("config_sum", C.c_uint64), ("picks_sum", C.c_uint64)]
+
+
+class MqStateSection(C.Structure):
+    _fields_ = [("id", C.c_uint32), ("reserved", C.c_uint32), ("offset", C.c_uint64), ("bytes", C.c_uint64)]
+
+
+STATE_POSTERIOR, STATE_BETA, STATE_TABLES = 1, 2, 4
+
+
 RECORD_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.POINTER(MqRecord))
 
 
@@ -138,6 +155,9 @@ def lib() -> C.CDLL:
         L.mq_sync.argtypes = [C.c_void_p]
         L.mq_timer.argtypes = [C.c_void_p, C.c_int, C.c_int, dp]
         L.mq_profile.argtypes = [C.c_void_p, C.c_int, dp, lp, lp]
+        L.mq_state_size.argtypes = [C.c_void_p, C.POINTER(C.c_uint64)]
+        L.mq_state_save.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
+        L.mq_state_load.argtypes = [C.c_void_p, C.c_char_p, C.c_uint64]
         L.mqio_read_config.argtypes = [C.c_char_p, C.POINTER(MqConfig)]
         L.mqio_read_picks.argtypes = [C.c_char_p, C.POINTER(MqioPicks)]
         L.mqio_free_picks.argtypes = [C.POINTER(MqioPicks)]
@@ -394,6 +414,24 @@ class Sampler:
         k = C.c_int32(0)
         check(lib().mq_temper_swap(self.h, round_, C.byref(k)))
         return k.value
+
+    def save_state(self) -> bytes:
+        """Sampler state of every chain (mq_state_save): what step() needs to continue each chain exactly where it is.
+        Drain the decimated records first."""
+        size = C.c_uint64(0)
+        check(lib().mq_state_size(self.h, C.byref(size)))
+        buf = C.create_string_buffer(size.value)
+        check(lib().mq_state_save(self.h, buf, size.value, C.byref(size)))
+        return buf.raw[:size.value]
+
+    def load_state(self, blob: bytes):
+        """Continue from a state of save_state (mq_state_load); the state's seed, chain offset, posterior and betas
+        replace this sampler's."""
+        blob = bytes(blob)
+        check(lib().mq_state_load(self.h, blob, len(blob)))
+        head = MqStateHeader.from_buffer_copy(blob[:C.sizeof(MqStateHeader)])
+        if head.flags & STATE_POSTERIOR:
+            self._pdims = MqPosteriorDims(head.post_ndv, head.post_ndvpvs, self.nz, self.picks.n_events, self.picks.n_stations)
 
     def sync(self):
         check(lib().mq_sync(self.h))

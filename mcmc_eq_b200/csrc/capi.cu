@@ -137,6 +137,7 @@ extern "C" int mq_create(const mq_config* cfg, const mq_picks* pk, int n_chains,
     h->cfg = *cfg;
     h->device = device;
     h->seed = seed;
+    h->picks_sum = picks_checksum(pk);
     h->n = n_chains;
     h->md = std::min(cfg->max_dim, 1000);   // MD, src/mc.h:49
     h->ne = pk->n_events; h->ns = pk->n_stations; h->np = pk->n_picks;

@@ -80,6 +80,7 @@ struct Handle {
     float xmin, xmax, ymin, ymax, zmin, zmax;
     size_t tab_stride;   // floats per (chain, phase) table
     uint64_t seed;
+    uint64_t picks_sum;  // checksum of the picks as mq_create received them (state.cu: a saved state belongs to them)
     bool models_set, forward_done;
 
     DevPicks pk;
@@ -139,6 +140,10 @@ struct Handle {
     void* comm;
     Posterior post;
 };
+
+// checksums a saved sampler state carries (state.cu)
+uint64_t config_checksum(const mq_config* cfg);
+uint64_t picks_checksum(const mq_picks* pk);
 
 }  // namespace mq
 

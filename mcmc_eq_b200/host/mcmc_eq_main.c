@@ -1,6 +1,7 @@
 /* mcmc_eq_main.c -- the reference's command line on top of the B200 library (plain C host code, C ABI only).
  *
- *     mcmc_eq <config_eqx.dat> <out> <picks> [-n chains] [-d device] [-s seed] [-q]
+ *     mcmc_eq <config_eqx.dat> <out> <picks> [-n chains] [-d device] [-s seed] [-r slots] [-q]
+ *             [-k checkpoint [-K minutes]] [-R checkpoint]
  *
  * The first three arguments are the reference's (src/mcmc_eq.c:332-338; it ignores anything after them).
  * With one chain (the default) <out> is written exactly like the reference writes it: a "sta ST" record, a
@@ -21,6 +22,16 @@
  * (src/mcmc_eq.c:234-248) into the per-chain files.  The reference writes and flushes each record from inside the
  * sampling loop (:1163).
  *
+ * Checkpoints: with -k <file> the run writes a checkpoint at a chunk boundary every -K minutes (default 30; 0 = after
+ * every chunk): every record of the chunks so far is written, the chain files are flushed and fsync'ed, and a header
+ * (chain count, seed, iterations done, records lost so far, the length of every chain file) followed by the sampler state
+ * of mq_state_save goes to <file>.tmp, which is fsync'ed and renamed over <file>: a process killed at any moment leaves
+ * the previous checkpoint intact.  -R <file> resumes: the checkpoint is read and checked before anything else happens,
+ * the handle is created with its chain count and seed and loads its state, each chain file is cut back to its recorded
+ * length and the run goes on from there (no "sta" record is written again).  A run killed after its first checkpoint and
+ * resumed with -R leaves chain files byte-identical to those of the uninterrupted run.  -n must be the checkpoint's (or
+ * absent); -d may differ.
+ *
  * Unlike the reference (which exit(0)s on every error) the exit status is non-zero on failure.
  */
 #include <pthread.h>
@@ -28,6 +39,7 @@
 #include <stdlib.h>
 #include <string.h>
 #include <time.h>
+#include <unistd.h>
 
 #include "../../include/mcmceq_b200.h"
 #include "mq_io.h"
@@ -181,12 +193,107 @@ static void out_name(char* dst, size_t cap, const char* pattern, int n_chains, i
     }
 }
 
+/* ---- checkpoints: CLI header, the length of every chain file, then the mq_state_save blob ------------------------------ */
+#define CKPT_MAGIC "MQCKPT1"
+typedef struct {
+    char magic[8];
+    int32_t n_chains, reserved;
+    uint64_t seed;
+    int64_t iters_done, lost;
+    uint64_t state_bytes;
+} ckpt_head;
+
+typedef struct {
+    ckpt_head head;
+    int64_t* file_len;   /* [n_chains] */
+    unsigned char* state;
+} ckpt_t;
+
+static void ckpt_free(ckpt_t* k) { free(k->file_len); free(k->state); memset(k, 0, sizeof *k); }
+
+/* Reads and checks a checkpoint file; nothing of the library is needed for that.  Returns 0 or 1 (message in err). */
+static int ckpt_read(const char* path, ckpt_t* k, char* err, size_t cap)
+{
+    FILE* f = fopen(path, "rb");
+    long size;
+    size_t n;
+    memset(k, 0, sizeof *k);
+    if (!f) { snprintf(err, cap, "checkpoint %s: cannot open", path); return 1; }
+    if (fseek(f, 0, SEEK_END) != 0 || (size = ftell(f)) < 0 || fseek(f, 0, SEEK_SET) != 0) { fclose(f); snprintf(err, cap, "checkpoint %s: cannot read", path); return 1; }
+    if ((size_t)size < sizeof k->head || fread(&k->head, sizeof k->head, 1, f) != 1 || memcmp(k->head.magic, CKPT_MAGIC, sizeof k->head.magic) != 0) {
+        fclose(f); snprintf(err, cap, "checkpoint %s: not a checkpoint of mcmc_eq", path); return 1;
+    }
+    n = (size_t)(k->head.n_chains > 0 ? k->head.n_chains : 0);
+    if (n < 1 || k->head.iters_done < 0 || k->head.lost < 0 || k->head.state_bytes < sizeof(mq_state_header) ||
+        (uint64_t)size != sizeof k->head + n * sizeof(int64_t) + k->head.state_bytes) {
+        fclose(f); snprintf(err, cap, "checkpoint %s: damaged header or truncated file (%ld bytes)", path, size); return 1;
+    }
+    k->file_len = (int64_t*)malloc(n * sizeof(int64_t));
+    k->state = (unsigned char*)malloc((size_t)k->head.state_bytes);
+    if (!k->file_len || !k->state || fread(k->file_len, sizeof(int64_t), n, f) != n ||
+        fread(k->state, 1, (size_t)k->head.state_bytes, f) != (size_t)k->head.state_bytes) {
+        fclose(f); ckpt_free(k); snprintf(err, cap, "checkpoint %s: cannot read", path); return 1;
+    }
+    fclose(f);
+    if (memcmp(((const mq_state_header*)k->state)->magic, MQ_STATE_MAGIC, 8) != 0) { ckpt_free(k); snprintf(err, cap, "checkpoint %s: no sampler state in it", path); return 1; }
+    return 0;
+}
+
+/* Writes a checkpoint at a chunk boundary; the caller has waited for the writer (writer_idle). */
+static int ckpt_write(const char* path, mq_handle* h, sink_t* sink, uint64_t seed, long iters_done, long lost)
+{
+    char tmp[4200];
+    ckpt_head head;
+    int64_t* len = (int64_t*)calloc((size_t)sink->n_chains, sizeof(int64_t));
+    unsigned char* state = NULL;
+    uint64_t bytes = 0;
+    FILE* f = NULL;
+    int c, ok = 0;
+    if (!len) return 1;
+    for (c = 0; c < sink->n_chains; c++) {
+        if (fflush(sink->out[c]) != 0 || fsync(fileno(sink->out[c])) != 0 || (len[c] = ftell(sink->out[c])) < 0) {
+            fprintf(stderr, "checkpoint: cannot flush chain file %d\n", c + 1); goto out;
+        }
+    }
+    if (mq_state_size(h, &bytes) != MQ_OK || !(state = (unsigned char*)malloc((size_t)bytes)) || mq_state_save(h, state, bytes, &bytes) != MQ_OK) {
+        fprintf(stderr, "checkpoint: mq_state_save failed: %s\n", mq_last_error()); goto out;
+    }
+    memset(&head, 0, sizeof head);
+    memcpy(head.magic, CKPT_MAGIC, sizeof head.magic);
+    head.n_chains = sink->n_chains; head.seed = seed; head.iters_done = iters_done; head.lost = lost; head.state_bytes = bytes;
+    snprintf(tmp, sizeof tmp, "%s.tmp", path);
+    f = fopen(tmp, "wb");
+    if (!f || fwrite(&head, sizeof head, 1, f) != 1 || fwrite(len, sizeof(int64_t), (size_t)sink->n_chains, f) != (size_t)sink->n_chains ||
+        fwrite(state, 1, (size_t)bytes, f) != (size_t)bytes || fflush(f) != 0 || fsync(fileno(f)) != 0) {
+        fprintf(stderr, "checkpoint: cannot write %s\n", tmp); goto out;
+    }
+    if (fclose(f) != 0) { f = NULL; fprintf(stderr, "checkpoint: cannot write %s\n", tmp); goto out; }
+    f = NULL;
+    if (rename(tmp, path) != 0) { fprintf(stderr, "checkpoint: cannot rename %s to %s\n", tmp, path); goto out; }
+    ok = 1;
+out:
+    if (f) fclose(f);
+    free(len); free(state);
+    return ok ? 0 : 1;
+}
+
+static double now_s(void)
+{
+    struct timespec t;
+    clock_gettime(CLOCK_MONOTONIC, &t);
+    return (double)t.tv_sec + 1e-9 * (double)t.tv_nsec;
+}
+
 #define FAIL(...) do { fprintf(stderr, __VA_ARGS__); fprintf(stderr, "\n"); rc = 1; goto done; } while (0)
 #define MQ(call) do { int rc_ = (call); if (rc_ != MQ_OK) FAIL("%s failed (%d): %s", #call, rc_, mq_last_error()); } while (0)
 
 int main(int argc, char** argv)
 {
-    int rc = 0, n_chains = 1, device = 0, quiet = 0, i, c, from_file = 0, ring = 0, writer_on = 0;
+    int rc = 0, n_chains = 1, device = 0, quiet = 0, i, c, from_file = 0, ring = 0, writer_on = 0, n_given = 0;
+    const char *ck_path = NULL, *resume_path = NULL;
+    double ck_minutes = 30.0, ck_last;
+    ckpt_t ck;
+    uint64_t seed_used = 0;
     writer_t wr;
     long seed_arg = -1;
     mq_config cfg;
@@ -202,14 +309,19 @@ int main(int argc, char** argv)
     memset(&pk, 0, sizeof pk);
     memset(&sink, 0, sizeof sink);
     memset(&wr, 0, sizeof wr);
+    memset(&ck, 0, sizeof ck);
     if (argc < 4) {
-        fprintf(stderr, "usage: %s config_eqx.dat outfile picks [-n chains] [-d device] [-s seed] [-r ring slots] [-q]\n", argv[0]);
+        fprintf(stderr, "usage: %s config_eqx.dat outfile picks [-n chains] [-d device] [-s seed] [-r ring slots] [-q] "
+                        "[-k checkpoint [-K minutes]] [-R checkpoint]\n", argv[0]);
         return 2;
     }
-    if ((env = getenv("MCMCEQ_CHAINS")) != NULL) n_chains = atoi(env);
+    if ((env = getenv("MCMCEQ_CHAINS")) != NULL) { n_chains = atoi(env); n_given = 1; }
     if ((env = getenv("MCMCEQ_DEVICE")) != NULL) device = atoi(env);
     for (i = 4; i < argc; i++) {
-        if (!strcmp(argv[i], "-n") && i + 1 < argc) n_chains = atoi(argv[++i]);
+        if (!strcmp(argv[i], "-n") && i + 1 < argc) { n_chains = atoi(argv[++i]); n_given = 1; }
+        else if (!strcmp(argv[i], "-k") && i + 1 < argc) ck_path = argv[++i];
+        else if (!strcmp(argv[i], "-K") && i + 1 < argc) ck_minutes = atof(argv[++i]);
+        else if (!strcmp(argv[i], "-R") && i + 1 < argc) resume_path = argv[++i];
         else if (!strcmp(argv[i], "-d") && i + 1 < argc) device = atoi(argv[++i]);
         else if (!strcmp(argv[i], "-s") && i + 1 < argc) seed_arg = atol(argv[++i]);
         else if (!strcmp(argv[i], "-r") && i + 1 < argc) ring = atoi(argv[++i]);
@@ -217,6 +329,13 @@ int main(int argc, char** argv)
         /* anything else is ignored, as the reference ignores extra arguments */
     }
     if (n_chains < 1) n_chains = 1;
+    if (ck_minutes < 0) ck_minutes = 0;
+    if (resume_path) {   /* checked before anything else: a garbage file fails before a handle exists or a file is touched */
+        char err[4400];
+        if (ckpt_read(resume_path, &ck, err, sizeof err)) FAIL("%s", err);
+        if (n_given && n_chains != ck.head.n_chains) FAIL("-n %d differs from the checkpoint's %d chains", n_chains, ck.head.n_chains);
+        n_chains = ck.head.n_chains;
+    }
 
     if (mqio_read_config(argv[1], &cfg) != MQ_OK) FAIL("%s", mqio_last_error());
     if (mqio_read_picks(argv[3], &pk) != MQ_OK) FAIL("%s", mqio_last_error());
@@ -224,11 +343,14 @@ int main(int argc, char** argv)
     if (cfg.aflag == 3) { from_file = 1; cfg.aflag = 0; }      /* src/mcmc_eq.c:381 */
 
     {
-        unsigned long seed = seed_arg >= 0 ? (unsigned long)seed_arg : (cfg.true_random > 0 ? (unsigned long)cfg.true_random : urandom_seed());
+        unsigned long seed = resume_path ? (unsigned long)ck.head.seed
+                           : seed_arg >= 0 ? (unsigned long)seed_arg : (cfg.true_random > 0 ? (unsigned long)cfg.true_random : urandom_seed());
+        seed_used = (uint64_t)seed;
         if (!quiet) fprintf(stderr, "%d chain(s) on device %d, seed %lu, %d events, %d stations, %d picks\n", n_chains, device, seed,
                             pk.view.n_events, pk.view.n_stations, pk.view.n_picks);
         MQ(mq_create(&cfg, &pk.view, n_chains, device, (uint64_t)seed, &h));
         if (ring > 0) MQ(mq_set_ring(h, ring));
+        if (resume_path) MQ(mq_state_load(h, ck.state, ck.head.state_bytes));
     }
 
     sink.n_chains = n_chains;
@@ -242,8 +364,21 @@ int main(int argc, char** argv)
     for (c = 0; c < n_chains; c++) {
         char name[4096];
         out_name(name, sizeof name, argv[2], n_chains, c + 1);
-        sink.out[c] = fopen(name, "w");
+        sink.out[c] = fopen(name, resume_path ? "r+" : "w");
         if (!sink.out[c]) FAIL("Could not open: %s", name);
+        if (resume_path) {   /* back to the length the checkpoint recorded: what was written after it is written again */
+            long have;
+            if (fseek(sink.out[c], 0, SEEK_END) != 0 || (have = ftell(sink.out[c])) < 0) FAIL("Could not read: %s", name);
+            if ((int64_t)have < ck.file_len[c]) FAIL("%s holds %ld bytes, fewer than the %lld of the checkpoint", name, have, (long long)ck.file_len[c]);
+            if (fflush(sink.out[c]) != 0 || ftruncate(fileno(sink.out[c]), (off_t)ck.file_len[c]) != 0 || fseek(sink.out[c], 0, SEEK_END) != 0)
+                FAIL("Could not truncate: %s", name);
+        }
+    }
+    if (resume_path) {
+        iters_done = (long)ck.head.iters_done;
+        wr.lost = (long)ck.head.lost;
+        if (!quiet) fprintf(stderr, "resumed from %s after %ld iterations\n", resume_path, iters_done);
+        goto main_loop;
     }
 
     /* start models + first forward (src/mcmc_eq.c:559-765) */
@@ -276,6 +411,7 @@ int main(int argc, char** argv)
     }
     MQ(mq_snapshot_all(h, 0, write_record, &sink));
 
+main_loop:
     /* main loop (src/mcmc_eq.c:845-1192): the chain ends after j_max_start + j_max_main ACCEPTED models.  A chain's
      * ring holds `ring` decimated records (at most one per deci iterations), so a chunk of ring/2 * deci iterations
      * between two drains loses nothing even with one drain still in flight. */
@@ -292,6 +428,7 @@ int main(int argc, char** argv)
         pthread_cond_init(&wr.cv, NULL);
         if (pthread_create(&wr.thread, NULL, writer_main, &wr) != 0) FAIL("could not start the writer thread");
         writer_on = 1;
+        ck_last = now_s();
         for (;;) {
             int running = 0;
             mq_batch* b = NULL;
@@ -311,6 +448,16 @@ int main(int argc, char** argv)
                         n_chains, rms[0], 100.0 * a / (a + r > 0 ? a + r : 1));
             }
             if (!running) break;
+            if (ck_path && now_s() - ck_last >= 60.0 * ck_minutes) {
+                long lost;
+                writer_idle(&wr);     /* every record of the chunks so far is in the files and the ring is empty */
+                if (wr.failed) FAIL("writing records failed: %s", mq_last_error());
+                pthread_mutex_lock(&wr.mu);
+                lost = wr.lost;
+                pthread_mutex_unlock(&wr.mu);
+                if (ckpt_write(ck_path, h, &sink, seed_used, iters_done, lost)) FAIL("could not write the checkpoint %s", ck_path);
+                ck_last = now_s();
+            }
         }
     }
 
@@ -334,5 +481,6 @@ done:
     free(sink.out); free(sink.written); free(counts); free(ll); free(rms);
     if (h) mq_destroy(h);
     mqio_free_picks(&pk);
+    ckpt_free(&ck);
     return rc;
 }
