@@ -290,6 +290,41 @@ int mq_posterior_get(mq_handle* h, int32_t* hist_vp, int32_t* hist_vpvs, int32_t
                      double* ressum, double* noisesum, int64_t* n_models);
 int mq_posterior_allreduce(mq_handle* h);
 
+/* Convergence diagnostics on the device: split R-hat and a batch-means effective sample size (ESS) of every quantity the
+ * posterior summarises, from the same used models (decimated, number > burn_in; a model dropped from a full ring counts).
+ * Q = 10 + 2 nz + 4 n_events + 2 n_stations quantities, in this order: 0 rms, 1 dim, 2..9 the sigmas (2*class+phase),
+ * Vp at each depth node, Vp/Vs at each depth node (the values mq_posterior_* bins: nearest nucleus or, with TRIA = 1, the
+ * interpolated profile, clipped to the prior range), x y z t of each event ([event][4]), P and S correction of each
+ * station ([station][2]).  Every chain with any temperature beta counts, as in the posterior.
+ *
+ * Per chain: ref[q] = the chain's first used model; K = n_batches slots (even, 8 .. 64) of sums of d = (double)x - ref and
+ * of d*d (round to nearest, no contraction); a slot holds batch_len models (L, starting at 1).  When the open slot is full
+ * full_batches (k) grows; when k reaches K, slot i = slot 2i + slot 2i+1 (i ascending), slots K/2 .. K-1 are zeroed,
+ * k = K/2 and L doubles.  Memory: (2K + 1) Q doubles + 16 bytes per chain (K = 16, config 3: 280 MB; config 4: 18 GB),
+ * plus 2 Q doubles per chain of work space on the first mq_diag_summary.
+ *
+ * Summary, over the chains with k >= 4 (chains_used): split R-hat from sequences A = batches [0, h) and B = [h, 2h),
+ * h = k/2; n_j = h L, m_j = S_j/n_j, s_j^2 = (T_j - S_j m_j)/(n_j - 1), mu_j = ref + m_j; over the M = 2 chains_used
+ * sequences W = mean s_j^2, Bv = sum (mu_j - mean mu)^2 / (M - 1), var+ = (nbar - 1)/nbar W + Bv, rhat = sqrt(var+/W).
+ * ESS: y_cb = S_cb / L_c over all k_c full batches, sigma2 = sum_c L_c sum_b (y_cb - ybar_c)^2 / sum_c (k_c - 1),
+ * N = sum_c k_c L_c, ess = N var+ / sigma2.  mean = sum_c (k_c L_c ref_c + sum_b S_cb) / N, sd = sqrt(var+).  No used
+ * chain: everything NaN; var+ == 0: rhat and ess NaN; W == 0 < var+: rhat +inf; sigma2 == 0 < var+: ess +inf.
+ *
+ * mq_diag_begin allocates and zeroes the accumulators (again = restart), before or after mq_init_chains; MQ_ERR_ARG for a
+ * negative burn_in or a bad n_batches.  mq_diag_chains copies the raw accumulators out (any pointer may be NULL): ref
+ * [n_chains][Q], sum and sumsq [n_chains][K][Q], batch_len, full_batches, n_models [n_chains].  mq_diag_summary computes the
+ * summary on the device (fixed-order reductions, no floating-point atomics: the same accumulators give the same bits);
+ * mean .. ess are [Q], *n_models = N and *chains_used one each (any may be NULL).  With collective != 0 and a communicator
+ * (mq_comm_init) the sums are all-reduced over the ranks in two rounds and every rank gets the job-wide numbers; without
+ * one, collective is ignored.  It first reports a pending error of an earlier asynchronous call.  Both return MQ_ERR_STATE
+ * before mq_diag_begin.  The accumulators are part of a saved state (MQ_STATE_DIAG). */
+typedef struct mq_diag_dims { int32_t n_quantities, nz, n_events, n_stations, n_batches; } mq_diag_dims;
+int mq_diag_begin(mq_handle* h, int64_t burn_in, int n_batches, mq_diag_dims* dims);
+int mq_diag_chains(mq_handle* h, double* ref, double* sum, double* sumsq, int32_t* batch_len, int32_t* full_batches,
+                   int64_t* n_models);
+int mq_diag_summary(mq_handle* h, int collective, double* mean, double* sd, double* rhat, double* ess, int64_t* n_models,
+                    int32_t* chains_used);
+
 /* NCCL communicator of the job (one rank per handle).  Rank 0 calls mq_comm_unique_id and hands the 128 bytes to the
  * other ranks by whatever means the host has (torch.distributed broadcast, a file, MPI); every rank then calls
  * mq_comm_init.  libnccl is bound at run time; MQ_ERR_UNSUPPORTED when it is absent. */
@@ -310,8 +345,8 @@ int mq_temper_swap(mq_handle* h, int64_t round, int32_t* n_swapped);
 /* ===== checkpoint and resume =================================================================================
  * Sampler state of every chain of the handle: what mq_step needs to continue each chain exactly where it is -- the
  * current model, hypocentres, origin times, station corrections, sigmas, per-event class sums, likelihood, counters, the
- * random-stream position (Philox counter) and LVZ switch of every chain, its best model so far, the posterior
- * accumulators and temperatures when they are on, the seed and the chain offset.  A handle that loads a state continues
+ * random-stream position (Philox counter) and LVZ switch of every chain, its best model so far, the posterior and
+ * diagnostics accumulators and temperatures when they are on, the seed and the chain offset.  A handle that loads a state continues
  * every chain with the same proposals, decisions and records as the handle that saved it, bit for bit.
  *
  * mq_state_size: *bytes = the size of a state of this handle as it is now (the posterior and temperatures count only when
@@ -338,16 +373,22 @@ int mq_temper_swap(mq_handle* h, int64_t round, int32_t* n_swapped);
  * (reftime != NULL, fix != NULL) and the arrays reftime and fix when present.  Sections: MQ_STATE_SEC_CHAINS = one record
  * per chain (layout given by the format version), MQ_STATE_SEC_TABLES = uint64 hash per (chain, phase P/S) of the stored
  * receiver rows, MQ_STATE_SEC_POSTERIOR = the int32 then (8-byte aligned) double accumulators of mq_posterior_begin,
- * MQ_STATE_SEC_BETA = float beta per chain. */
+ * MQ_STATE_SEC_BETA = float beta per chain, MQ_STATE_SEC_DIAG = the diagnostics' own parameters (int64 burn_in, int32
+ * n_batches, int32 n_quantities), then ref, sum, sumsq (double), n_models (int64), batch_len and full_batches (int32) as
+ * mq_diag_chains lays them out.  A state without diagnostics has no such flag or section: its layout does not depend on
+ * whether the library knows them.  Loading replaces the handle's diagnostics, or frees them when the state has none; a
+ * diagnostics section of another quantity count or a bad n_batches is refused with MQ_ERR_ARG. */
 #define MQ_STATE_MAGIC "MQSTATE"
 #define MQ_STATE_FORMAT 1
 #define MQ_STATE_POSTERIOR 1u    /* flags */
 #define MQ_STATE_BETA 2u
 #define MQ_STATE_TABLES 4u       /* table hashes present (no tables exist with eikonal == 0 or aflag == 1) */
+#define MQ_STATE_DIAG 8u         /* diagnostics accumulators present (mq_diag_begin) */
 #define MQ_STATE_SEC_CHAINS 1u
 #define MQ_STATE_SEC_TABLES 2u
 #define MQ_STATE_SEC_POSTERIOR 3u
 #define MQ_STATE_SEC_BETA 4u
+#define MQ_STATE_SEC_DIAG 5u
 typedef struct mq_state_header {
     char magic[8];             /* MQ_STATE_MAGIC */
     uint32_t format;           /* MQ_STATE_FORMAT */
@@ -356,7 +397,7 @@ typedef struct mq_state_header {
     int32_t n_chains, max_dim, n_events, n_stations, n_picks, nz, nxmod, n_rows;
     uint64_t seed;
     int64_t chain_offset;
-    uint32_t flags;            /* MQ_STATE_POSTERIOR | MQ_STATE_BETA | MQ_STATE_TABLES */
+    uint32_t flags;            /* MQ_STATE_POSTERIOR | MQ_STATE_BETA | MQ_STATE_TABLES | MQ_STATE_DIAG */
     uint32_t n_sections;
     float post_dv, post_dvpvs; /* mq_posterior_begin's arguments and the histogram sizes (0 when off) */
     int32_t post_ndv, post_ndvpvs;

@@ -81,6 +81,11 @@ class MqPosteriorDims(C.Structure):
     _fields_ = [("ndv", C.c_int32), ("ndvpvs", C.c_int32), ("nz", C.c_int32), ("n_events", C.c_int32), ("n_stations", C.c_int32)]
 
 
+class MqDiagDims(C.Structure):
+    _fields_ = [("n_quantities", C.c_int32), ("nz", C.c_int32), ("n_events", C.c_int32), ("n_stations", C.c_int32),
+                ("n_batches", C.c_int32)]
+
+
 class MqStateHeader(C.Structure):
     """Start of a saved sampler state (include/mcmceq_b200.h: mq_state_header)."""
     _fields_ = [("magic", C.c_char * 8), ("format", C.c_uint32), ("header_bytes", C.c_uint32), ("version", C.c_char * 48),
@@ -95,7 +100,8 @@ class MqStateSection(C.Structure):
     _fields_ = [("id", C.c_uint32), ("reserved", C.c_uint32), ("offset", C.c_uint64), ("bytes", C.c_uint64)]
 
 
-STATE_POSTERIOR, STATE_BETA, STATE_TABLES = 1, 2, 4
+STATE_POSTERIOR, STATE_BETA, STATE_TABLES, STATE_DIAG = 1, 2, 4, 8
+STATE_SEC_DIAG = 5
 
 
 RECORD_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.POINTER(MqRecord))
@@ -125,6 +131,9 @@ def lib() -> C.CDLL:
         L.mq_posterior_begin.argtypes = [C.c_void_p, C.c_float, C.c_float, C.c_int64, C.POINTER(MqPosteriorDims)]
         L.mq_posterior_get.argtypes = [C.c_void_p, ip, ip, ip, dp, dp, dp, dp, lp]
         L.mq_posterior_allreduce.argtypes = [C.c_void_p]
+        L.mq_diag_begin.argtypes = [C.c_void_p, C.c_int64, C.c_int, C.POINTER(MqDiagDims)]
+        L.mq_diag_chains.argtypes = [C.c_void_p, dp, dp, dp, ip, ip, lp]
+        L.mq_diag_summary.argtypes = [C.c_void_p, C.c_int, dp, dp, dp, dp, lp, ip]
         L.mq_comm_unique_id.argtypes = [u8p]
         L.mq_comm_init.argtypes = [C.c_void_p, u8p, C.c_int, C.c_int]
         L.mq_comm_destroy.argtypes = [C.c_void_p]
@@ -393,6 +402,35 @@ class Sampler:
     def posterior_allreduce(self):
         check(lib().mq_posterior_allreduce(self.h))
 
+    # ---- convergence diagnostics (mq_diag_*, mcmc_eq_b200/diag.py) ------------------------------------------------
+    def diag_begin(self, burn_in: int = 0, n_batches: int = 16) -> MqDiagDims:
+        """Split R-hat and ESS of every posterior quantity from the decimated models with number > burn_in."""
+        d = MqDiagDims()
+        check(lib().mq_diag_begin(self.h, burn_in, n_batches, C.byref(d)))
+        self._ddims = (d.n_quantities, d.n_batches)
+        return d
+
+    def diag_chains(self) -> dict:
+        """Raw per-chain accumulators: ref [n, Q], sum / sumsq [n, K, Q], batch_len, full_batches, n_models [n]."""
+        Q, K = self._ddims
+        out = dict(ref=np.zeros((self.n, Q)), sum=np.zeros((self.n, K, Q)), sumsq=np.zeros((self.n, K, Q)),
+                   batch_len=np.zeros(self.n, np.int32), full_batches=np.zeros(self.n, np.int32), n_models=np.zeros(self.n, np.int64))
+        check(lib().mq_diag_chains(self.h, _p(out["ref"], dp), _p(out["sum"], dp), _p(out["sumsq"], dp), _p(out["batch_len"], ip),
+                                   _p(out["full_batches"], ip), _p(out["n_models"], lp)))
+        return out
+
+    def diag_summary(self, collective: bool = False) -> dict:
+        """mean, sd, rhat, ess [Q], n_models (N), chains_used and the quantity names (diag.quantity_names)."""
+        from .diag import quantity_names
+        Q, _K = self._ddims
+        out = {k: np.zeros(Q) for k in ("mean", "sd", "rhat", "ess")}
+        n, used = C.c_int64(0), C.c_int32(0)
+        check(lib().mq_diag_summary(self.h, int(collective), _p(out["mean"], dp), _p(out["sd"], dp), _p(out["rhat"], dp),
+                                    _p(out["ess"], dp), C.byref(n), C.byref(used)))
+        out["n_models"], out["chains_used"] = n.value, used.value
+        out["names"] = quantity_names(self.nz, self.picks.n_events, self.picks.n_stations)
+        return out
+
     def comm_init(self, unique_id: bytes, rank: int, world: int):
         buf = (C.c_uint8 * 128).from_buffer_copy(unique_id)
         check(lib().mq_comm_init(self.h, buf, rank, world))
@@ -432,6 +470,12 @@ class Sampler:
         head = MqStateHeader.from_buffer_copy(blob[:C.sizeof(MqStateHeader)])
         if head.flags & STATE_POSTERIOR:
             self._pdims = MqPosteriorDims(head.post_ndv, head.post_ndvpvs, self.nz, self.picks.n_events, self.picks.n_stations)
+        if head.flags & STATE_DIAG:   # the section starts with int64 burn_in, int32 n_batches, int32 n_quantities
+            for k in range(head.n_sections):
+                sec = MqStateSection.from_buffer_copy(blob, C.sizeof(MqStateHeader) + k * C.sizeof(MqStateSection))
+                if sec.id == STATE_SEC_DIAG:
+                    K, Q = np.frombuffer(blob, np.int32, 2, sec.offset + 8)
+                    self._ddims = (int(Q), int(K))
 
     def sync(self):
         check(lib().mq_sync(self.h))

@@ -94,6 +94,7 @@ extern "C" int mq_destroy(mq_handle* hh)
     cudaSetDevice(h->device);
     if (h->stream) cudaStreamSynchronize(h->stream);
     comm_destroy(h);
+    diag_destroy(h);
     sampler_destroy(h);
     profile_destroy(h);
     cudaFree(h->pk.ev_off); cudaFree(h->pk.n_p); cudaFree(h->pk.st_id); cudaFree(h->pk.r0); cudaFree(h->pk.cp);

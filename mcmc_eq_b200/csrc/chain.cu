@@ -678,6 +678,34 @@ __global__ void __launch_bounds__(128) pack_records_kernel(int n, Ring R, float*
     if (threadIdx.x == 0) *(volatile int32_t*)&R.rd[c] = w;
 }
 
+// Vp and Vp/Vs of a model at depth node i as analyse_eq bins them (src/analyse_eq.c:564-606): the nearest nucleus, or with
+// TRIA = 1 the interpolated profile (:573-580,593-598), clipped to the prior range.  *nearest: the nucleus taken (-1 with
+// TRIA = 1).  The posterior and the diagnostics both rasterise through here.
+__device__ void node_velocity(const mq_config& g, const float* z, const float* vp, const float* vpvs, int dim, int i, float* vv_out,
+                              float* rr_out, int* nearest)
+{
+    const float zz = __fadd_rn(__fmul_rn((float)i, g.grid.h), g.grid.z0);
+    float vv, rr;
+    if (g.tria == 1) {
+        int lo, hi;
+        tria::segment_of_node(z, dim, i, g.grid.h, g.grid.z0, &lo, &hi);
+        vv = tria::line_through(zz, z[lo], vp[lo], z[hi], vp[hi]);
+        rr = tria::line_through(zz, z[lo], vpvs[lo], z[hi], vpvs[hi]);
+        *nearest = -1;
+    } else {
+        const int k = find_in_cell_dev(z, dim, zz);
+        vv = vp[k];
+        rr = vpvs[k];
+        *nearest = k;
+    }
+    if (vv > g.vpmax) vv = g.vpmax;
+    if (vv < g.vpmin) vv = g.vpmin;
+    if (rr > g.vpvsmax) rr = g.vpvsmax;
+    if (rr < g.vpvsmin) rr = g.vpvsmin;
+    *vv_out = vv;
+    *rr_out = rr;
+}
+
 // analyse_eq pass 1 for one decimated model (src/analyse_eq.c:564-640): per depth node the velocity of the nearest
 // nucleus, clipped to the prior range, goes into the Vp and Vp/Vs histograms; hypocentres, origin times, station
 // corrections and sigmas into running sums.
@@ -697,27 +725,16 @@ __device__ void posterior_accumulate(const SamplerParams& p, const Handle& hd, i
     double* noisesum = ressum + 4 * (size_t)p.ns;
     const mq_config& g = p.cfg;
     for (int i = threadIdx.x; i < p.nz; i += blockDim.x) {
-        const float zz = __fadd_rn(__fmul_rn((float)i, g.grid.h), g.grid.z0);
         float vv, rr;
-        if (g.tria == 1) {   // interpolated profile, no layer boundaries (src/analyse_eq.c:573-580,593-598)
-            int lo, hi;
-            tria::segment_of_node(z, dim, i, g.grid.h, g.grid.z0, &lo, &hi);
-            vv = tria::line_through(zz, z[lo], vp[lo], z[hi], vp[hi]);
-            rr = tria::line_through(zz, z[lo], vpvs[lo], z[hi], vpvs[hi]);
-        } else {
-            const int k = find_in_cell_dev(z, dim, zz);
-            vv = vp[k];
-            rr = vpvs[k];
-            const float vvx = vp[find_in_cell_dev(z, dim, __fsub_rn(zz, g.grid.h))];
-            if (vv != vvx) atomicAdd(&boundary[i], 1);
+        int k;
+        node_velocity(g, z, vp, vpvs, dim, i, &vv, &rr, &k);
+        if (k >= 0) {   // a layer boundary at node i: the nucleus above is another one (no boundaries with TRIA = 1)
+            const float zz = __fadd_rn(__fmul_rn((float)i, g.grid.h), g.grid.z0);
+            if (vp[k] != vp[find_in_cell_dev(z, dim, __fsub_rn(zz, g.grid.h))]) atomicAdd(&boundary[i], 1);
         }
-        if (vv > g.vpmax) vv = g.vpmax;
-        if (vv < g.vpmin) vv = g.vpmin;
         int j = (int)__fdiv_rn(__fsub_rn(vv, g.vpmin), P.dv);
         if (j > P.ndv - 1) j = P.ndv - 1;
         atomicAdd(&hist_vp[(size_t)j * p.nz + i], 1);
-        if (rr > g.vpvsmax) rr = g.vpvsmax;
-        if (rr < g.vpvsmin) rr = g.vpvsmin;
         j = (int)__fdiv_rn(__fsub_rn(rr, g.vpvsmin), P.dvpvs);
         if (j > P.ndvpvs - 1) j = P.ndvpvs - 1;
         atomicAdd(&hist_vs[(size_t)j * p.nz + i], 1);
@@ -741,12 +758,71 @@ __device__ void posterior_accumulate(const SamplerParams& p, const Handle& hd, i
     if (threadIdx.x == 0) atomicAdd(&noisesum[16], 1.0);
 }
 
+// Convergence diagnostics for one used model (DESIGN.md section 4d): quantity q of the record (q = 0 rms, 1 dim, 2..9 the
+// sigmas, then Vp and Vp/Vs per depth node, x y z t per event, P and S correction per station) goes into the chain's open
+// batch slot as d = x - ref.  Threads over quantities; each (chain, quantity) is summed in the same order whatever the
+// stepping, so the accumulators are a function of the chain's records alone.
+__device__ void diag_accumulate(const SamplerParams& p, const Handle& hd, const Ring& R, int c)
+{
+    const Diag& D = hd.diag;
+    const int n = p.n, mc = hd.mcur[c], ec = hd.ecur[c];
+    const int dim = hd.dim[mc * n + c];
+    const size_t mo = ((size_t)mc * n + c) * p.md;
+    const float* z = hd.z + mo; const float* vp = hd.vp + mo; const float* vpvs = hd.vpvs + mo;
+    const int Q = D.Q, K = D.K, nz = p.nz, ne = p.ne;
+    const int64_t m = D.n_models[c];
+    const int k = D.full_batches[c], L = D.batch_len[c];
+    const bool fills = m + 1 - (int64_t)k * L == L;          // this model fills the open slot
+    double* ref = D.ref + (size_t)c * Q;
+    double* S = D.sum + (size_t)c * K * Q;
+    double* T = D.sumsq + (size_t)c * K * Q;
+    for (int q = threadIdx.x; q < Q; q += blockDim.x) {
+        double x;
+        if (q == 0) x = R.rms[c];
+        else if (q == 1) x = (double)dim;
+        else if (q < 10) x = (double)hd.noise[8 * (size_t)c + q - 2];
+        else if (q < 10 + 2 * nz) {
+            const int i = (q - 10) % nz;
+            float vv, rr;
+            int near;
+            node_velocity(p.cfg, z, vp, vpvs, dim, i, &vv, &rr, &near);
+            x = (double)(q < 10 + nz ? vv : rr);
+        } else if (q < 10 + 2 * nz + 4 * ne) {
+            const int e = (q - 10 - 2 * nz) >> 2, j = (q - 10 - 2 * nz) & 3;
+            x = (double)(j < 3 ? hd.eq[((size_t)c * ne + e) * 3 + j] : hd.origin[((size_t)ec * n + c) * ne + e]);
+        } else {
+            const int st = (q - 10 - 2 * nz - 4 * ne) >> 1;
+            x = (double)((q & 1) == 0 ? hd.pres[(size_t)c * p.ns + st] : hd.sres[(size_t)c * p.ns + st]);
+        }
+        if (m == 0) ref[q] = x;
+        const double d = __dsub_rn(x, ref[q]);
+        S[(size_t)k * Q + q] = __dadd_rn(S[(size_t)k * Q + q], d);
+        T[(size_t)k * Q + q] = __dadd_rn(T[(size_t)k * Q + q], __dmul_rn(d, d));
+        if (fills && k + 1 == K) {   // every slot full: pairs merge, slots K/2 .. K-1 are empty again
+            for (int i = 0; i < K / 2; i++) {
+                S[(size_t)i * Q + q] = __dadd_rn(S[(size_t)(2 * i) * Q + q], S[(size_t)(2 * i + 1) * Q + q]);
+                T[(size_t)i * Q + q] = __dadd_rn(T[(size_t)(2 * i) * Q + q], T[(size_t)(2 * i + 1) * Q + q]);
+            }
+            for (int i = K / 2; i < K; i++) { S[(size_t)i * Q + q] = 0.0; T[(size_t)i * Q + q] = 0.0; }
+        }
+    }
+    __syncthreads();   // every thread has read m, k and L
+    if (threadIdx.x == 0) {
+        D.n_models[c] = m + 1;
+        if (fills) {
+            if (k + 1 == K) { D.full_batches[c] = K / 2; D.batch_len[c] = 2 * L; }
+            else D.full_batches[c] = k + 1;
+        }
+    }
+}
+
 __global__ void snapshot_kernel(SamplerParams p, Handle hd, SamplerDev s)
 {
     const int c = blockIdx.x;
     const int pend = s.ring.pend[c];
     if (pend) {
         if (hd.post.on && (long long)s.ring.number[c] > hd.post.burn_in) posterior_accumulate(p, hd, c);
+        if (hd.diag.on && (long long)s.ring.number[c] > hd.diag.burn_in) diag_accumulate(p, hd, s.ring, c);
         if (pend == 1) {
             const int wr = s.ring.wr[c];
             record_write(p, hd, s.ring, c, s.ring.data + ((size_t)c * s.ring.slots + wr % s.ring.slots) * s.ring.rec_floats);

@@ -309,6 +309,14 @@ extern "C" int mq_temper_swap(mq_handle* hh, int64_t round, int32_t* n_swapped)
 }
 
 namespace mq {
+int comm_allreduce_sum(Handle* h, double* buf, size_t count)
+{
+    Comm* c = (Comm*)h->comm;
+    if (!c || c->world < 2) return MQ_OK;
+    MQ_NCCL(nccl()->AllReduce(buf, buf, count, ncclFloat64, ncclSum, c->comm, h->stream));
+    return MQ_OK;
+}
+
 void comm_destroy(Handle* h)
 {
     mq_handle* hh = reinterpret_cast<mq_handle*>(h);   // Handle is the first and only member of mq_handle

@@ -218,18 +218,29 @@ namespace {
 struct Plan {   // sizes and places of everything in a blob of this handle
     mq_state_header head;
     int n_sections;
-    mq_state_section sec[4];
+    mq_state_section sec[5];
     size_t payload_off, payload_bytes, total_bytes;
     size_t rec_bytes;
-    size_t chains_off, hash_off, post_off, post_int_bytes, beta_off;   // offsets inside the payload (= the staging buffer)
+    size_t chains_off, hash_off, post_off, post_int_bytes, beta_off, diag_off;   // offsets inside the payload (= the staging buffer)
 };
+
+// The diagnostics section: DiagHead, then ref [n][Q], sum [n][K][Q], sumsq [n][K][Q] (double), n_models [n] (int64),
+// batch_len [n], full_batches [n] (int32).
+struct DiagHead {
+    int64_t burn_in;
+    int32_t n_batches, n_quantities;
+};
+inline size_t diag_section_bytes(size_t n, size_t K, size_t Q)
+{
+    return sizeof(DiagHead) + (n * Q * (2 * K + 1)) * sizeof(double) + n * (sizeof(int64_t) + 2 * sizeof(int32_t));
+}
 
 inline size_t up8(size_t x) { return (x + 7) / 8 * 8; }
 
 bool has_tables(const Handle* h) { return h->cfg.eikonal == 1 && h->cfg.aflag != 1; }
 
 // the sections of a blob with the given options; the header's identity fields from the handle
-void make_plan(const Handle* h, bool post, bool beta, bool tables, Plan* P)
+void make_plan(const Handle* h, bool post, bool beta, bool tables, bool diag, Plan* P)
 {
     memset(P, 0, sizeof *P);
     mq_state_header& H = P->head;
@@ -241,7 +252,7 @@ void make_plan(const Handle* h, bool post, bool beta, bool tables, Plan* P)
     H.nz = h->nz; H.nxmod = h->nxmod; H.n_rows = h->n_rows;
     H.config_sum = config_checksum(&h->cfg);
     H.picks_sum = h->picks_sum;
-    H.flags = (post ? MQ_STATE_POSTERIOR : 0) | (beta ? MQ_STATE_BETA : 0) | (tables ? MQ_STATE_TABLES : 0);
+    H.flags = (post ? MQ_STATE_POSTERIOR : 0) | (beta ? MQ_STATE_BETA : 0) | (tables ? MQ_STATE_TABLES : 0) | (diag ? MQ_STATE_DIAG : 0);
     const size_t n = h->n;
     P->rec_bytes = chain_bytes(h->md, h->ne, h->ns);
     size_t off = 0;
@@ -260,6 +271,7 @@ void make_plan(const Handle* h, bool post, bool beta, bool tables, Plan* P)
         P->post_off = add(MQ_STATE_SEC_POSTERIOR, P->post_int_bytes + Q.n_dbl * sizeof(double));
     }
     if (beta) P->beta_off = add(MQ_STATE_SEC_BETA, n * sizeof(float));
+    if (diag) P->diag_off = add(MQ_STATE_SEC_DIAG, diag_section_bytes(n, h->diag.K, h->diag.Q));
     H.n_sections = P->n_sections;
     P->payload_off = sizeof(mq_state_header) + P->n_sections * sizeof(mq_state_section);
     P->payload_bytes = off;
@@ -270,7 +282,7 @@ void make_plan(const Handle* h, bool post, bool beta, bool tables, Plan* P)
 
 void plan_of_handle(const Handle* h, Plan* P)
 {
-    make_plan(h, h->post.on != 0, h->beta != nullptr, has_tables(h), P);
+    make_plan(h, h->post.on != 0, h->beta != nullptr, has_tables(h), h->diag.on != 0, P);
     mq_state_header& H = P->head;
     H.seed = h->seed;
     H.chain_offset = h->chain_offset;
@@ -365,6 +377,20 @@ extern "C" int mq_state_save(mq_handle* hh, void* buf, uint64_t cap, uint64_t* b
         MQ_CUDA(cudaMemcpyAsync(d + P.post_off + P.post_int_bytes, h->post.dblock, h->post.n_dbl * sizeof(double), cudaMemcpyDeviceToDevice, st));
     }
     if (P.head.flags & MQ_STATE_BETA) MQ_CUDA(cudaMemcpyAsync(d + P.beta_off, h->beta, n * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    if (P.head.flags & MQ_STATE_DIAG) {
+        const Diag& D = h->diag;
+        const DiagHead dh = {(int64_t)D.burn_in, D.K, D.Q};
+        const size_t nq = n * D.Q, nkq = nq * D.K;
+        char* o = d + P.diag_off;
+        MQ_CUDA(cudaMemcpyAsync(o, &dh, sizeof dh, cudaMemcpyHostToDevice, st)); o += sizeof dh;
+        MQ_CUDA(cudaMemcpyAsync(o, D.ref, nq * sizeof(double), cudaMemcpyDeviceToDevice, st)); o += nq * sizeof(double);
+        MQ_CUDA(cudaMemcpyAsync(o, D.sum, nkq * sizeof(double), cudaMemcpyDeviceToDevice, st)); o += nkq * sizeof(double);
+        MQ_CUDA(cudaMemcpyAsync(o, D.sumsq, nkq * sizeof(double), cudaMemcpyDeviceToDevice, st)); o += nkq * sizeof(double);
+        MQ_CUDA(cudaMemcpyAsync(o, D.n_models, n * sizeof(int64_t), cudaMemcpyDeviceToDevice, st)); o += n * sizeof(int64_t);
+        MQ_CUDA(cudaMemcpyAsync(o, D.batch_len, n * sizeof(int32_t), cudaMemcpyDeviceToDevice, st)); o += n * sizeof(int32_t);
+        MQ_CUDA(cudaMemcpyAsync(o, D.full_batches, n * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
+        MQ_CUDA(cudaStreamSynchronize(st));   // dh is on this stack frame
+    }
     char* out = (char*)buf;
     memcpy(out, &P.head, sizeof P.head);
     memcpy(out + sizeof P.head, P.sec, P.n_sections * sizeof(mq_state_section));
@@ -404,7 +430,8 @@ extern "C" int mq_state_load(mq_handle* hh, const void* buf, uint64_t bytes)
     if (H.config_sum != config_checksum(&h->cfg)) { set_error("mq_state_load: the state was saved with another configuration"); return MQ_ERR_ARG; }
     if (H.picks_sum != h->picks_sum) { set_error("mq_state_load: the state was saved with other picks"); return MQ_ERR_ARG; }
     const bool post = (H.flags & MQ_STATE_POSTERIOR) != 0, beta = (H.flags & MQ_STATE_BETA) != 0, tables = (H.flags & MQ_STATE_TABLES) != 0;
-    if ((H.flags & ~(uint32_t)(MQ_STATE_POSTERIOR | MQ_STATE_BETA | MQ_STATE_TABLES)) || tables != has_tables(h)) {
+    const bool diag = (H.flags & MQ_STATE_DIAG) != 0;
+    if ((H.flags & ~(uint32_t)(MQ_STATE_POSTERIOR | MQ_STATE_BETA | MQ_STATE_TABLES | MQ_STATE_DIAG)) || tables != has_tables(h)) {
         set_error("mq_state_load: flags 0x%x do not fit the handle", H.flags);
         return MQ_ERR_ARG;
     }
@@ -415,12 +442,34 @@ extern "C" int mq_state_load(mq_handle* hh, const void* buf, uint64_t bytes)
         posterior_sizes(h, H.post_dv, H.post_dvpvs, &ndv, &ndvpvs, &n_int, &n_dbl);
         if (ndv != H.post_ndv || ndvpvs != H.post_ndvpvs) { set_error("mq_state_load: posterior histogram sizes do not fit"); return MQ_ERR_ARG; }
     }
+    // the diagnostics section starts with its own parameters: they must fit the handle
+    DiagHead dh = {0, 0, 0};
+    if (diag) {
+        const mq_state_section* sec = nullptr;
+        if (H.n_sections <= 5 && sizeof H + H.n_sections * sizeof(mq_state_section) <= bytes)
+            for (uint32_t k = 0; k < H.n_sections; k++) {
+                const mq_state_section* e = (const mq_state_section*)(in + sizeof H + k * sizeof(mq_state_section));
+                if (e->id == MQ_STATE_SEC_DIAG) sec = e;
+            }
+        if (!sec || sec->bytes < sizeof dh || sec->offset > bytes - sizeof(uint64_t) || sec->bytes > bytes - sizeof(uint64_t) - sec->offset) {
+            set_error("mq_state_load: flags 0x%x without a diagnostics section", H.flags);
+            return MQ_ERR_ARG;
+        }
+        memcpy(&dh, in + sec->offset, sizeof dh);
+        if (dh.burn_in < 0 || dh.n_batches < 8 || dh.n_batches > 64 || (dh.n_batches & 1) ||
+            dh.n_quantities != diag_quantities(h->nz, h->ne, h->ns)) {
+            set_error("mq_state_load: diagnostics of %d quantities x %d batches (burn-in %lld) do not fit the handle (%d quantities)",
+                      dh.n_quantities, dh.n_batches, (long long)dh.burn_in, diag_quantities(h->nz, h->ne, h->ns));
+            return MQ_ERR_ARG;
+        }
+    }
     // the layout these options give must be the blob's, section by section
     Plan P;
     {
-        Handle tmp = *h;                  // sizes of the posterior block as the state has it
+        Handle tmp = *h;                  // sizes of the posterior and diagnostics blocks as the state has them
         tmp.post.n_int = n_int; tmp.post.n_dbl = n_dbl;
-        make_plan(&tmp, post, beta, tables, &P);
+        tmp.diag.K = dh.n_batches; tmp.diag.Q = dh.n_quantities;
+        make_plan(&tmp, post, beta, tables, diag, &P);
     }
     if (bytes != P.total_bytes || H.n_sections != (uint32_t)P.n_sections ||
         memcmp(in + sizeof H, P.sec, P.n_sections * sizeof(mq_state_section)) != 0) {
@@ -467,6 +516,25 @@ extern "C" int mq_state_load(mq_handle* hh, const void* buf, uint64_t bytes)
         cudaStreamSynchronize(st);
         cudaFree(h->beta);
         h->beta = nullptr;
+    }
+    if (diag) {
+        Diag& D = h->diag;
+        if (!D.on || D.K != dh.n_batches) {
+            MQ_CUDA(cudaStreamSynchronize(st));
+            rc = diag_alloc(h, dh.n_batches, dh.burn_in);
+            if (rc != MQ_OK) return rc;
+        }
+        D.burn_in = dh.burn_in;
+        const size_t nq = n * D.Q, nkq = nq * D.K;
+        const char* o = d + P.diag_off + sizeof dh;
+        MQ_CUDA(cudaMemcpyAsync(D.ref, o, nq * sizeof(double), cudaMemcpyDeviceToDevice, st)); o += nq * sizeof(double);
+        MQ_CUDA(cudaMemcpyAsync(D.sum, o, nkq * sizeof(double), cudaMemcpyDeviceToDevice, st)); o += nkq * sizeof(double);
+        MQ_CUDA(cudaMemcpyAsync(D.sumsq, o, nkq * sizeof(double), cudaMemcpyDeviceToDevice, st)); o += nkq * sizeof(double);
+        MQ_CUDA(cudaMemcpyAsync(D.n_models, o, n * sizeof(int64_t), cudaMemcpyDeviceToDevice, st)); o += n * sizeof(int64_t);
+        MQ_CUDA(cudaMemcpyAsync(D.batch_len, o, n * sizeof(int32_t), cudaMemcpyDeviceToDevice, st)); o += n * sizeof(int32_t);
+        MQ_CUDA(cudaMemcpyAsync(D.full_batches, o, n * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
+    } else if (h->diag.on) {
+        diag_destroy(h);
     }
     h->seed = H.seed;
     h->chain_offset = H.chain_offset;

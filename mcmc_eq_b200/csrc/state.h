@@ -67,6 +67,23 @@ struct Posterior {
     size_t n_int, n_dbl;
 };
 
+// On-device convergence diagnostics (diag.cu, DESIGN.md section 4d): per chain and posterior quantity, batch sums of
+// d = x - ref over the same decimated models the posterior takes, in K slots whose length doubles when they are full.
+// Memory: (2K + 1) Q doubles + 16 bytes per chain, Q = 10 + 2 nz + 4 ne + 2 ns quantities.
+struct Diag {
+    int on;
+    int K, Q;               // batch slots (n_batches), quantities
+    long long burn_in;      // models with number <= burn_in are skipped, as in the posterior
+    double* ref;            // [n][Q] the chain's first used model
+    double* sum;            // [n][K][Q] sums of d per batch slot
+    double* sumsq;          // [n][K][Q] sums of d*d
+    int64_t* n_models;      // [n] used models so far
+    int32_t* batch_len;     // [n] models per full batch (L)
+    int32_t* full_batches;  // [n] full batches (k); slot k is the open one
+    double* scratch;        // summary work space (diag.cu), allocated on the first mq_diag_summary
+    size_t scratch_bytes;
+};
+
 struct Handle {
     mq_config cfg;
     int device;
@@ -139,11 +156,19 @@ struct Handle {
     float* beta;         // [n] or nullptr (all 1)
     void* comm;
     Posterior post;
+    Diag diag;
 };
 
 // checksums a saved sampler state carries (state.cu)
 uint64_t config_checksum(const mq_config* cfg);
 uint64_t picks_checksum(const mq_picks* pk);
+
+// diagnostics (diag.cu): number of quantities of a handle; allocate (zeroed) / free the accumulators
+inline int diag_quantities(int nz, int ne, int ns) { return 10 + 2 * nz + 4 * ne + 2 * ns; }
+int diag_alloc(Handle* h, int K, long long burn_in);
+void diag_destroy(Handle* h);
+// comm.cu: in-place sum of `count` doubles over the ranks of the handle's communicator; nothing without one
+int comm_allreduce_sum(Handle* h, double* buf, size_t count);
 
 }  // namespace mq
 

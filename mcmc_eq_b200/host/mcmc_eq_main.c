@@ -1,7 +1,7 @@
 /* mcmc_eq_main.c -- the reference's command line on top of the B200 library (plain C host code, C ABI only).
  *
  *     mcmc_eq <config_eqx.dat> <out> <picks> [-n chains] [-d device] [-s seed] [-r slots] [-q]
- *             [-k checkpoint [-K minutes]] [-R checkpoint]
+ *             [-k checkpoint [-K minutes]] [-R checkpoint] [-D diagnostics]
  *
  * The first three arguments are the reference's (src/mcmc_eq.c:332-338; it ignores anything after them).
  * With one chain (the default) <out> is written exactly like the reference writes it: a "sta ST" record, a
@@ -32,8 +32,16 @@
  * resumed with -R leaves chain files byte-identical to those of the uninterrupted run.  -n must be the checkpoint's (or
  * absent); -d may differ.
  *
+ * Diagnostics: -D <file> computes split R-hat and the effective sample size of every posterior quantity on the device
+ * (mq_diag_*) from the decimated models after the start phase (burn-in = j_max_start, 16 batch slots), and writes <file>
+ * at every checkpoint and at the end of the run: a "#" header line (chains used, burn-in, batches, iterations done), then
+ * one line per quantity "name index n_models mean sd rhat ess" (names rms dim noise vp vpvs x y z t pres sres), plus one
+ * stderr line with the largest R-hat and the smallest ESS and where they occur.  The accumulators are part of the
+ * checkpoint: under -R they continue, and -D with a checkpoint that has none fails before any chain file is touched.
+ *
  * Unlike the reference (which exit(0)s on every error) the exit status is non-zero on failure.
  */
+#include <math.h>
 #include <pthread.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -277,6 +285,83 @@ out:
     return ok ? 0 : 1;
 }
 
+/* ---- diagnostics: the parameters a saved state holds, the report file --------------------------------------------------- */
+static int state_diag_params(const unsigned char* state, uint64_t bytes, int64_t* burn_in, int32_t* n_batches)
+{
+    const mq_state_header* H = (const mq_state_header*)state;
+    uint32_t k;
+    if (!(H->flags & MQ_STATE_DIAG) || bytes < sizeof *H + H->n_sections * sizeof(mq_state_section)) return 1;
+    for (k = 0; k < H->n_sections; k++) {
+        mq_state_section sec;
+        memcpy(&sec, state + sizeof *H + k * sizeof sec, sizeof sec);
+        if (sec.id == MQ_STATE_SEC_DIAG && sec.bytes >= 16 && sec.offset + 16 <= bytes) {
+            memcpy(burn_in, state + sec.offset, sizeof *burn_in);
+            memcpy(n_batches, state + sec.offset + 8, sizeof *n_batches);
+            return 0;
+        }
+    }
+    return 1;
+}
+
+/* name and index of quantity q (include/mcmceq_b200.h, mq_diag_*) */
+static const char* diag_name(int q, int nz, int ne, int* index)
+{
+    static const char* ev[4] = {"x", "y", "z", "t"};
+    *index = 0;
+    if (q == 0) return "rms";
+    if (q == 1) return "dim";
+    if (q < 10) { *index = q - 2; return "noise"; }
+    q -= 10;
+    if (q < 2 * nz) { *index = q % nz; return q < nz ? "vp" : "vpvs"; }
+    q -= 2 * nz;
+    if (q < 4 * ne) { *index = q / 4; return ev[q % 4]; }
+    q -= 4 * ne;
+    *index = q / 2;
+    return q % 2 ? "sres" : "pres";
+}
+
+static int diag_write(const char* path, mq_handle* h, int nz, int ne, int ns, int64_t burn_in, int n_batches, long iters_done)
+{
+    const int Q = 10 + 2 * nz + 4 * ne + 2 * ns;
+    double* v = (double*)malloc(4 * (size_t)Q * sizeof(double));
+    double *mean = v, *sd = v + Q, *rhat = v + 2 * Q, *ess = v + 3 * Q;
+    int64_t n_models = 0;
+    int32_t used = 0;
+    int q, qr = -1, qe = -1, ir, ie, ok = 0;
+    char tmp[4200];
+    FILE* f = NULL;
+    if (!v) return 1;
+    if (mq_diag_summary(h, 0, mean, sd, rhat, ess, &n_models, &used) != MQ_OK) {
+        fprintf(stderr, "diagnostics: mq_diag_summary failed: %s\n", mq_last_error()); goto out;
+    }
+    snprintf(tmp, sizeof tmp, "%s.tmp", path);
+    if (!(f = fopen(tmp, "w"))) { fprintf(stderr, "diagnostics: cannot write %s\n", tmp); goto out; }
+    fprintf(f, "# chains_used %d burn_in %lld batches %d iterations %ld\n", used, (long long)burn_in, n_batches, iters_done);
+    for (q = 0; q < Q; q++) {
+        int idx;
+        const char* name = diag_name(q, nz, ne, &idx);
+        fprintf(f, "%-5s %5d %12lld %.9e %.9e %.6f %.1f\n", name, idx, (long long)n_models, mean[q], sd[q], rhat[q], ess[q]);
+        if (!isnan(rhat[q]) && (qr < 0 || rhat[q] > rhat[qr])) qr = q;
+        if (!isnan(ess[q]) && (qe < 0 || ess[q] < ess[qe])) qe = q;
+    }
+    if (fclose(f) != 0) { f = NULL; fprintf(stderr, "diagnostics: cannot write %s\n", tmp); goto out; }
+    f = NULL;
+    if (rename(tmp, path) != 0) { fprintf(stderr, "diagnostics: cannot rename %s to %s\n", tmp, path); goto out; }
+    if (qr >= 0 && qe >= 0) {
+        const char* nr = diag_name(qr, nz, ne, &ir);
+        const char* ne_ = diag_name(qe, nz, ne, &ie);
+        fprintf(stderr, "diagnostics after %ld iterations (%d chains used): max R-hat %.4f (%s %d), min ESS %.1f (%s %d)\n", iters_done,
+                used, rhat[qr], nr, ir, ess[qe], ne_, ie);
+    } else {
+        fprintf(stderr, "diagnostics after %ld iterations (%d chains used): no R-hat yet\n", iters_done, used);
+    }
+    ok = 1;
+out:
+    if (f) fclose(f);
+    free(v);
+    return ok ? 0 : 1;
+}
+
 static double now_s(void)
 {
     struct timespec t;
@@ -290,7 +375,9 @@ static double now_s(void)
 int main(int argc, char** argv)
 {
     int rc = 0, n_chains = 1, device = 0, quiet = 0, i, c, from_file = 0, ring = 0, writer_on = 0, n_given = 0;
-    const char *ck_path = NULL, *resume_path = NULL;
+    const char *ck_path = NULL, *resume_path = NULL, *diag_path = NULL;
+    int64_t diag_burn_in = 0;
+    int32_t diag_batches = 16;
     double ck_minutes = 30.0, ck_last;
     ckpt_t ck;
     uint64_t seed_used = 0;
@@ -312,7 +399,7 @@ int main(int argc, char** argv)
     memset(&ck, 0, sizeof ck);
     if (argc < 4) {
         fprintf(stderr, "usage: %s config_eqx.dat outfile picks [-n chains] [-d device] [-s seed] [-r ring slots] [-q] "
-                        "[-k checkpoint [-K minutes]] [-R checkpoint]\n", argv[0]);
+                        "[-k checkpoint [-K minutes]] [-R checkpoint] [-D diagnostics]\n", argv[0]);
         return 2;
     }
     if ((env = getenv("MCMCEQ_CHAINS")) != NULL) { n_chains = atoi(env); n_given = 1; }
@@ -322,6 +409,7 @@ int main(int argc, char** argv)
         else if (!strcmp(argv[i], "-k") && i + 1 < argc) ck_path = argv[++i];
         else if (!strcmp(argv[i], "-K") && i + 1 < argc) ck_minutes = atof(argv[++i]);
         else if (!strcmp(argv[i], "-R") && i + 1 < argc) resume_path = argv[++i];
+        else if (!strcmp(argv[i], "-D") && i + 1 < argc) diag_path = argv[++i];
         else if (!strcmp(argv[i], "-d") && i + 1 < argc) device = atoi(argv[++i]);
         else if (!strcmp(argv[i], "-s") && i + 1 < argc) seed_arg = atol(argv[++i]);
         else if (!strcmp(argv[i], "-r") && i + 1 < argc) ring = atoi(argv[++i]);
@@ -335,6 +423,8 @@ int main(int argc, char** argv)
         if (ckpt_read(resume_path, &ck, err, sizeof err)) FAIL("%s", err);
         if (n_given && n_chains != ck.head.n_chains) FAIL("-n %d differs from the checkpoint's %d chains", n_chains, ck.head.n_chains);
         n_chains = ck.head.n_chains;
+        if (diag_path && state_diag_params(ck.state, ck.head.state_bytes, &diag_burn_in, &diag_batches))
+            FAIL("-D: the checkpoint %s holds no diagnostics (the run was started without -D)", resume_path);
     }
 
     if (mqio_read_config(argv[1], &cfg) != MQ_OK) FAIL("%s", mqio_last_error());
@@ -351,6 +441,10 @@ int main(int argc, char** argv)
         MQ(mq_create(&cfg, &pk.view, n_chains, device, (uint64_t)seed, &h));
         if (ring > 0) MQ(mq_set_ring(h, ring));
         if (resume_path) MQ(mq_state_load(h, ck.state, ck.head.state_bytes));
+        else if (diag_path) {   /* the models of the start phase are burn-in */
+            diag_burn_in = cfg.j_max_start;
+            MQ(mq_diag_begin(h, diag_burn_in, diag_batches, NULL));
+        }
     }
 
     sink.n_chains = n_chains;
@@ -456,6 +550,8 @@ main_loop:
                 lost = wr.lost;
                 pthread_mutex_unlock(&wr.mu);
                 if (ckpt_write(ck_path, h, &sink, seed_used, iters_done, lost)) FAIL("could not write the checkpoint %s", ck_path);
+                if (diag_path && diag_write(diag_path, h, cfg.grid.nz, pk.view.n_events, pk.view.n_stations, diag_burn_in, diag_batches, iters_done))
+                    FAIL("could not write the diagnostics %s", diag_path);
                 ck_last = now_s();
             }
         }
@@ -466,6 +562,8 @@ main_loop:
     if (wr.lost) fprintf(stderr, "warning: %ld decimated record(s) were dropped because a chain's ring was full (-r)\n", wr.lost);
     MQ(mq_snapshot_all(h, 1, write_record, &sink));
     for (c = 0; c < n_chains; c++) mqio_write_counts(sink.out[c], counts + 20 * c);
+    if (diag_path && diag_write(diag_path, h, cfg.grid.nz, pk.view.n_events, pk.view.n_stations, diag_burn_in, diag_batches, iters_done))
+        FAIL("could not write the diagnostics %s", diag_path);
 
 done:
     if (writer_on) {
