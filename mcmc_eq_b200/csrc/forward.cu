@@ -502,7 +502,10 @@ cudaError_t launch_misfit(Handle* h, const EvalView& v)
     MisfitParams p;
     p.n = h->n; p.ne = h->ne; p.ns = h->ns; p.np = h->np; p.nz = h->nz; p.nxmod = h->nxmod; p.xp = h->xp; p.md = h->md;
     p.hgrid = h->cfg.grid.h; p.z0 = h->cfg.grid.z0; p.rh = 1.0f / p.hgrid;
-    { int ex = 0; p.h_pow2 = (p.hgrid > 0.f && frexpf(p.hgrid, &ex) == 0.5f) ? 1 : 0; }
+    // MCMCEQ_MISFIT_POW2=0: the general instantiation for every spacing (checks that the power-of-two one is bit-identical)
+    static int allow_pow2 = -1;
+    if (allow_pow2 < 0) { const char* e = getenv("MCMCEQ_MISFIT_POW2"); allow_pow2 = (e && e[0] == '0') ? 0 : 1; }
+    { int ex = 0; p.h_pow2 = (allow_pow2 && p.hgrid > 0.f && frexpf(p.hgrid, &ex) == 0.5f) ? 1 : 0; }
     p.eikonal = h->cfg.eikonal; p.scor_flag = h->cfg.scor_flag;
     p.tab_stride = h->tab_stride; p.pk = h->pk; p.v = v; p.dim = h->dim; p.z = h->z; p.vp = h->vp; p.vpvs = h->vpvs;
     p.eq = h->eq; p.pres = h->pres; p.sres = h->sres; p.tab = h->tab; p.evsum = h->evsum; p.origin = h->origin;
