@@ -92,6 +92,17 @@ struct FineMedium {
 
 // Time field of one lane: node (x,y) lives at t[(x*ny + y)*ts]; ts = 32 interleaves the
 // lanes of a warp so that lanes working on the same node touch one 128-byte line.
+// View: what a sweep reads of a grid, handed to it by value.  Through a reference the struct
+// would live in the caller's frame, and since a store to a node may alias it, every node
+// access would re-read t, ny, ts and the medium from local memory.
+template <class Medium>
+struct View {
+    float* t;
+    int ts, ny;
+    Medium S;
+    EIK_HD float& T(int x, int y) const { return t[((size_t)x * ny + y) * ts]; }
+};
+
 template <class Medium>
 struct Grid {
     float* t;
@@ -100,10 +111,11 @@ struct Grid {
     Medium S;
     int ys;               // source node (0, ys)
     int X1, Y0, Y1;       // timed box, inclusive; X0 == 0 always
-    int side_limit;
     int status;
     Counters* cnt;
     EIK_HD float& T(int x, int y) const { return t[((size_t)x * ny + y) * ts]; }
+    EIK_HD View<Medium> view() const { return View<Medium>{t, ts, ny, S}; }
+    EIK_HD void note(int st) { if (st != kOk) status = st; }
 };
 
 #define EIK_CNT(g, f) do { if ((g).cnt) (g).cnt->f++; } while (0)
@@ -244,46 +256,62 @@ EIK_HD int walk_line(const G& g, int line, int future, int kb, int ke, int* long
 }
 
 // A side of the box plus, when a head wave ran along it, the reverse propagation of
-// src/time_2d.c:1128-1143 / 1355-1369, unrolled into an explicit stack.
-template <int AXIS, class G>
-EIK_HD_NOINLINE void sweep_line(G& g, int line, int future, int kb, int ke)
+// src/time_2d.c:1128-1143 / 1355-1369, unrolled into an explicit stack.  Recursively:
+//     side(line, F): walk the line; if a head wave called for it,
+//                    for l = line - F, line - 2F, ... (not side_limit, inside the grid): stop once side(l, -F) updates nothing
+// `across`: the last line of this axis (mx for columns, my for rows).  Returns kOk or kErrReverseDepth.
+// The stack holds one int per frame, in registers: frame f walks lines in the direction -F_f, where F_0 = future and
+// F_{f+1} = -F_f (a frame is opened by a sweep of its parent's lines, whose future is -F_f), so only the frame's current
+// line has to be kept; it lives in a shift register (lines[0] is the top), which unrolls to fixed indices, where an array
+// indexed by the stack pointer would live in local memory.  Every frame is opened by a sweep that updated nodes (a head
+// wave is an update), so a closed frame always tells its parent to go on.
+template <int AXIS, class Medium>
+EIK_HD_NOINLINE int sweep_line(const View<Medium> g, int across, int line, int future, int kb, int ke, Counters* cnt)
 {
-    const int across = (AXIS == 0) ? g.mx : g.my;
-    int fL[kMaxReverseDepth], fF[kMaxReverseDepth], fl[kMaxReverseDepth], fU[kMaxReverseDepth];
-    int sp = 0, ret = 0;
-    bool have_ret = false;
+    int lines[kMaxReverseDepth];
+#pragma unroll
+    for (int i = 0; i < kMaxReverseDepth; i++) lines[i] = 0;
+    int sp = 0, status = kOk;
+    const int side_limit = line + future;
     int curL = line, curF = future;
-    g.side_limit = line + future;
     for (;;) {
         int lh = 0;
         const int upd = walk_line<AXIS>(g, curL, curF, kb, ke, &lh);
-        if (g.cnt) {
-            if (AXIS == 0) g.cnt->col_sweeps++; else g.cnt->row_sweeps++;
-            if (sp) g.cnt->reverse_sweeps++;
-            g.cnt->headwaves += lh;
+        if (cnt) {
+            if (AXIS == 0) cnt->col_sweeps++; else cnt->row_sweeps++;
+            if (sp) cnt->reverse_sweeps++;
+            cnt->headwaves += lh;
         }
-        if (lh && sp == kMaxReverseDepth) { g.status = kErrReverseDepth; lh = 0; }
+        if (lh && sp == kMaxReverseDepth) { status = kErrReverseDepth; lh = 0; }
+        bool advance;   // move the top frame on to its next line (else: check the line it was just opened at)
         if (lh) {
-            fL[sp] = curL; fF[sp] = curF; fl[sp] = curL - curF; fU[sp] = upd;
+#pragma unroll
+            for (int i = kMaxReverseDepth - 1; i > 0; i--) lines[i] = lines[i - 1];
+            lines[0] = curL - curF;
             sp++;
+            advance = false;
         } else {
-            ret = upd;
-            have_ret = true;
+            if (sp == 0) return status;
+            advance = true;
+            if (upd == 0) {              // the re-timed line changed nothing: the frame is closed
+#pragma unroll
+                for (int i = 0; i < kMaxReverseDepth - 1; i++) lines[i] = lines[i + 1];
+                if (--sp == 0) return status;
+            }
         }
         for (;;) {
-            if (sp == 0) return;
-            const int f = sp - 1;
-            if (have_ret) {              // the re-timed line fl[f] came back
-                have_ret = false;
-                if (ret == 0) { ret = fU[f]; have_ret = true; sp--; continue; }
-                fl[f] -= fF[f];
-            }
-            if (fl[f] == g.side_limit || fl[f] < 0 || fl[f] > across) {
-                ret = fU[f]; have_ret = true; sp--;
+            const int F = (sp & 1) ? future : -future;   // F of the top frame, number sp - 1
+            if (advance) lines[0] -= F;
+            advance = true;
+            const int l = lines[0];
+            if (l == side_limit || l < 0 || l > across) {
+#pragma unroll
+                for (int i = 0; i < kMaxReverseDepth - 1; i++) lines[i] = lines[i + 1];
+                if (--sp == 0) return status;
                 continue;
             }
-            curL = fl[f];
-            curF = -fF[f];
+            curL = l;
+            curF = -F;
             break;
         }
     }
@@ -296,9 +324,9 @@ EIK_HD void expand_box(G& g)
     int moved;
     do {
         moved = 0;
-        if (g.Y0 > 0) { g.Y0--; sweep_line<1>(g, g.Y0, -1, 0, g.X1); moved++; }
-        if (g.X1 < g.mx) { g.X1++; sweep_line<0>(g, g.X1, 1, g.Y0, g.Y1); moved++; }
-        if (g.Y1 < g.my) { g.Y1++; sweep_line<1>(g, g.Y1, 1, 0, g.X1); moved++; }
+        if (g.Y0 > 0) { g.Y0--; g.note(sweep_line<1>(g.view(), g.my, g.Y0, -1, 0, g.X1, g.cnt)); moved++; }
+        if (g.X1 < g.mx) { g.X1++; g.note(sweep_line<0>(g.view(), g.mx, g.X1, 1, g.Y0, g.Y1, g.cnt)); moved++; }
+        if (g.Y1 < g.my) { g.Y1++; g.note(sweep_line<1>(g.view(), g.my, g.Y1, 1, 0, g.X1, g.cnt)); moved++; }
     } while (moved);
 }
 
@@ -455,7 +483,7 @@ EIK_HD int solve(const float* s, int sstride, int nx, int ny, int iz, float* t, 
     Grid<CoarseMedium> g;
     g.t = t; g.ts = ts; g.nx = nx; g.ny = ny; g.mx = nx - 1; g.my = ny - 1;
     g.S = CoarseMedium{s, sstride, nx - 1, ny - 1};
-    g.ys = iz; g.status = kOk; g.cnt = cnt; g.side_limit = 0;
+    g.ys = iz; g.status = kOk; g.cnt = cnt;
     for (int i = 0; i < nx * ny; i++) t[(size_t)i * ts] = kInf;
 
     if (seed_source(g, true)) {
@@ -468,7 +496,7 @@ EIK_HD int solve(const float* s, int sstride, int nx, int ny, int iz, float* t, 
         Grid<FineMedium> f;
         f.t = tf; f.ts = ts; f.nx = nxf; f.ny = nyf; f.mx = nxf - 1; f.my = nyf - 1;
         f.S = FineMedium{g.S, j0, hy};
-        f.ys = ysf; f.status = kOk; f.cnt = cnt; f.side_limit = 0;
+        f.ys = ysf; f.status = kOk; f.cnt = cnt;
         for (int i = 0; i < nxf * nyf; i++) tf[(size_t)i * ts] = kInf;
         seed_source(f, false);
         expand_box(f);

@@ -261,7 +261,8 @@ cudaError_t eik_order_tasks(const EikBatch& b, int32_t* order, void* work, size_
 // per SM share the shared-memory slices (7 with the second column buffer of the lock-step box phase, Dims::lock_cols) and 8 TMEM sets (past column, current column, slowness column = 3 x 64
 // columns; two sets per lane quarter): a warp takes a slice for the box phase of a task, moves the task's last column and
 // slowness column into a TMEM set, gives the slice back and marches in tensor memory.  At any time about half of the warps
-// are in the latency-bound box phase and half in the issue-bound march, and there are 12 of them instead of 9 (146 registers each: no spills).
+// are in the latency-bound box phase and half in the issue-bound march, and there are 12 of them instead of 9 (168 registers each, the most 12 warps allow: no spills, no stack frame;
+// tests/test_sass_footprint_cpu.py).
 // Resources are taken in a fixed order (slice, then TMEM set; the tie scratch last and never while waiting for anything
 // else), holders of a TMEM set never wait for a slice: no cycle, no deadlock.
 // Two instantiations, chosen by the depth of the plane (pipe_shape): column arrays of CA = 64 nodes for nz <= 62 (the Example
