@@ -271,11 +271,10 @@ extern "C" int mq_create(const mq_config* cfg, const mq_picks* pk, int n_chains,
         if (fine) TRY(cudaMalloc(&h->eik_slice_scratch, (size_t)warps * eik_fine_slice_floats_per_warp(h->nxmod, h->nz) * sizeof(float)));
     }
     {
-        // regrouping of the solves of a table rebuild (MCMCEQ_EIKONAL_ORDER=0 keeps the natural order)
-        const char* e = getenv("MCMCEQ_EIKONAL_ORDER");
+        // regrouping of the solves of a table rebuild
         // (planes that do not fit a shared-memory slice keep the natural order: a chain's P and S solves of one source
         //  depth are neighbours there, which is the grouping their long box phases want; measured, tools/fine_probe2.py)
-        if (!(e && e[0] == '0') && eik_fast_supported(h->nxmod, h->nz)) {
+        if (eik_fast_supported(h->nxmod, h->nz)) {
             const int max_solves = 2 * n_chains * h->nz;
             h->eik_order_bytes = eik_order_bytes(max_solves);
             TRY(cudaMalloc(&h->eik_order_work, h->eik_order_bytes));

@@ -52,20 +52,11 @@ struct Counters {  // optional diagnostics, one per lane
 
 EIK_HD float fmin_ref(float a, float b) { return (a < b) ? a : b; }
 
-// t + sqrt(r) rounded once, the way the reference's (float)(t + sqrt((double)r)) is
-// (src/time_2d.c:1008): the correctly rounded sqrtf plus its first-order residual.
+// the reference's (float)(t + sqrt((double)r)) (src/time_2d.c:1008) in single precision: the correctly rounded sqrtf,
+// then the sum.
 EIK_HD float add_sqrt(float t, float r)
 {
     const float s = sqrtf(r);
-#ifdef EIK_COMPENSATED
-    if (s > 0.f) {
-        const float e = fmaf(-s, s, r);       // r - s*s, exact
-        const float c = e * (0.5f / s);       // sqrt(r) ~= s + c
-        const float sum = t + s;
-        const float err = (t - sum) + s;      // Fast2Sum tail (t >= s away from the source; harmless otherwise)
-        return sum + (err + c);
-    }
-#endif
     return t + s;
 }
 
@@ -435,12 +426,6 @@ EIK_HD float box_time(float hs0, int x, int dy)
     const float fy = (float)dy;
     const float sq = fmaf((float)x, (float)x, fy * fy);   // exact: small integers
     const float s = sqrtf(sq);
-#ifdef EIK_COMPENSATED
-    if (s > 0.f) {
-        const float c = fmaf(-s, s, sq) * (0.5f / s);
-        return fmaf(hs0, s, hs0 * c);
-    }
-#endif
     return hs0 * s;
 }
 

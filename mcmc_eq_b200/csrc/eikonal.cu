@@ -110,7 +110,7 @@ bool eik_fast_supported(int nxmod, int nz)
 // shared-memory slice, so that the lock-step sweeps (rows, the march) touch one 128-byte line per access.  Same code,
 // same results; what hides the memory latency is the number of resident warps.
 template <bool GLOBAL_SLICE>
-__device__ __forceinline__ void eik_fast_body(const EikBatch& b, const eikf::Dims& D, float* slice)
+__device__ __forceinline__ void eik_fast_body(const EikBatch& b, const eikf::Dims& D, float* slice, int lpt)
 {
     const int lane = threadIdx.x;
     const int nodes = b.nxmod * b.nz;
@@ -121,7 +121,6 @@ __device__ __forceinline__ void eik_fast_body(const EikBatch& b, const eikf::Dim
     L.WF = L.W + (size_t)D.wx * D.nz * 32;
     const int n_items = b.n_items_dev ? *b.n_items_dev : b.n_items;
     const int n_solves = b.src_iz ? b.n_solves : n_items * b.nz;
-    const int lpt = b.lanes_per_task;           // lanes of a warp that carry a solve
     const int n_tasks = (n_solves + lpt - 1) / lpt;
 
     for (int task = blockIdx.x; task < n_tasks; task += gridDim.x) {
@@ -143,9 +142,6 @@ __device__ __forceinline__ void eik_fast_body(const EikBatch& b, const eikf::Dim
             }
             if (b.full_out) t.full = b.full_out + (size_t)g * nodes;
         }
-#ifdef EIKF_TRACE
-        t.trace = (g == EIKF_TRACE);
-#endif
         const int rc = eikf::solve_warp<GLOBAL_SLICE>(D, L, t, b.rows, b.n_rows);
         if (t.valid) {
             if (b.status) b.status[g] = rc;
@@ -155,15 +151,16 @@ __device__ __forceinline__ void eik_fast_body(const EikBatch& b, const eikf::Dim
     }
 }
 
-__global__ void __launch_bounds__(32, 9) eik_fast_kernel(EikBatch b, eikf::Dims D)
+// lanes_per_task: lanes of a warp that carry a solve (32, 16, 8 or 4)
+__global__ void __launch_bounds__(32, 9) eik_fast_kernel(EikBatch b, eikf::Dims D, int lanes_per_task)
 {
     extern __shared__ float smem[];
-    eik_fast_body<false>(b, D, smem);
+    eik_fast_body<false>(b, D, smem, lanes_per_task);
 }
 
-__global__ void __launch_bounds__(32, 8) eik_fine_kernel(EikBatch b, eikf::Dims D)
+__global__ void __launch_bounds__(32, 8) eik_fine_kernel(EikBatch b, eikf::Dims D, int lanes_per_task)
 {
-    eik_fast_body<true>(b, D, b.slice_scratch + (size_t)blockIdx.x * ((size_t)eikf::gmem_floats_per_lane(D) * 32));
+    eik_fast_body<true>(b, D, b.slice_scratch + (size_t)blockIdx.x * ((size_t)eikf::gmem_floats_per_lane(D) * 32), lanes_per_task);
 }
 
 // ---- regrouping of solves --------------------------------------------------------------------------------------
@@ -208,20 +205,7 @@ __global__ void eik_key_kernel(EikBatch b, int max_solves, uint64_t* keys, int32
     // half-width of the seed box first: it decides the kind of initialisation (src/time_2d.c:682-711)
     const uint64_t wd = (d0 == 31) ? 15 : (d0 >> 1), wu = (u0 == 31) ? 15 : (u0 >> 1), w = wd < wu ? wd : wu;
     (void)u2;
-#if defined(MCMCEQ_ORDER_EDGES_FIRST)      // A/B builds: source depths from the edges of the depth range inwards (long box phases first)
-    const int zk = (iz <= my / 2) ? 2 * iz : 2 * (my - iz) + 1;
-#elif defined(MCMCEQ_ORDER_INTERLEAVE)     // upper and lower half of the depth range alternately: long and short box phases mixed
-    const int zk = (iz <= my / 2) ? 2 * iz : 2 * (iz - my / 2 - 1) + 1;
-#elif defined(MCMCEQ_ORDER_MID_UP_DOWN)     // from the middle down to the bottom, then from the middle up to the top (two monotone runs)
-    const int zk = (iz > my / 2) ? iz - my / 2 - 1 : my - iz;
-#elif defined(MCMCEQ_ORDER_TOP_BOTTOM_IN)  // from the top to the middle, then from the bottom to the middle
-    const int zk = (iz <= my / 2) ? iz : my / 2 + 1 + (my - iz);
-#elif defined(MCMCEQ_ORDER_MIDDLE_FIRST)
-    const int zk = 2 * my + 1 - ((iz <= my / 2) ? 2 * iz : 2 * (my - iz) + 1);
-#else
-    const int zk = iz;
-#endif
-    keys[g] = ((uint64_t)zk << 32) | (w << 28) | (d0 << 23) | (u0 << 18) | (d1 << 13) | (u1 << 8) | (d2 << 3);
+    keys[g] = ((uint64_t)iz << 32) | (w << 28) | (d0 << 23) | (u0 << 18) | (d1 << 13) | (u1 << 8) | (d2 << 3);
     vals[g] = g;
 }
 
@@ -269,53 +253,40 @@ cudaError_t eik_order_tasks(const EikBatch& b, int32_t* order, void* work, size_
 // plane), and CA = 128 for 88 <= nz <= 126, which holds the planes of the example grids refined by halving the spacing.  A CA = 128 set is 384
 // columns, so a lane quarter holds one and 4 marches are in flight per SM; slices are 48 - 64 KB at those depths (3 - 4 per
 // SM), so fewer warps per CTA (profiles/README.md, deep planes).
-#ifndef MCMCEQ_PIPE_WARPS
-#define MCMCEQ_PIPE_WARPS 12
-#endif
-#ifndef MCMCEQ_PIPE_WARPS_DEEP
-#define MCMCEQ_PIPE_WARPS_DEEP 8
-#endif
-constexpr int kPipeWarps = MCMCEQ_PIPE_WARPS;     // CA = 64.  Measured 10 .. 20: 12 - 13 are best at 1024 chains, 12 - 16 equal at 8192 (profiles/README.md)
-constexpr int kPipeWarpsDeep = MCMCEQ_PIPE_WARPS_DEEP;   // CA = 128.  Measured 6, 8, 12: 8 is best or level (profiles/README.md)
+constexpr int kPipeWarps = 12;       // CA = 64.  Measured 10 .. 20: 12 - 13 are best at 1024 chains, 12 - 16 equal at 8192 (profiles/README.md)
+constexpr int kPipeWarpsDeep = 8;    // CA = 128.  Measured 6, 8, 12: 8 is best or level (profiles/README.md)
 constexpr int kPipeMaxCtas = 256;    // one CTA per SM; the tie scratch is sized for this many
 // two time columns + slowness column of the tie scratch of a CTA
 template <int CA>
 constexpr size_t kPipeTieFloats = (size_t)(3 * CA + 2) * 32;
-// The instantiation a plane of nz depth nodes takes (ca = 0: none), its warps per CTA and its default box-phase variant
-// (Dims::lock_cols; MCMCEQ_PIPE_LC overrides it).
+// The instantiation a plane of nz depth nodes takes (ca = 0: none) and its warps per CTA.
 struct PipeShape {
-    int ca, warps, lock_cols;
+    int ca, warps;
 };
 // Lowest nz for CA = 128: a shallower plane fills too little of the column arrays, and the fused kernel is faster (B200,
 // 1024 chains: 21.3 against 22.7 ms per launch at nz = 80, 33.4 against 27.5 at nz = 88; DESIGN.md section 3).
 constexpr int kPipeDeepMinNz = 88;
 static PipeShape pipe_shape(int nz)
 {
-    if (nz + 2 <= 64) return {64, kPipeWarps, 1};
-    if (nz >= kPipeDeepMinNz && nz + 2 <= 128) return {128, kPipeWarpsDeep, 1};
-    return {0, 0, 0};
+    if (nz + 2 <= 64) return {64, kPipeWarps};
+    if (nz >= kPipeDeepMinNz && nz + 2 <= 128) return {128, kPipeWarpsDeep};
+    return {0, 0};
 }
 
 // The box phase of a task.  Until round 2 it had to be compiled as a function of its own: inlined next to the tensor-memory
 // march, nvcc 12.9 produced a kernel whose box-region output was wrong (bisected on the GPU in round 1: any variant with the
 // call inlined and the top-row site of run_grid present failed).  Printing one solve's box phase from both kernels
-// (-DEIKF_TRACE) showed what goes wrong: at that site the row's own strip slowness c came out as the far side's c2.  With the
-// two reads volatile (eik_fast.cuh, run_grid) the inlined kernel is bit-identical to the fused one and 8 % faster (LDS / STS
-// instead of generic loads and stores); tests/test_pipe_gpu.py compares the two kernels bit for bit on four model families
-// and guards this.  -DMCMCEQ_PIPE_NOINLINE restores the out-of-line call.
+// (profiles/README.md r2c) showed what goes wrong: at that site the row's own strip slowness c came out as the far side's c2.
+// With the two reads volatile (eik_fast.cuh, run_grid) the inlined kernel is bit-identical to the fused one and 8 % faster
+// (LDS / STS instead of generic loads and stores); tests/test_pipe_gpu.py compares the two kernels bit for bit on four model
+// families and guards this.  The columns of the growing box are swept in lock-step (Dims::lock_cols).
 // Arguments by value: as references they would live in the caller's stack frame and be re-read through it.
 // x1 receives the column at which the box phase ended (-1: nothing left to march).
-#ifdef MCMCEQ_PIPE_NOINLINE
-#define MQ_PIPE_CALL __noinline__
-#else
-#define MQ_PIPE_CALL __forceinline__
-#endif
-template <bool LC>
-__device__ MQ_PIPE_CALL int solve_warp_call(eikf::Dims D, eikf::Lane L, eikf::LaneTask t, const int* rows, int n_rows, int* x1_out)
+__device__ __forceinline__ int solve_warp_call(eikf::Dims D, eikf::Lane L, eikf::LaneTask t, const int* rows, int n_rows, int* x1_out)
 {
     int x1 = -1;
     t.hand_x1 = &x1;
-    const int rc = eikf::solve_warp<false, LC>(D, L, t, rows, n_rows);
+    const int rc = eikf::solve_warp<false, true>(D, L, t, rows, n_rows);
     *x1_out = x1;
     return rc;
 }
@@ -407,10 +378,7 @@ __global__ void __launch_bounds__(WARPS * 32, 1) eik_pipe_kernel(EikBatch b, eik
             t.out = tab + (size_t)t.iz * b.xpitch;
             t.out_rstride = (long)nz * b.xpitch;
         }
-#ifdef EIKF_TRACE
-        t.trace = (g == EIKF_TRACE);
-#endif
-        const int rc = D.lock_cols ? solve_warp_call<true>(D, L, t, b.rows, b.n_rows, &x1) : solve_warp_call<false>(D, L, t, b.rows, b.n_rows, &x1);
+        const int rc = solve_warp_call(D, L, t, b.rows, b.n_rows, &x1);
         if (t.valid && b.status_min && rc < 0) atomicMin(b.status_min, rc);
         const bool live = x1 >= 0 && x1 < mx;
         if (!__any_sync(0xffffffffu, live)) { pipe_release(&ctl.slice_free, sl, lane); continue; }
@@ -518,30 +486,19 @@ cudaError_t eik_launch_pipe(const EikBatch& b, int* task_counter, cudaStream_t s
     if (!sh.ca) return cudaErrorInvalidValue;
     void (*const kernel)(EikBatch, eikf::Dims, int, int*) = sh.ca == 64 ? eik_pipe_kernel<64, kPipeWarps> : eik_pipe_kernel<128, kPipeWarpsDeep>;
     eikf::Dims D = fast_dims(b.nxmod, b.nz);
-    {
-        // Lock-step columns in the box phase (a second column buffer per slice: 7 slices instead of 9 on the Example plane).
-        // Kernel ms per launch at 1024 / 2048 / 4096 / 8192 chains with the box phase inlined: 7.70 / 13.99 / 26.42 / 51.07
-        // against 8.03 / 14.24 / 26.66 / 51.07 with the per-lane in-place walk (profiles/README.md r2c).  MCMCEQ_PIPE_LC=0
-        // selects the in-place walk.
-        static int lc_env = -2;
-        if (lc_env == -2) { const char* e = getenv("MCMCEQ_PIPE_LC"); lc_env = e ? atoi(e) : -1; }
-        D.lock_cols = (lc_env >= 0) ? (lc_env != 0) : sh.lock_cols;
-    }
+    // Lock-step columns in the box phase (a second column buffer per slice: 7 slices instead of 9 on the Example plane).
+    // Kernel ms per launch at 1024 / 2048 / 4096 / 8192 chains with the box phase inlined: 7.70 / 13.99 / 26.42 / 51.07
+    // against 8.03 / 14.24 / 26.66 / 51.07 with the per-lane in-place walk (profiles/README.md r2c).
+    D.lock_cols = 1;
     const size_t slice = fast_smem_floats_per_warp(D) * sizeof(float);
-    const size_t tie = 0;      // the tie scratch lives in global memory (b.tie_scratch)
     int dev = 0, sms = 148, smem_max = 232448;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-    int n_slices = (int)(((size_t)smem_max - tie - 256) / slice);
+    int n_slices = (int)(((size_t)smem_max - 256) / slice);
     if (n_slices > sh.warps) n_slices = sh.warps;
-    {
-        static int env_slices = -1;      // experiment: fewer slices than fit (profiles/README.md)
-        if (env_slices < 0) { const char* e = getenv("MCMCEQ_PIPE_SLICES"); env_slices = e ? atoi(e) : 0; }
-        if (env_slices >= 2 && env_slices < n_slices) n_slices = env_slices;
-    }
     if (n_slices < 2) return cudaErrorInvalidValue;
-    const size_t smem = (size_t)n_slices * slice + tie;
+    const size_t smem = (size_t)n_slices * slice;
     // per instantiation and device: largest dynamic shared-memory size the kernel has been opted in for
     static size_t configured[2][64] = {};
     size_t* conf = (dev >= 0 && dev < 64) ? &configured[sh.ca == 128][dev] : nullptr;
@@ -604,23 +561,12 @@ cudaError_t eik_launch_fast(const EikBatch& b, cudaStream_t stream)
     if (warps > resident) warps = resident;
     // A launch with fewer warp-tasks than warps that can be resident lasts as long as one task, and a task is the shorter
     // the fewer lanes have to wait for each other in the box phase: spread it over the idle warps.
-    EikBatch bb = b;
-    static int lanes_env = -1;
-    if (lanes_env < 0) {
-        const char* e = getenv("MCMCEQ_EIKONAL_LANES");     // 32 / 16 / 8 / 4: fixed; unset: chosen per launch
-        lanes_env = e ? atoi(e) : 0;
-    }
-    if (!bb.lanes_per_task) bb.lanes_per_task = lanes_env;
-    int lpt = (bb.lanes_per_task == 32 || bb.lanes_per_task == 16 || bb.lanes_per_task == 8 || bb.lanes_per_task == 4) ? bb.lanes_per_task : 0;
-    if (!lpt) {
-        lpt = 32;
-        while (lpt > 4 && ((long)n_solves + lpt / 2 - 1) / (lpt / 2) <= warps) lpt /= 2;
-    }
-    bb.lanes_per_task = lpt;
+    int lpt = 32;
+    while (lpt > 4 && ((long)n_solves + lpt / 2 - 1) / (lpt / 2) <= warps) lpt /= 2;
     const int n_tasks = (n_solves + lpt - 1) / lpt;
     if (warps > n_tasks) warps = n_tasks;
     if (warps < 1) warps = 1;
-    eik_fast_kernel<<<(unsigned)warps, 32, smem, stream>>>(bb, D);
+    eik_fast_kernel<<<(unsigned)warps, 32, smem, stream>>>(b, D, lpt);
     count_launch();
     return cudaGetLastError();
 }
@@ -642,8 +588,6 @@ cudaError_t eik_launch_fine(const EikBatch& b, cudaStream_t stream)
     if (n_solves <= 0) return cudaSuccess;
     if (!b.slice_scratch) return cudaErrorInvalidValue;
     const eikf::Dims D = fast_dims(b.nxmod, b.nz);
-    EikBatch bb = b;
-    bb.lanes_per_task = 32;
     const int n_tasks = (n_solves + 31) / 32;
     // one warp per CTA; the window (b.scratch) and the slice were sized for max_warps warps
     const size_t have = (size_t)b.max_warps * eik_scratch_floats_per_warp(b.nxmod, b.nz);
@@ -651,7 +595,7 @@ cudaError_t eik_launch_fine(const EikBatch& b, cudaStream_t stream)
     if (warps > b.max_warps) warps = b.max_warps;
     if (warps > n_tasks) warps = n_tasks;
     if (warps < 1) warps = 1;
-    eik_fine_kernel<<<(unsigned)warps, 32, 0, stream>>>(bb, D);
+    eik_fine_kernel<<<(unsigned)warps, 32, 0, stream>>>(b, D, 32);
     count_launch();
     return cudaGetLastError();
 }
@@ -676,9 +620,8 @@ cudaError_t eik_launch(const EikBatch& b, cudaStream_t stream, int* which)
         const int warps = pipe_shape(b.nz).warps;
         if ((long)(have / fast_scratch_floats_per_warp(D)) >= (long)sms * warps && n_tasks >= (long)sms * warps &&
             sms <= kPipeMaxCtas) {
-            EikBatch piped = b;
             *which = kEikPipe;
-            return eik_launch_pipe(piped, b.task_counter, stream);
+            return eik_launch_pipe(b, b.task_counter, stream);
         }
     }
     if (!force_generic && eik_fast_supported(b.nxmod, b.nz)) { *which = kEikFast; return eik_launch_fast(b, stream); }

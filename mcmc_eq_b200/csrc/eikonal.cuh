@@ -24,8 +24,6 @@ struct EikBatch {
     // task j / 32 runs, or -1 (eik_order_tasks fills it: solves of one source depth that initialise and grow their
     // boxes alike are made neighbours so that the lanes of a warp stay in step).
     const int32_t* order;
-    int lanes_per_task;       // fused kernel: solves per warp-task (32, 16, 8 or 4; 0 = chosen by eik_launch_fast: fewer when
-                              // the launch has fewer tasks than resident warps, so that a small launch spreads over the SMs)
     int32_t* task_counter;    // [1] device: work counter of the pipelined kernel (eik_launch_pipe), or nullptr
     float* tie_scratch;       // device, eik_pipe_tie_floats(nz) floats: per-CTA scratch of the pipelined kernel's tie fallback
     // Outputs (device).  full_out: [n_solves][nxmod*nz] in the reference layout (x*nz+y).

@@ -23,13 +23,10 @@ extern "C" int emu_time_2d(const float* s, int nx, int ny, int iz, float* t, int
 // gm == 2: shared-memory slice with a second column buffer (Dims::lock_cols): lock-step columns without the read-ahead
 static int g_gm = 0;
 extern "C" void emu_set_gm(int on) { g_gm = on; }
-static int g_row_march = 1;   // 0: rows by the general per-lane walk (MCMCEQ_ROW_MARCH=0)
-extern "C" void emu_set_row_march(int on) { g_row_march = on; }
 extern "C" int emu_fast_time_2d(const float* s, int nx, int ny, int iz, float* t, const int* rows, int n_rows, float* rows_out)
 {
     eikf::Dims D = eikf::make_dims(nx, ny);
     D.lock_cols = (g_gm == 2) ? 1 : 0;
-    D.row_march = g_row_march;
     std::vector<float> SM(eikf::gmem_floats_per_lane(D)), W((size_t)D.wx * ny), WF(22 * 43);
     eikf::Lane L;
     if (g_gm == 1) eikf::carve_global(SM.data(), D, &L);
@@ -40,6 +37,3 @@ extern "C" int emu_fast_time_2d(const float* s, int nx, int ny, int iz, float* t
     return g_gm == 1 ? eikf::solve_warp<true, false>(D, L, task, rows, n_rows)
          : g_gm == 2 ? eikf::solve_warp<false, true>(D, L, task, rows, n_rows) : eikf::solve_warp<false, false>(D, L, task, rows, n_rows);
 }
-#ifdef EIKF_STATS
-extern "C" void emu_stats(long* out) { for (int i = 0; i < 12; i++) out[i] = eikf::g_stats[i]; }
-#endif

@@ -58,11 +58,9 @@ np.savez(sys.argv[1], **out)
 """
 
 
-def _run(path, pipe, lock_cols=None, planes=PLANES, kinds=KINDS):
+def _run(path, pipe, planes=PLANES, kinds=KINDS):
     import json
     env = dict(os.environ, MCMCEQ_EIKONAL_PIPE="1" if pipe else "0")
-    if lock_cols is not None:
-        env["MCMCEQ_PIPE_LC"] = "1" if lock_cols else "0"
     r = subprocess.run([sys.executable, "-c", SCRIPT % util.ROOT, path, json.dumps(planes), ",".join(kinds), str(N_CHAINS)],
                        env=env, capture_output=True, text=True, timeout=1800)
     assert r.returncode == 0, r.stderr[-1500:]
@@ -71,18 +69,16 @@ def _run(path, pipe, lock_cols=None, planes=PLANES, kinds=KINDS):
 
 def test_deep_pipelined_kernel_is_bit_identical_to_the_fused_kernel(tmp_path):
     """Class sums, origin times, per-pick predictions of the first and the last chain, counters and log-likelihoods after a
-    few mixed steps: identical bits, on every plane and model family, with and without the second column buffer of the box
-    phase (Dims::lock_cols)."""
+    few mixed steps: identical bits, on every plane and model family."""
     a = _run(str(tmp_path / "fused.npz"), False)
-    for lc in (True, False):
-        b = _run(str(tmp_path / "pipe.npz"), True, lock_cols=lc)
-        for k in a:
-            if k.endswith("_kernels"):
-                assert list(a[k]) == ["eik_fast_kernel"], (k, a[k])
-                assert list(b[k]) == ["eik_pipe_kernel"], (lc, k, b[k])
-                continue
-            assert np.array_equal(a[k], b[k]), (lc, k, int((a[k] != b[k]).sum()), a[k].size,
-                                                float(np.nanmax(np.abs(a[k].astype(float) - b[k].astype(float)))))
+    b = _run(str(tmp_path / "pipe.npz"), True)
+    for k in a:
+        if k.endswith("_kernels"):
+            assert list(a[k]) == ["eik_fast_kernel"], (k, a[k])
+            assert list(b[k]) == ["eik_pipe_kernel"], (k, b[k])
+            continue
+        assert np.array_equal(a[k], b[k]), (k, int((a[k] != b[k]).sum()), a[k].size,
+                                            float(np.nanmax(np.abs(a[k].astype(float) - b[k].astype(float)))))
 
 
 def _kernels_taken(directory, name, nz_override=None):

@@ -38,10 +38,8 @@ np.savez(sys.argv[1], **out)
 """
 
 
-def _run(path, pipe, n, row_march=True, lock_cols=None, kinds="lvz,posterior"):
+def _run(path, pipe, n, row_march=True, kinds="lvz,posterior"):
     env = dict(os.environ, MCMCEQ_EIKONAL_PIPE="1" if pipe else "0", MCMCEQ_ROW_MARCH="1" if row_march else "0")
-    if lock_cols is not None:
-        env["MCMCEQ_PIPE_LC"] = "1" if lock_cols else "0"
     r = subprocess.run([sys.executable, "-c", SCRIPT % util.ROOT, path, str(n), kinds], env=env, capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stderr[-1500:]
     return dict(np.load(path))
@@ -51,12 +49,9 @@ def test_pipelined_kernel_is_bit_identical_to_the_fused_kernel(tmp_path):
     """One persistent CTA per SM, 16 warps sharing a pool of shared-memory slices (box phase) and a pool of TMEM sets (march)."""
     # the pipelined kernel only takes launches with work for all 148 x 12 warps: 1230 chains x 2 phases x 61 depths
     a = _run(str(tmp_path / "fused.npz"), False, 1230)
-    # both box-phase variants of the pipelined kernel: lock-step columns (launches up to 3 tasks per warp deep) and the
-    # per-lane in-place walk (deeper launches)
-    for lc in (True, False):
-        b = _run(str(tmp_path / "pipe.npz"), True, 1230, lock_cols=lc)
-        for k in a:
-            assert np.array_equal(a[k], b[k]), (lc, k, int((a[k] != b[k]).sum()), a[k].size, float(np.nanmax(np.abs(a[k].astype(float) - b[k].astype(float)))))
+    b = _run(str(tmp_path / "pipe.npz"), True, 1230)
+    for k in a:
+        assert np.array_equal(a[k], b[k]), (k, int((a[k] != b[k]).sum()), a[k].size, float(np.nanmax(np.abs(a[k].astype(float) - b[k].astype(float)))))
 
 
 @pytest.mark.parametrize("kinds", ["posterior,contrast", "contrast,lvz", "gradient,gradient"])
@@ -65,10 +60,9 @@ def test_pipelined_kernel_is_bit_identical_on_other_model_families(tmp_path, kin
     round 1 (eikonal.cu, solve_warp_call) gave wrong times on one model family and right ones on another, so the comparison
     runs on all of them (Example2 grid, Example grid): low-velocity zones, posterior-like, high-contrast, gradient models."""
     a = _run(str(tmp_path / "fused.npz"), False, 1230, kinds=kinds)
-    for lc in (True, False):
-        b = _run(str(tmp_path / "pipe.npz"), True, 1230, lock_cols=lc, kinds=kinds)
-        for k in a:
-            assert np.array_equal(a[k], b[k]), (kinds, lc, k, int((a[k] != b[k]).sum()), a[k].size)
+    b = _run(str(tmp_path / "pipe.npz"), True, 1230, kinds=kinds)
+    for k in a:
+        assert np.array_equal(a[k], b[k]), (kinds, k, int((a[k] != b[k]).sum()), a[k].size)
 
 
 def test_lock_step_row_sweeps_are_bit_identical_to_the_general_walk(tmp_path):

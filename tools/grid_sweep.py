@@ -9,7 +9,7 @@ switch is read once per process), the two settings alternating; a run warms up w
 steps with CUDA events on the library's stream (mq_timer) and the eikonal launches with mq_profile, reads the kernel taken
 from mq_profile_kernels, and checks 4 chains against the CPU oracle (tests/test_bench_scale_gpu.py: predictions, class sums,
 origin times, receiver rows), so that a fast but wrong plane does not pass.  The environment passes through to the
-subprocesses (MCMCEQ_LIB, MCMCEQ_PIPE_LC, ...).  Writes DIR/runs.jsonl (one line per run), DIR/summary.json and
+subprocesses (MCMCEQ_LIB, ...).  Writes DIR/runs.jsonl (one line per run), DIR/summary.json and
 DIR/summary.md (median and spread of the repeats per plane and setting), with the card name and power limit."""
 from __future__ import annotations
 
