@@ -178,6 +178,19 @@ int mq_get_table(mq_handle* h, int chain, int phase, float* ttt);
  * status; either output may be NULL (call with both NULL to learn n_rows). */
 int mq_get_rows(mq_handle* h, int chain, int phase, float* rows_out, int32_t* row_index);
 
+/* How the travel-time tables are built (opt-in fast mode).  MQ_TABLES_PARITY (the default): one solve per source depth,
+ * nz per (chain, phase) table, as the reference does (src/misfit.c:270-289).  MQ_TABLES_RECIPROCAL: one solve per stored
+ * receiver row, with the source at that row, and the event depth read off its field: rows_out[r][iz][i] of mq_get_rows
+ * is then the time from a source at (0, row_index[r]) to node (i, iz), used as the time from (0, iz) to (i, row_index[r]).
+ * n_rows solves instead of nz (3 instead of 62 on the Example grid).  The finite-difference scheme is not exactly
+ * reciprocal, so predictions differ from the parity mode's: DESIGN.md section 6 gives the measured error.  mq_forward,
+ * mq_forward_host, mq_step, mq_replay_step and the rebuild in mq_state_load follow the mode; mq_get_table gives
+ * MQ_ERR_UNSUPPORTED (no parity table exists).  No effect with eikonal == 0 or aflag == 1.  Call before mq_set_models /
+ * mq_init_chains / mq_state_load: MQ_ERR_STATE afterwards; MQ_ERR_ARG for any other mode. */
+#define MQ_TABLES_PARITY 0
+#define MQ_TABLES_RECIPROCAL 1
+int mq_set_tables(mq_handle* h, int mode);
+
 /* Per-pick predictions of one chain after mq_forward: what cal_fit_newx prints with out=1
  * (src/misfit.c:130-143).  resid / tpred are [n_picks] in the handle's pick order. */
 int mq_get_predictions(mq_handle* h, int chain, float* resid, float* tpred);
@@ -363,7 +376,9 @@ int mq_temper_swap(mq_handle* h, int64_t round, int32_t* n_swapped);
  *   damaged) -- is refused with MQ_ERR_ARG before anything on the device changes: the handle stays as it was.  The
  *   travel-time tables are not in the state; they are rebuilt, and their hashes compared with the saved ones: a table
  *   that differs (a library whose eikonal results differ) gives MQ_ERR_STATE, mq_last_error() names the first chain and
- *   phase, and the handle has no usable state until the next mq_state_load / mq_init_chains / mq_set_models.
+ *   phase, and the handle has no usable state until the next mq_state_load / mq_init_chains / mq_set_models.  A state
+ *   saved with reciprocal tables (MQ_STATE_RECIPROCAL) loads only into a handle set to MQ_TABLES_RECIPROCAL, a state
+ *   without the flag only into a parity handle; anything else is refused with MQ_ERR_ARG before the device changes.
  *
  * Layout (native little-endian): an mq_state_header, n_sections mq_state_section entries, the sections at their offsets
  * (8-byte aligned, zero padding), and a trailing uint64 checksum of every byte before it.  Checksums are sum64: starting
@@ -384,6 +399,7 @@ int mq_temper_swap(mq_handle* h, int64_t round, int32_t* n_swapped);
 #define MQ_STATE_BETA 2u
 #define MQ_STATE_TABLES 4u       /* table hashes present (no tables exist with eikonal == 0 or aflag == 1) */
 #define MQ_STATE_DIAG 8u         /* diagnostics accumulators present (mq_diag_begin) */
+#define MQ_STATE_RECIPROCAL 16u  /* saved from a handle with reciprocal tables (mq_set_tables); set only with MQ_STATE_TABLES */
 #define MQ_STATE_SEC_CHAINS 1u
 #define MQ_STATE_SEC_TABLES 2u
 #define MQ_STATE_SEC_POSTERIOR 3u
@@ -397,7 +413,7 @@ typedef struct mq_state_header {
     int32_t n_chains, max_dim, n_events, n_stations, n_picks, nz, nxmod, n_rows;
     uint64_t seed;
     int64_t chain_offset;
-    uint32_t flags;            /* MQ_STATE_POSTERIOR | MQ_STATE_BETA | MQ_STATE_TABLES | MQ_STATE_DIAG */
+    uint32_t flags;            /* MQ_STATE_POSTERIOR | MQ_STATE_BETA | MQ_STATE_TABLES | MQ_STATE_DIAG | MQ_STATE_RECIPROCAL */
     uint32_t n_sections;
     float post_dv, post_dvpvs; /* mq_posterior_begin's arguments and the histogram sizes (0 when off) */
     int32_t post_ndv, post_ndvpvs;
@@ -411,8 +427,8 @@ int mq_state_load(mq_handle* h, const void* buf, uint64_t bytes);
 
 /* Measurement aid for bench.py: with enable != 0 every eikonal launch is bracketed by CUDA events on
  * the handle's stream.  Returns the time and number of launches accumulated since the previous call
- * (and restarts the accumulation); solves_per_full_launch = 2 * n_chains * nz, the number of solves one
- * launch performs when every chain rebuilds both tables. */
+ * (and restarts the accumulation); solves_per_full_launch = 2 * n_chains * nz (2 * n_chains * n_rows with reciprocal
+ * tables), the number of solves one launch performs when every chain rebuilds both tables. */
 int mq_profile(mq_handle* h, int enable, double* eikonal_ms, int64_t* eikonal_launches,
                int64_t* solves_per_full_launch);
 

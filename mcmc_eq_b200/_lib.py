@@ -100,7 +100,8 @@ class MqStateSection(C.Structure):
     _fields_ = [("id", C.c_uint32), ("reserved", C.c_uint32), ("offset", C.c_uint64), ("bytes", C.c_uint64)]
 
 
-STATE_POSTERIOR, STATE_BETA, STATE_TABLES, STATE_DIAG = 1, 2, 4, 8
+STATE_POSTERIOR, STATE_BETA, STATE_TABLES, STATE_DIAG, STATE_RECIPROCAL = 1, 2, 4, 8, 16
+TABLES_PARITY, TABLES_RECIPROCAL = 0, 1     # mq_set_tables
 STATE_SEC_DIAG = 5
 
 
@@ -144,6 +145,7 @@ def lib() -> C.CDLL:
         L.mq_tables_restore.argtypes = [C.c_void_p]
         L.mq_get_table.argtypes = [C.c_void_p, C.c_int, C.c_int, fp]
         L.mq_get_rows.argtypes = [C.c_void_p, C.c_int, C.c_int, fp, C.POINTER(C.c_int32)]
+        L.mq_set_tables.argtypes = [C.c_void_p, C.c_int]
         L.mq_get_predictions.argtypes = [C.c_void_p, C.c_int, fp, fp]
         L.mq_init_chains.argtypes = [C.c_void_p]
         L.mq_step.argtypes = [C.c_void_p, C.c_int, C.c_char_p]
@@ -334,6 +336,14 @@ class Sampler:
 
     def tables_restore(self):
         check(lib().mq_tables_restore(self.h))
+
+    def set_tables(self, mode: str):
+        """How tables are built: "parity" (the default, one solve per source depth) or "reciprocal" (one solve per receiver
+        row, an approximation: DESIGN.md section 6).  Before set_models / init_chains / load_state."""
+        modes = {"parity": TABLES_PARITY, "reciprocal": TABLES_RECIPROCAL}
+        if mode not in modes:
+            raise ValueError(f"table mode {mode!r}: 'parity' or 'reciprocal'")
+        check(lib().mq_set_tables(self.h, modes[mode]))
 
     def table(self, chain: int, phase: int) -> np.ndarray:
         t = np.zeros((self.nz, self.nz, self.nxmod), np.float32)

@@ -100,7 +100,7 @@ extern "C" int mq_destroy(mq_handle* hh)
     cudaFree(h->pk.ev_off); cudaFree(h->pk.n_p); cudaFree(h->pk.st_id); cudaFree(h->pk.r0); cudaFree(h->pk.cp);
     cudaFree(h->pk.x); cudaFree(h->pk.y); cudaFree(h->pk.t); cudaFree(h->pk.w1); cudaFree(h->pk.w2); cudaFree(h->pk.fix);
     cudaFree(h->pk.rec4); cudaFree(h->pk.rec2);
-    cudaFree(h->d_rows);
+    cudaFree(h->d_rows); cudaFree(h->d_all_rows);
     free(h->rows_host);
     cudaFree(h->dim); cudaFree(h->mcur); cudaFree(h->tcur); cudaFree(h->ecur);
     cudaFree(h->z); cudaFree(h->vp); cudaFree(h->vpvs); cudaFree(h->eq); cudaFree(h->pres); cudaFree(h->sres);
@@ -230,6 +230,12 @@ extern "C" int mq_create(const mq_config* cfg, const mq_picks* pk, int n_chains,
         TRY(cudaStreamSynchronize(s));
     }
     TRY(dalloc(&h->d_rows, h->n_rows)); TRY(h2d(h->d_rows, h->rows_host, h->n_rows, s));
+    {
+        std::vector<int32_t> all(g.nz);
+        for (int j = 0; j < g.nz; j++) all[j] = j;
+        TRY(dalloc(&h->d_all_rows, g.nz)); TRY(h2d(h->d_all_rows, all.data(), g.nz, s));
+        TRY(cudaStreamSynchronize(s));
+    }
 
     TRY(dalloc(&h->dim, 2 * n)); TRY(dalloc(&h->mcur, n)); TRY(dalloc(&h->tcur, 2 * n)); TRY(dalloc(&h->ecur, n));
     TRY(dalloc(&h->z, 2 * n * h->md)); TRY(dalloc(&h->vp, 2 * n * h->md)); TRY(dalloc(&h->vpvs, 2 * n * h->md));
@@ -563,10 +569,25 @@ extern "C" int mq_get_rows(mq_handle* hh, int chain, int phase, float* rows_out,
     return h->n_rows;
 }
 
+extern "C" int mq_set_tables(mq_handle* hh, int mode)
+{
+    if (!hh) { set_error("mq_set_tables: null"); return MQ_ERR_ARG; }
+    if (mode != MQ_TABLES_PARITY && mode != MQ_TABLES_RECIPROCAL) { set_error("mq_set_tables: mode %d", mode); return MQ_ERR_ARG; }
+    Handle* h = &hh->h;
+    // the tables of the chains in the handle were built in the current mode: it cannot change under them
+    if (h->models_set) { set_error("mq_set_tables: call it before mq_set_models / mq_init_chains / mq_state_load"); return MQ_ERR_STATE; }
+    h->tables_mode = mode;
+    return MQ_OK;
+}
+
 extern "C" int mq_get_table(mq_handle* hh, int chain, int phase, float* ttt)
 {
     if (!hh || !ttt || chain < 0 || chain >= hh->h.n || (phase != 1 && phase != 2)) { set_error("mq_get_table: bad argument"); return MQ_ERR_ARG; }
     Handle* h = &hh->h;
+    if (h->tables_mode == MQ_TABLES_RECIPROCAL && h->cfg.eikonal == 1 && h->cfg.aflag != 1) {
+        set_error("mq_get_table: the handle builds reciprocal tables (mq_set_tables); no parity table exists, mq_get_rows reads the stored rows");
+        return MQ_ERR_UNSUPPORTED;
+    }
     if (!h->models_set) { set_error("mq_get_table: no models"); return MQ_ERR_STATE; }
     MQ_CUDA(cudaSetDevice(h->device));
     cudaStream_t s = h->stream;
@@ -636,7 +657,8 @@ extern "C" int mq_profile(mq_handle* hh, int enable, double* eikonal_ms, int64_t
     profile_enable(h, enable != 0);
     if (eikonal_ms) *eikonal_ms = ms;
     if (eikonal_launches) *eikonal_launches = n;
-    if (solves_per_full_launch) *solves_per_full_launch = (int64_t)2 * h->n * h->nz;
+    if (solves_per_full_launch)
+        *solves_per_full_launch = (int64_t)2 * h->n * (h->tables_mode == MQ_TABLES_RECIPROCAL ? h->n_rows : h->nz);
     return MQ_OK;
 }
 

@@ -62,6 +62,12 @@ __device__ __forceinline__ void tmem_wait_ld(float (&a)[4], float (&b)[4])
     asm volatile("tcgen05.wait::ld.sync.aligned;"
                  : "+f"(a[0]), "+f"(a[1]), "+f"(a[2]), "+f"(a[3]), "+f"(b[0]), "+f"(b[1]), "+f"(b[2]), "+f"(b[3])::"memory");
 }
+__device__ __forceinline__ void tmem_wait_ld(float (&a)[4][4])
+{
+    asm volatile("tcgen05.wait::ld.sync.aligned;"
+                 : "+f"(a[0][0]), "+f"(a[0][1]), "+f"(a[0][2]), "+f"(a[0][3]), "+f"(a[1][0]), "+f"(a[1][1]), "+f"(a[1][2]), "+f"(a[1][3]),
+                   "+f"(a[2][0]), "+f"(a[2][1]), "+f"(a[2][2]), "+f"(a[2][3]), "+f"(a[3][0]), "+f"(a[3][1]), "+f"(a[3][2]), "+f"(a[3][3])::"memory");
+}
 __device__ __forceinline__ void tmem_wait_ld(float& a) { asm volatile("tcgen05.wait::ld.sync.aligned;" : "+f"(a)::"memory"); }
 __device__ __forceinline__ void tmem_st4(uint32_t taddr, const float (&v)[4])
 {

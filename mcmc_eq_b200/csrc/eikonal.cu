@@ -24,6 +24,37 @@ size_t eik_scratch_floats_per_warp(int nxmod, int nz)
     return ((size_t)nxmod * nz + kFineNodes) * 32;
 }
 
+// Solve g of a batch: its source depth, its slowness column (item), where its output starts in the item's table and the
+// stride between its output rows (b.rows[r] goes to out_off + r*out_rstride).  Table mode decodes g as parity or, with
+// src_rows, reciprocal tables (EikBatch::src_rows); list mode takes src_iz[g] and column g.
+struct TableSolve {
+    int iz, item;
+    size_t out_off;
+    long out_rstride;
+};
+__device__ __forceinline__ TableSolve table_solve(const EikBatch& b, int n_items, int g)
+{
+    TableSolve t;
+    if (b.src_iz) {
+        t.iz = b.src_iz[g];
+        t.item = g;
+        t.out_off = (size_t)t.iz * b.xpitch;
+        t.out_rstride = (long)b.nz * b.xpitch;
+    } else if (b.src_rows) {
+        const int rho = g / n_items;
+        t.item = g - rho * n_items;
+        t.iz = b.src_rows[rho];
+        t.out_off = (size_t)rho * b.n_rows * b.xpitch;
+        t.out_rstride = b.xpitch;
+    } else {
+        t.iz = g / n_items;
+        t.item = g - t.iz * n_items;
+        t.out_off = (size_t)t.iz * b.xpitch;
+        t.out_rstride = (long)b.nz * b.xpitch;
+    }
+    return t;
+}
+
 // Generic kernel: the whole time field of a lane lives in global memory, interleaved by
 // lane (node i of lane l at scratch[i*32 + l]) so that lanes that sweep the same node
 // -- the common case, all lanes of a warp share the source depth -- touch one 128-byte line.
@@ -38,15 +69,14 @@ eik_generic_kernel(EikBatch b)
     float* W = b.scratch + (size_t)warp * (((size_t)nodes + kFineNodes) * 32) + lane;
     float* WF = W + (size_t)nodes * 32;
     const int n_items = b.n_items_dev ? *b.n_items_dev : b.n_items;
-    const int n_solves = b.src_iz ? b.n_solves : n_items * b.nz;
+    const int n_solves = b.src_iz ? b.n_solves : n_items * eik_sources(b);
     const int n_tasks = (n_solves + 31) >> 5;
 
     for (int task = warp; task < n_tasks; task += n_warps) {
         const int g = task * 32 + lane;
         if (g < n_solves) {
-            int iz, item;
-            if (b.src_iz) { iz = b.src_iz[g]; item = g; }
-            else { iz = g / n_items; item = g - iz * n_items; }
+            const TableSolve ts = table_solve(b, n_items, g);
+            const int iz = ts.iz, item = ts.item;
             const float* s = b.slow + (size_t)item * b.nz;
             const int rc = eik::solve(s, 1, b.nxmod, b.nz, iz, W, WF, 32, nullptr);
             if (b.status) b.status[g] = rc;
@@ -56,10 +86,10 @@ eik_generic_kernel(EikBatch b)
                 for (int i = 0; i < nodes; i++) o[i] = W[(size_t)i * 32];
             }
             if (b.n_rows > 0 && (b.row_out || b.row_out_base)) {
-                float* tab = b.row_out ? b.row_out[item] : b.row_out_base + (size_t)item * b.row_item_stride;
+                float* tab = (b.row_out ? b.row_out[item] : b.row_out_base + (size_t)item * b.row_item_stride) + ts.out_off;
                 for (int r = 0; r < b.n_rows; r++) {
                     const int j = b.rows[r];
-                    float* o = tab + ((size_t)r * b.nz + iz) * b.xpitch;
+                    float* o = tab + (long)r * ts.out_rstride;
                     for (int x = 0; x < b.nxmod; x++) o[x] = W[((size_t)x * b.nz + j) * 32];
                 }
             }
@@ -70,7 +100,7 @@ eik_generic_kernel(EikBatch b)
 
 cudaError_t eik_launch_generic(const EikBatch& b, cudaStream_t stream)
 {
-    const int n_solves = b.src_iz ? b.n_solves : b.n_items * b.nz;   // upper bound when n_items_dev is set
+    const int n_solves = b.src_iz ? b.n_solves : b.n_items * eik_sources(b);   // upper bound when n_items_dev is set
     if (n_solves <= 0) return cudaSuccess;
     const int n_tasks = (n_solves + 31) / 32;
     const int warps = n_tasks < b.max_warps ? n_tasks : b.max_warps;
@@ -120,7 +150,7 @@ __device__ __forceinline__ void eik_fast_body(const EikBatch& b, const eikf::Dim
     L.W = b.scratch + (size_t)blockIdx.x * (((size_t)D.wx * D.nz + kFineNodes) * 32) + lane;
     L.WF = L.W + (size_t)D.wx * D.nz * 32;
     const int n_items = b.n_items_dev ? *b.n_items_dev : b.n_items;
-    const int n_solves = b.src_iz ? b.n_solves : n_items * b.nz;
+    const int n_solves = b.src_iz ? b.n_solves : n_items * eik_sources(b);
     const int n_tasks = (n_solves + lpt - 1) / lpt;
 
     for (int task = blockIdx.x; task < n_tasks; task += gridDim.x) {
@@ -131,14 +161,14 @@ __device__ __forceinline__ void eik_fast_body(const EikBatch& b, const eikf::Dim
         t.valid = g >= 0 && g < n_solves;
         t.iz = 0; t.slow = nullptr; t.out = nullptr; t.out_rstride = 0; t.full = nullptr; t.hand_col = nullptr; t.hand_x1 = nullptr;
         if (t.valid) {
-            int item;
-            if (b.src_iz) { t.iz = b.src_iz[g]; item = g; }
-            else { t.iz = g / n_items; item = g - t.iz * n_items; }
+            const TableSolve ts = table_solve(b, n_items, g);
+            t.iz = ts.iz;
+            const int item = ts.item;
             t.slow = b.slow + (size_t)item * b.nz;
             if (b.n_rows > 0 && (b.row_out || b.row_out_base)) {
                 float* tab = b.row_out ? b.row_out[item] : b.row_out_base + (size_t)item * b.row_item_stride;
-                t.out = tab + (size_t)t.iz * b.xpitch;
-                t.out_rstride = (long)b.nz * b.xpitch;
+                t.out = tab + ts.out_off;
+                t.out_rstride = ts.out_rstride;
             }
             if (b.full_out) t.full = b.full_out + (size_t)g * nodes;
         }
@@ -174,9 +204,10 @@ __global__ void eik_key_kernel(EikBatch b, int max_solves, uint64_t* keys, int32
     const int g = blockIdx.x * blockDim.x + threadIdx.x;
     if (g >= max_solves) return;
     const int n_items = b.n_items_dev ? *b.n_items_dev : b.n_items;
-    const int n_solves = n_items * b.nz;
+    const int n_solves = n_items * eik_sources(b);
     if (g >= n_solves) { keys[g] = ~0ull; vals[g] = -1; return; }
-    const int iz = g / n_items, item = g - iz * n_items;
+    const TableSolve ts = table_solve(b, n_items, g);
+    const int iz = ts.iz, item = ts.item;
     const float* s = b.slow + (size_t)item * b.nz;
     const int my = b.nz - 1;
     const int ysc = (iz == my) ? iz - 1 : iz;
@@ -220,7 +251,7 @@ size_t eik_order_bytes(int max_solves)
 
 cudaError_t eik_order_tasks(const EikBatch& b, int32_t* order, void* work, size_t work_bytes, cudaStream_t stream)
 {
-    const int max_solves = b.n_items * b.nz;
+    const int max_solves = b.n_items * eik_sources(b);
     if (max_solves <= 0) return cudaSuccess;
     const size_t n = ((size_t)max_solves + 31) / 32 * 32;
     char* w = (char*)work;
@@ -321,9 +352,10 @@ __device__ __forceinline__ void pipe_release(unsigned* mask, int bit, int lane)
     if (lane == 0) { __threadfence_block(); atomicOr(mask, 1u << bit); }
 }
 
-// CA: nodes -1 .. CA-2 per TMEM column array (nz <= CA - 2); WARPS: warps per CTA
-template <int CA, int WARPS>
-__global__ void __launch_bounds__(WARPS * 32, 1) eik_pipe_kernel(EikBatch b, eikf::Dims D, int n_slices, int* task_counter)
+// CA: nodes -1 .. CA-2 per TMEM column array (nz <= CA - 2); WARPS: warps per CTA; RECIP: reciprocal tables
+// (EikBatch::src_rows, with rows = 0 .. nz-1): every row of each column is output.
+template <int CA, int WARPS, bool RECIP>
+__device__ __forceinline__ void eik_pipe_body(const EikBatch& b, const eikf::Dims& D, int n_slices, int* task_counter)
 {
     constexpr int NB = CA / 4;
     constexpr int kSets = 512 / (3 * CA);        // TMEM sets per lane quarter: 2 at CA = 64, 1 at CA = 128
@@ -346,7 +378,7 @@ __global__ void __launch_bounds__(WARPS * 32, 1) eik_pipe_kernel(EikBatch b, eik
     float* tieS = tieC + (size_t)CA * 32 + 32;                             // cell k at tieS[k*32], k = -2 .. CA-1
     const int nz = b.nz, ke = nz - 1, mx = b.nxmod - 1;
     const int n_items = b.n_items_dev ? *b.n_items_dev : b.n_items;
-    const int n_solves = n_items * nz;
+    const int n_solves = n_items * (RECIP ? b.n_src_rows : nz);
     const int n_tasks = (n_solves + 31) >> 5;
     const size_t wfloats = ((size_t)D.wx * D.nz + kFineNodes) * 32;
     float* Wbase = b.scratch + (size_t)(blockIdx.x * WARPS + warp) * wfloats + lane;
@@ -371,12 +403,13 @@ __global__ void __launch_bounds__(WARPS * 32, 1) eik_pipe_kernel(EikBatch b, eik
         t.hand_col = L.COL;          // the last column of the box phase already sits there
         t.hand_x1 = nullptr;         // set inside solve_warp_call
         if (t.valid) {
-            t.iz = g / n_items;
-            const int item = g - t.iz * n_items;
+            // table_solve with the mode known at compile time (no list mode here)
+            const int s = g / n_items, item = g - s * n_items;
+            t.iz = RECIP ? b.src_rows[s] : s;
             t.slow = b.slow + (size_t)item * nz;
             float* tab = b.row_out ? b.row_out[item] : b.row_out_base + (size_t)item * b.row_item_stride;
-            t.out = tab + (size_t)t.iz * b.xpitch;
-            t.out_rstride = (long)nz * b.xpitch;
+            t.out = tab + (RECIP ? (size_t)s * nz * b.xpitch : (size_t)s * b.xpitch);
+            t.out_rstride = RECIP ? (long)b.xpitch : (long)nz * b.xpitch;
         }
         const int rc = solve_warp_call(D, L, t, b.rows, b.n_rows, &x1);
         if (t.valid && b.status_min && rc < 0) atomicMin(b.status_min, rc);
@@ -455,10 +488,31 @@ __global__ void __launch_bounds__(WARPS * 32, 1) eik_pipe_kernel(EikBatch b, eik
                 }
             }
             eikm::tmem_wait_st();
-            for (int r = 0; r < b.n_rows; r++) {
-                float v = eikm::tmem_ld1(tc + b.rows[r] + 1);
-                eikm::tmem_wait_ld(v);
-                if (need) t.out[(long)r * t.out_rstride + line] = v;
+            if (RECIP) {
+                // every row of the column: .x4 loads of four groups (16 nodes) and one wait per four groups (groups
+                // 4q0 .. 4q0+3 never pass group NB-1: NB is a multiple of four)
+                const int q_end = (ke + 1) / 4 + 1;      // node ke is in group (ke + 1) / 4
+                for (int q0 = 0; q0 < q_end; q0 += 4) {
+                    float v[4][4];
+#pragma unroll
+                    for (int u = 0; u < 4; u++) eikm::tmem_ld4(tc + 4 * (q0 + u), v[u]);
+                    eikm::tmem_wait_ld(v);
+                    if (need) {
+#pragma unroll
+                        for (int u = 0; u < 4; u++)
+#pragma unroll
+                            for (int c = 0; c < 4; c++) {
+                                const int k = 4 * (q0 + u) - 1 + c;
+                                if (k >= 0 && k <= ke) t.out[(long)k * t.out_rstride + line] = v[u][c];
+                            }
+                    }
+                }
+            } else {
+                for (int r = 0; r < b.n_rows; r++) {
+                    float v = eikm::tmem_ld1(tc + b.rows[r] + 1);
+                    eikm::tmem_wait_ld(v);
+                    if (need) t.out[(long)r * t.out_rstride + line] = v;
+                }
             }
             const uint32_t tt = tp; tp = tc; tc = tt;
         }
@@ -467,6 +521,18 @@ __global__ void __launch_bounds__(WARPS * 32, 1) eik_pipe_kernel(EikBatch b, eik
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
     if (warp == 0) eikm::tmem_dealloc<512>(ctl.tmem);
+}
+
+template <int CA, int WARPS>
+__global__ void __launch_bounds__(WARPS * 32, 1) eik_pipe_kernel(EikBatch b, eikf::Dims D, int n_slices, int* task_counter)
+{
+    eik_pipe_body<CA, WARPS, false>(b, D, n_slices, task_counter);
+}
+// The reciprocal-table instantiation (a kernel of its own name: the parity kernel's code stays as it is)
+template <int CA, int WARPS>
+__global__ void __launch_bounds__(WARPS * 32, 1) eik_pipe_recip_kernel(EikBatch b, eikf::Dims D, int n_slices, int* task_counter)
+{
+    eik_pipe_body<CA, WARPS, true>(b, D, n_slices, task_counter);
 }
 
 bool eik_pipe_supported(int nxmod, int nz)
@@ -482,9 +548,12 @@ bool eik_pipe_supported(int nxmod, int nz)
 cudaError_t eik_launch_pipe(const EikBatch& b, int* task_counter, cudaStream_t stream)
 {
     if (b.src_iz || b.full_out || !task_counter || !b.tie_scratch) return cudaErrorInvalidValue;
+    if (b.src_rows && b.n_rows != b.nz) return cudaErrorInvalidValue;   // the reciprocal march stores every row
     const PipeShape sh = pipe_shape(b.nz);
     if (!sh.ca) return cudaErrorInvalidValue;
-    void (*const kernel)(EikBatch, eikf::Dims, int, int*) = sh.ca == 64 ? eik_pipe_kernel<64, kPipeWarps> : eik_pipe_kernel<128, kPipeWarpsDeep>;
+    void (*const kernel)(EikBatch, eikf::Dims, int, int*) =
+        b.src_rows ? (sh.ca == 64 ? eik_pipe_recip_kernel<64, kPipeWarps> : eik_pipe_recip_kernel<128, kPipeWarpsDeep>)
+                     : (sh.ca == 64 ? eik_pipe_kernel<64, kPipeWarps> : eik_pipe_kernel<128, kPipeWarpsDeep>);
     eikf::Dims D = fast_dims(b.nxmod, b.nz);
     // Lock-step columns in the box phase (a second column buffer per slice: 7 slices instead of 9 on the Example plane).
     // Kernel ms per launch at 1024 / 2048 / 4096 / 8192 chains with the box phase inlined: 7.70 / 13.99 / 26.42 / 51.07
@@ -500,14 +569,14 @@ cudaError_t eik_launch_pipe(const EikBatch& b, int* task_counter, cudaStream_t s
     if (n_slices < 2) return cudaErrorInvalidValue;
     const size_t smem = (size_t)n_slices * slice;
     // per instantiation and device: largest dynamic shared-memory size the kernel has been opted in for
-    static size_t configured[2][64] = {};
-    size_t* conf = (dev >= 0 && dev < 64) ? &configured[sh.ca == 128][dev] : nullptr;
+    static size_t configured[4][64] = {};
+    size_t* conf = (dev >= 0 && dev < 64) ? &configured[(sh.ca == 128) * 2 + (b.src_rows ? 1 : 0)][dev] : nullptr;
     if (!conf || smem > *conf) {
         cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
         if (conf) *conf = smem;
     }
-    const int n_tasks = (b.n_items * b.nz + 31) / 32;
+    const int n_tasks = (b.n_items * eik_sources(b) + 31) / 32;
     // per-warp global window: the scratch was sized for max_warps warps of the generic kernel
     const size_t have = (size_t)b.max_warps * eik_scratch_floats_per_warp(b.nxmod, b.nz);
     const long warps_by_scratch = (long)(have / fast_scratch_floats_per_warp(D));
@@ -543,7 +612,7 @@ int eik_fast_max_warps(int nxmod, int nz, int device)
 
 cudaError_t eik_launch_fast(const EikBatch& b, cudaStream_t stream)
 {
-    const int n_solves = b.src_iz ? b.n_solves : b.n_items * b.nz;
+    const int n_solves = b.src_iz ? b.n_solves : b.n_items * eik_sources(b);
     if (n_solves <= 0) return cudaSuccess;
     const eikf::Dims D = fast_dims(b.nxmod, b.nz);
     const size_t smem = fast_smem_floats_per_warp(D) * sizeof(float);
@@ -584,7 +653,7 @@ size_t eik_fine_slice_floats_per_warp(int nxmod, int nz)
 
 cudaError_t eik_launch_fine(const EikBatch& b, cudaStream_t stream)
 {
-    const int n_solves = b.src_iz ? b.n_solves : b.n_items * b.nz;
+    const int n_solves = b.src_iz ? b.n_solves : b.n_items * eik_sources(b);
     if (n_solves <= 0) return cudaSuccess;
     if (!b.slice_scratch) return cudaErrorInvalidValue;
     const eikf::Dims D = fast_dims(b.nxmod, b.nz);
@@ -609,11 +678,12 @@ cudaError_t eik_launch(const EikBatch& b, cudaStream_t stream, int* which)
         const char* e = getenv("MCMCEQ_EIKONAL");
         force_generic = (e && strcmp(e, "generic") == 0) ? 1 : 0;
     }
-    if (!force_generic && b.task_counter && b.tie_scratch && !b.src_iz && !b.full_out && eik_pipe_supported(b.nxmod, b.nz)) {
+    if (!force_generic && b.task_counter && b.tie_scratch && !b.src_iz && !b.full_out && (!b.src_rows || b.n_rows == b.nz) &&
+        eik_pipe_supported(b.nxmod, b.nz)) {
         // worth it (and the per-warp scratch windows suffice) only when there is work for every warp of every SM
         const eikf::Dims D = fast_dims(b.nxmod, b.nz);
         const size_t have = (size_t)b.max_warps * eik_scratch_floats_per_warp(b.nxmod, b.nz);
-        const long n_tasks = ((long)b.n_items * b.nz + 31) / 32;
+        const long n_tasks = ((long)b.n_items * eik_sources(b) + 31) / 32;
         int dev = 0, sms = 148;
         cudaGetDevice(&dev);
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);

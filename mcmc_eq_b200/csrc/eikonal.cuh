@@ -20,7 +20,7 @@ struct EikBatch {
                                 // (n_items is then the upper bound the grid is sized for)
     const int32_t* src_iz;    // [n_solves] device or nullptr
     int n_solves;
-    // Table mode only: optional execution order.  order[j] = the solve (iz * n_items + item) that lane j % 32 of warp
+    // Table mode only: optional execution order.  order[j] = the solve g (source * n_items + item) that lane j % 32 of warp
     // task j / 32 runs, or -1 (eik_order_tasks fills it: solves of one source depth that initialise and grow their
     // boxes alike are made neighbours so that the lanes of a warp stay in step).
     const int32_t* order;
@@ -35,6 +35,14 @@ struct EikBatch {
     size_t row_item_stride;
     const int32_t* rows;      // [n_rows] device: grid rows (receiver layers) that are kept
     int n_rows, xpitch;
+    // Table mode only: reciprocal tables.  When non-null the sources of an item sit at the n_src_rows grid rows src_rows[rho]
+    // instead of at every depth: n_solves = n_items*n_src_rows, solve g -> rho = g / n_items, item = g % n_items, and its
+    // kept rows go to block rho of the item's table, row r at (rho*n_rows + r)*xpitch.  With rows = 0 .. nz-1 (the handle's
+    // reciprocal mode) that is the [n_src_rows][nz][xpitch] layout of the parity table with its receiver-row and
+    // source-depth axes swapped: t[x][y] of the source at row src_rows[rho] where parity has the time from (0, y) to
+    // (x, src_rows[rho]) (by reciprocity T(a -> b) ~ T(b -> a)).  The pipelined kernel requires rows = 0 .. nz-1 then.
+    const int32_t* src_rows;
+    int n_src_rows;
     int32_t* status;          // [n_solves] device or nullptr
     int32_t* status_min;      // [1] device or nullptr: atomicMin of every solve's status
     // Scratch: per resident warp (nxmod*nz + kFineNodes) * 32 floats.
@@ -46,6 +54,9 @@ struct EikBatch {
 };
 
 constexpr int kFineNodes = 22 * 43;   // refined grid of a left-edge source, src/time_2d.c:844-864
+
+// Solves per item of a table-mode batch: one per depth (parity) or one per receiver row (reciprocal).
+__host__ __device__ inline int eik_sources(const EikBatch& b) { return b.src_rows ? b.n_src_rows : b.nz; }
 
 size_t eik_scratch_floats_per_warp(int nxmod, int nz);
 // Generic one-lane-per-solve kernel, time field in global memory.

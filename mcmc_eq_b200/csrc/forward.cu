@@ -180,6 +180,11 @@ cudaError_t launch_tables(Handle* h, int max_items)
     b.nxmod = h->nxmod; b.nz = h->nz;
     b.slow = h->slow; b.n_items = max_items; b.n_items_dev = h->n_items;
     b.row_out = h->item_tab; b.rows = h->d_rows; b.n_rows = h->n_rows; b.xpitch = h->xp;
+    if (h->tables_mode == MQ_TABLES_RECIPROCAL) {
+        // sources at the receiver rows, every row of their fields kept
+        b.src_rows = h->d_rows; b.n_src_rows = h->n_rows;
+        b.rows = h->d_all_rows; b.n_rows = h->nz;
+    }
     b.status_min = h->solve_status;
     b.scratch = h->scratch; b.max_warps = h->scratch_warps; b.slice_scratch = h->eik_slice_scratch;
     if (h->eik_order) {

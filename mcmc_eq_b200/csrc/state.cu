@@ -239,6 +239,9 @@ inline size_t up8(size_t x) { return (x + 7) / 8 * 8; }
 
 bool has_tables(const Handle* h) { return h->cfg.eikonal == 1 && h->cfg.aflag != 1; }
 
+// reciprocal tables are part of a state's identity only where tables exist
+bool reciprocal_tables(const Handle* h) { return has_tables(h) && h->tables_mode == MQ_TABLES_RECIPROCAL; }
+
 // the sections of a blob with the given options; the header's identity fields from the handle
 void make_plan(const Handle* h, bool post, bool beta, bool tables, bool diag, Plan* P)
 {
@@ -252,7 +255,8 @@ void make_plan(const Handle* h, bool post, bool beta, bool tables, bool diag, Pl
     H.nz = h->nz; H.nxmod = h->nxmod; H.n_rows = h->n_rows;
     H.config_sum = config_checksum(&h->cfg);
     H.picks_sum = h->picks_sum;
-    H.flags = (post ? MQ_STATE_POSTERIOR : 0) | (beta ? MQ_STATE_BETA : 0) | (tables ? MQ_STATE_TABLES : 0) | (diag ? MQ_STATE_DIAG : 0);
+    H.flags = (post ? MQ_STATE_POSTERIOR : 0) | (beta ? MQ_STATE_BETA : 0) | (tables ? MQ_STATE_TABLES : 0) | (diag ? MQ_STATE_DIAG : 0) |
+              (tables && reciprocal_tables(h) ? MQ_STATE_RECIPROCAL : 0);
     const size_t n = h->n;
     P->rec_bytes = chain_bytes(h->md, h->ne, h->ns);
     size_t off = 0;
@@ -431,8 +435,14 @@ extern "C" int mq_state_load(mq_handle* hh, const void* buf, uint64_t bytes)
     if (H.picks_sum != h->picks_sum) { set_error("mq_state_load: the state was saved with other picks"); return MQ_ERR_ARG; }
     const bool post = (H.flags & MQ_STATE_POSTERIOR) != 0, beta = (H.flags & MQ_STATE_BETA) != 0, tables = (H.flags & MQ_STATE_TABLES) != 0;
     const bool diag = (H.flags & MQ_STATE_DIAG) != 0;
-    if ((H.flags & ~(uint32_t)(MQ_STATE_POSTERIOR | MQ_STATE_BETA | MQ_STATE_TABLES | MQ_STATE_DIAG)) || tables != has_tables(h)) {
+    if ((H.flags & ~(uint32_t)(MQ_STATE_POSTERIOR | MQ_STATE_BETA | MQ_STATE_TABLES | MQ_STATE_DIAG | MQ_STATE_RECIPROCAL)) ||
+        tables != has_tables(h)) {
         set_error("mq_state_load: flags 0x%x do not fit the handle", H.flags);
+        return MQ_ERR_ARG;
+    }
+    if (((H.flags & MQ_STATE_RECIPROCAL) != 0) != reciprocal_tables(h)) {
+        set_error("mq_state_load: the state was saved with %s tables, the handle builds %s tables (mq_set_tables)",
+                  (H.flags & MQ_STATE_RECIPROCAL) ? "reciprocal" : "parity", reciprocal_tables(h) ? "reciprocal" : "parity");
         return MQ_ERR_ARG;
     }
     int ndv = 0, ndvpvs = 0;

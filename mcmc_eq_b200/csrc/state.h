@@ -7,7 +7,8 @@
 //   eq        [n][ne][3]   pres/sres [n][ns]   noise [n][8]
 //   tables    [2][n][2 phases][R][nz][xp]               double-buffered per chain AND phase: tcur[2c+ph]
 //             only the receiver rows the misfit can ever read are kept (reference keeps all nz rows,
-//             src/misfit.c:281-288; the values are the same, SURVEY.md section 7 H2-v)
+//             src/misfit.c:281-288; the values are the same, SURVEY.md section 7 H2-v); with reciprocal tables
+//             (mq_set_tables) [R][nz][xp] is the field of a source at receiver row R read at every depth instead
 //   evsum     [2][n][ne][8], origin [2][n][ne]          per-event class sums; ecur[c] = current buffer
 //   mf [n][8], ll/rms/misfit [n] (double)               current likelihood
 //
@@ -99,10 +100,12 @@ struct Handle {
     uint64_t seed;
     uint64_t picks_sum;  // checksum of the picks as mq_create received them (state.cu: a saved state belongs to them)
     bool models_set, forward_done;
+    int tables_mode;     // MQ_TABLES_PARITY or MQ_TABLES_RECIPROCAL (mq_set_tables): how table rebuilds solve (eikonal.cuh)
 
     DevPicks pk;
     int32_t* d_rows;     // [n_rows] kept grid rows
     int32_t* rows_host;  // [n_rows] (malloc)
+    int32_t* d_all_rows; // [nz] 0 .. nz-1: the rows a reciprocal table rebuild keeps
 
     // chain state
     int32_t *dim, *mcur, *tcur, *ecur;

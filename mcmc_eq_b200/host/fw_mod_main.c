@@ -1,7 +1,7 @@
 /* fw_mod_main.c -- the reference's forward programs `fw_mod` and `fw` on top of the B200 library (plain C over the C ABI).
  *
- *     fw_mod <config_eqx.dat> <model_block> <picks> [-d device]
- *     fw     <config.dat>     <res.dat>     <picks> [-d device]        (this file compiled with -DFW_GRIDDED)
+ *     fw_mod <config_eqx.dat> <model_block> <picks> [-d device] [-x]
+ *     fw     <config.dat>     <res.dat>     <picks> [-d device] [-x]   (this file compiled with -DFW_GRIDDED)
  *
  * Arguments as the reference's.  fw_mod (src/fw_mod.c): <model_block> is one record cut from a chain file: the "mod ..."
  * line (src/fw_mod.c:421-445), then one "EQ ..." line per event (:450-457) and one "RES ..." line per station (:460-464).
@@ -14,6 +14,8 @@
  *     residual dist z origin t_observed t_predicted P|S
  * and on stderr "Start model found with loglikelihood ... RMS=..." (src/fw_mod.c:480).  make_synthetics / mkSynthetics.sh /
  * disp_msft_dist.sh use exactly these lines.
+ * -x: the same forward with reciprocal travel-time tables (mq_set_tables, MQ_TABLES_RECIPROCAL; one stderr line says so).
+ * Comparing the output with and without -x on one's own picks shows what the mode costs per pick on that data.
  */
 #include <math.h>
 #include <stdio.h>
@@ -31,7 +33,7 @@ static float dst(float x1, float x2, float y1, float y2) { return (float)sqrt(((
 
 int main(int argc, char** argv)
 {
-    int rc = 0, device = 0, i, j, dim = 0, ne, ns, np;
+    int rc = 0, device = 0, i, j, dim = 0, ne, ns, np, reciprocal = 0;
     mq_config cfg;
     mqio_picks pk;
     mq_handle* h = NULL;
@@ -46,9 +48,11 @@ int main(int argc, char** argv)
 
     memset(&pk, 0, sizeof pk);
     memset(&m, 0, sizeof m);
-    if (argc < 4) { fprintf(stderr, "usage: %s config.dat model picks [-d device]\n", argv[0]); return 2; }
-    for (i = 4; i + 1 < argc; i++)
-        if (!strcmp(argv[i], "-d")) device = atoi(argv[++i]);
+    if (argc < 4) { fprintf(stderr, "usage: %s config.dat model picks [-d device] [-x]\n", argv[0]); return 2; }
+    for (i = 4; i < argc; i++) {
+        if (!strcmp(argv[i], "-d") && i + 1 < argc) device = atoi(argv[++i]);
+        else if (!strcmp(argv[i], "-x")) reciprocal = 1;
+    }
     if (mqio_read_config(argv[1], &cfg) != MQ_OK) FAIL("%s", mqio_last_error());
     if (mqio_read_picks(argv[3], &pk) != MQ_OK) FAIL("%s", mqio_last_error());
     ne = pk.view.n_events; ns = pk.view.n_stations; np = pk.view.n_picks;
@@ -126,6 +130,10 @@ int main(int argc, char** argv)
 #endif
     if (cfg.max_dim < dim) cfg.max_dim = dim;      /* the reference's forward programs do not look at line 8 */
     MQ(mq_create(&cfg, &pk.view, 1, device, 1, &h));
+    if (reciprocal) {
+        MQ(mq_set_tables(h, MQ_TABLES_RECIPROCAL));
+        fprintf(stderr, "reciprocal travel-time tables (-x): sources at the receiver rows, not the parity forward\n");
+    }
     dim32 = dim;
     m.n_chains = 1; m.max_dim = dim; m.n_events = ne; m.n_stations = ns;
     m.dim = &dim32; m.z = z; m.vp = vp; m.vpvs = vpvs; m.eq = eq; m.pres = pres; m.sres = sres; m.noise = noise; m.origin = origin;

@@ -1,7 +1,7 @@
 /* mcmc_eq_main.c -- the reference's command line on top of the B200 library (plain C host code, C ABI only).
  *
  *     mcmc_eq <config_eqx.dat> <out> <picks> [-n chains] [-d device] [-s seed] [-r slots] [-q]
- *             [-k checkpoint [-K minutes]] [-R checkpoint] [-D diagnostics]
+ *             [-k checkpoint [-K minutes]] [-R checkpoint] [-D diagnostics] [-x]
  *
  * The first three arguments are the reference's (src/mcmc_eq.c:332-338; it ignores anything after them).
  * With one chain (the default) <out> is written exactly like the reference writes it: a "sta ST" record, a
@@ -38,6 +38,11 @@
  * one line per quantity "name index n_models mean sd rhat ess" (names rms dim noise vp vpvs x y z t pres sres), plus one
  * stderr line with the largest R-hat and the smallest ESS and where they occur.  The accumulators are part of the
  * checkpoint: under -R they continue, and -D with a checkpoint that has none fails before any chain file is touched.
+ *
+ * Reciprocal tables: -x builds the travel-time tables with the source at each receiver row instead of at each event depth
+ * (mq_set_tables, MQ_TABLES_RECIPROCAL): n_rows solves per table instead of nz, at the price of the finite-difference
+ * scheme's reciprocity error in every prediction (DESIGN.md section 6).  One stderr line says so.  Under -R the mode is the
+ * checkpoint's (its state flags); -x against a checkpoint written with parity tables fails before any chain file is touched.
  *
  * Unlike the reference (which exit(0)s on every error) the exit status is non-zero on failure.
  */
@@ -374,7 +379,7 @@ static double now_s(void)
 
 int main(int argc, char** argv)
 {
-    int rc = 0, n_chains = 1, device = 0, quiet = 0, i, c, from_file = 0, ring = 0, writer_on = 0, n_given = 0;
+    int rc = 0, n_chains = 1, device = 0, quiet = 0, i, c, from_file = 0, ring = 0, writer_on = 0, n_given = 0, reciprocal = 0;
     const char *ck_path = NULL, *resume_path = NULL, *diag_path = NULL;
     int64_t diag_burn_in = 0;
     int32_t diag_batches = 16;
@@ -399,7 +404,7 @@ int main(int argc, char** argv)
     memset(&ck, 0, sizeof ck);
     if (argc < 4) {
         fprintf(stderr, "usage: %s config_eqx.dat outfile picks [-n chains] [-d device] [-s seed] [-r ring slots] [-q] "
-                        "[-k checkpoint [-K minutes]] [-R checkpoint] [-D diagnostics]\n", argv[0]);
+                        "[-k checkpoint [-K minutes]] [-R checkpoint] [-D diagnostics] [-x]\n", argv[0]);
         return 2;
     }
     if ((env = getenv("MCMCEQ_CHAINS")) != NULL) { n_chains = atoi(env); n_given = 1; }
@@ -414,6 +419,7 @@ int main(int argc, char** argv)
         else if (!strcmp(argv[i], "-s") && i + 1 < argc) seed_arg = atol(argv[++i]);
         else if (!strcmp(argv[i], "-r") && i + 1 < argc) ring = atoi(argv[++i]);
         else if (!strcmp(argv[i], "-q")) quiet = 1;
+        else if (!strcmp(argv[i], "-x")) reciprocal = 1;
         /* anything else is ignored, as the reference ignores extra arguments */
     }
     if (n_chains < 1) n_chains = 1;
@@ -425,6 +431,12 @@ int main(int argc, char** argv)
         n_chains = ck.head.n_chains;
         if (diag_path && state_diag_params(ck.state, ck.head.state_bytes, &diag_burn_in, &diag_batches))
             FAIL("-D: the checkpoint %s holds no diagnostics (the run was started without -D)", resume_path);
+        {   /* the table mode is the checkpoint's; a state without tables (eikonal == 0, aflag == 1) has none */
+            const uint32_t flags = ((const mq_state_header*)ck.state)->flags;
+            if (reciprocal && (flags & MQ_STATE_TABLES) && !(flags & MQ_STATE_RECIPROCAL))
+                FAIL("-x: the checkpoint %s was written with parity tables (the run was started without -x)", resume_path);
+            if (flags & MQ_STATE_RECIPROCAL) reciprocal = 1;
+        }
     }
 
     if (mqio_read_config(argv[1], &cfg) != MQ_OK) FAIL("%s", mqio_last_error());
@@ -439,6 +451,10 @@ int main(int argc, char** argv)
         if (!quiet) fprintf(stderr, "%d chain(s) on device %d, seed %lu, %d events, %d stations, %d picks\n", n_chains, device, seed,
                             pk.view.n_events, pk.view.n_stations, pk.view.n_picks);
         MQ(mq_create(&cfg, &pk.view, n_chains, device, (uint64_t)seed, &h));
+        if (reciprocal) {
+            MQ(mq_set_tables(h, MQ_TABLES_RECIPROCAL));
+            fprintf(stderr, "reciprocal travel-time tables (-x): sources at the receiver rows, not the parity forward\n");
+        }
         if (ring > 0) MQ(mq_set_ring(h, ring));
         if (resume_path) MQ(mq_state_load(h, ck.state, ck.head.state_bytes));
         else if (diag_path) {   /* the models of the start phase are burn-in */
