@@ -109,7 +109,8 @@ extern "C" int mq_destroy(mq_handle* hh)
     free_view(&h->cur_view); free_view(&h->prop_view);
     cudaFree(h->evq); cudaFree(h->oq); cudaFree(h->mf_eval); cudaFree(h->resid); cudaFree(h->tpred);
     cudaFree(h->item_chain); cudaFree(h->item_phase); cudaFree(h->n_items); cudaFree(h->slow); cudaFree(h->item_tab);
-    cudaFree(h->solve_status); cudaFree(h->scratch); cudaFree(h->eik_slice_scratch); cudaFree(h->eik_order); cudaFree(h->eik_order_work); cudaFree(h->eik_task_counter); cudaFree(h->eik_tie_scratch);
+    cudaFree(h->solve_status);
+    eik_work_free(&h->eik);
     if (h->host_flags) cudaFreeHost(h->host_flags);
     if (h->flags_ev) cudaEventDestroy(h->flags_ev);
     for (int i = 0; i < 2; i++)
@@ -253,41 +254,7 @@ extern "C" int mq_create(const mq_config* cfg, const mq_picks* pk, int n_chains,
     // h->resid ([n][np] per-pick scratch) is allocated by launch_misfit when it is first needed
     TRY(dalloc(&h->item_chain, 2 * n)); TRY(dalloc(&h->item_phase, 2 * n)); TRY(dalloc(&h->n_items, 1));
     TRY(dalloc(&h->slow, 2 * n * h->nz)); TRY(dalloc(&h->item_tab, 2 * n)); TRY(dalloc(&h->solve_status, 1));
-    {
-        // scratch of the generic eikonal kernel: enough warps for one full wave, never more than needed
-        int sms = 148;
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
-        const long need = ((long)2 * n * h->nz + 31) / 32;
-        const bool fine = !eik_fast_supported(h->nxmod, h->nz);
-        long warps = std::min<long>(need, (long)sms * (fine ? 12 : 16));
-        // large planes (the 0.1 km fine-grid case: 565 x 2001 nodes = 145 MB of window + 0.8 MB of slice per warp): never
-        // more than 70 % of the device memory that is still free (the tables are allocated); the kernels loop over the
-        // tasks with however many warps they are given.  MCMCEQ_SCRATCH_FRACTION overrides the fraction.
-        size_t free_b = 0, total_b = 0;
-        if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess) {
-            double frac = fine ? 0.7 : 0.25;
-            if (const char* e = getenv("MCMCEQ_SCRATCH_FRACTION")) { const double f = atof(e); if (f > 0.0 && f < 0.95) frac = f; }
-            const size_t per_warp = (eik_scratch_floats_per_warp(h->nxmod, h->nz) + (fine ? eik_fine_slice_floats_per_warp(h->nxmod, h->nz) : 0)) * sizeof(float);
-            const long by_mem = (long)(((double)free_b * frac) / (double)per_warp);
-            warps = std::min<long>(warps, std::max<long>(by_mem, 4));
-        }
-        warps = (warps + 3) / 4 * 4;
-        h->scratch_warps = (int)warps;
-        TRY(cudaMalloc(&h->scratch, (size_t)warps * eik_scratch_floats_per_warp(h->nxmod, h->nz) * sizeof(float)));
-        if (fine) TRY(cudaMalloc(&h->eik_slice_scratch, (size_t)warps * eik_fine_slice_floats_per_warp(h->nxmod, h->nz) * sizeof(float)));
-    }
-    {
-        // regrouping of the solves of a table rebuild
-        // (planes that do not fit a shared-memory slice keep the natural order: a chain's P and S solves of one source
-        //  depth are neighbours there, which is the grouping their long box phases want; measured, tools/fine_probe2.py)
-        if (eik_fast_supported(h->nxmod, h->nz)) {
-            const int max_solves = 2 * n_chains * h->nz;
-            h->eik_order_bytes = eik_order_bytes(max_solves);
-            TRY(cudaMalloc(&h->eik_order_work, h->eik_order_bytes));
-            TRY(cudaMalloc((void**)&h->eik_order, (((size_t)max_solves + 31) / 32 * 32) * sizeof(int32_t)));
-        }
-        if (eik_pipe_supported(h->nxmod, h->nz)) { TRY(dalloc(&h->eik_task_counter, 1)); TRY(dalloc(&h->eik_tie_scratch, eik_pipe_tie_floats(h->nz))); }
-    }
+    TRY(eik_work_alloc(&h->eik, h->nxmod, h->nz, 2 * n_chains * h->nz, true, device));
     TRY(cudaStreamSynchronize(s));
 #undef TRY
     *out = hh;
@@ -593,7 +560,8 @@ extern "C" int mq_get_table(mq_handle* hh, int chain, int phase, float* ttt)
     cudaStream_t s = h->stream;
     const int nz = h->nz, nx = h->nxmod;
     const size_t nodes = (size_t)nx * nz;
-    // slowness column of (chain, phase) via the regular rasteriser, then nz solves with full fields
+    // slowness column of (chain, phase) via the regular rasteriser, then a table-mode batch of that one column with full
+    // fields: solve g has its source at depth g and its field at d_out + g * nodes
     int32_t one = 1, ph = phase - 1;
     sync_cur_view<<<(h->n + 127) / 128, 128, 0, s>>>(h->n, h->mcur, h->tcur, h->ecur, h->cur_view);
     count_launch();
@@ -601,24 +569,17 @@ extern "C" int mq_get_table(mq_handle* hh, int chain, int phase, float* ttt)
     MQ_CUDA(h2d(h->item_chain, &chain, 1, s));
     MQ_CUDA(h2d(h->item_phase, &ph, 1, s));
     MQ_CUDA(launch_rasterise(h, h->cur_view, 1));
-    float *d_slow = nullptr, *d_out = nullptr;
-    int32_t* d_iz = nullptr;
-    std::vector<int32_t> iz(nz);
-    for (int i = 0; i < nz; i++) iz[i] = i;
-    MQ_CUDA(cudaMalloc(&d_slow, (size_t)nz * nz * sizeof(float)));
+    float* d_out = nullptr;
     MQ_CUDA(cudaMalloc(&d_out, (size_t)nz * nodes * sizeof(float)));
-    MQ_CUDA(cudaMalloc(&d_iz, nz * sizeof(int32_t)));
-    for (int i = 0; i < nz; i++) MQ_CUDA(cudaMemcpyAsync(d_slow + (size_t)i * nz, h->slow, nz * sizeof(float), cudaMemcpyDeviceToDevice, s));
-    MQ_CUDA(h2d(d_iz, iz.data(), nz, s));
     EikBatch b = {};
-    b.nxmod = nx; b.nz = nz; b.slow = d_slow; b.n_items = nz; b.src_iz = d_iz; b.n_solves = nz;
-    b.full_out = d_out; b.status_min = h->solve_status; b.scratch = h->scratch; b.max_warps = h->scratch_warps;
-    b.slice_scratch = h->eik_slice_scratch;
-    MQ_CUDA(eik_launch(b, s));
+    b.nxmod = nx; b.nz = nz; b.slow = h->slow; b.n_items = 1;
+    b.full_out = d_out; b.status_min = h->solve_status;
     std::vector<float> t((size_t)nz * nodes);
-    MQ_CUDA(d2h(t.data(), d_out, t.size(), s));
-    MQ_CUDA(cudaStreamSynchronize(s));
-    cudaFree(d_slow); cudaFree(d_out); cudaFree(d_iz);
+    cudaError_t e = eik_launch(b, h->eik, s);
+    if (e == cudaSuccess) e = d2h(t.data(), d_out, t.size(), s);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+    cudaFree(d_out);
+    MQ_CUDA(e);
     // ttt[j][iz][i] = t_iz[i*nz + j]   (src/misfit.c:281-288)
     for (int j = 0; j < nz; j++)
         for (int k = 0; k < nz; k++)

@@ -46,10 +46,10 @@ extern "C" int mq_eikonal_batch(const float* slow, const int32_t* src_iz, int n,
     const size_t nodes = (size_t)nxmod * nz;
     // bound the device footprint: process the batch in chunks
     const int chunk_max = 32 * 1024;
-    float *d_slow = nullptr, *d_out = nullptr, *d_scr = nullptr, *d_slice = nullptr;
+    float *d_slow = nullptr, *d_out = nullptr;
     int32_t *d_iz = nullptr, *d_st = nullptr;
+    EikWork work = {};
     const int chunk = n < chunk_max ? n : chunk_max;
-    const int max_warps = ((chunk + 31) / 32 + 3) / 4 * 4;
     int rc = MQ_OK;
     cudaError_t e;
 #define TRY(x) do { e = (x); if (e != cudaSuccess) { set_error("%s: %s", #x, cudaGetErrorString(e)); rc = MQ_ERR_CUDA; goto done; } } while (0)
@@ -57,17 +57,15 @@ extern "C" int mq_eikonal_batch(const float* slow, const int32_t* src_iz, int n,
     TRY(cudaMalloc(&d_iz, (size_t)chunk * sizeof(int32_t)));
     TRY(cudaMalloc(&d_st, (size_t)chunk * sizeof(int32_t)));
     TRY(cudaMalloc(&d_out, (size_t)chunk * nodes * sizeof(float)));
-    TRY(cudaMalloc(&d_scr, (size_t)max_warps * eik_scratch_floats_per_warp(nxmod, nz) * sizeof(float)));
-    // planes that do not fit a shared-memory slice keep their per-lane arrays in global memory (eik_fine_kernel)
-    if (!eik_fast_supported(nxmod, nz)) TRY(cudaMalloc(&d_slice, (size_t)max_warps * eik_fine_slice_floats_per_warp(nxmod, nz) * sizeof(float)));
+    TRY(eik_work_alloc(&work, nxmod, nz, chunk, false, device));
     for (int off = 0; off < n; off += chunk) {
         const int m = (n - off) < chunk ? (n - off) : chunk;
         TRY(cudaMemcpy(d_slow, slow + (size_t)off * nz, (size_t)m * nz * sizeof(float), cudaMemcpyHostToDevice));
         TRY(cudaMemcpy(d_iz, src_iz + off, (size_t)m * sizeof(int32_t), cudaMemcpyHostToDevice));
         EikBatch b = {};
         b.nxmod = nxmod; b.nz = nz; b.slow = d_slow; b.n_items = m; b.src_iz = d_iz; b.n_solves = m;
-        b.full_out = d_out; b.status = d_st; b.scratch = d_scr; b.max_warps = max_warps; b.slice_scratch = d_slice;
-        TRY(eik_launch(b, 0));
+        b.full_out = d_out; b.status = d_st;
+        TRY(eik_launch(b, work, 0));
         TRY(cudaDeviceSynchronize());
         TRY(cudaMemcpy(t_out + (size_t)off * nodes, d_out, (size_t)m * nodes * sizeof(float), cudaMemcpyDeviceToHost));
         std::vector<int32_t> st(m);
@@ -82,7 +80,8 @@ extern "C" int mq_eikonal_batch(const float* slow, const int32_t* src_iz, int n,
     }
 done:
 #undef TRY
-    cudaFree(d_slow); cudaFree(d_iz); cudaFree(d_st); cudaFree(d_out); cudaFree(d_scr); cudaFree(d_slice);
+    cudaFree(d_slow); cudaFree(d_iz); cudaFree(d_st); cudaFree(d_out);
+    eik_work_free(&work);
     return rc;
 }
 

@@ -12,14 +12,32 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <algorithm>
 #include "launch_count.h"
 #include <cub/device/device_radix_sort.cuh>
 
 namespace mq {
 
 constexpr float kInfM = eik::kInf;
+constexpr int kFineNodes = 22 * 43;   // refined grid of a left-edge source, src/time_2d.c:844-864
 
-size_t eik_scratch_floats_per_warp(int nxmod, int nz)
+// What the fused, fine and pipelined kernels read of the work space (EikWork; the generic kernel takes the window alone:
+// given the whole view its stack frame grows).  The order is set only when it was filled for the batch.
+struct EikView {
+    float* window;
+    float* slices;
+    const int32_t* order;
+    int32_t* task_counter;
+    float* tie;
+    int pipe_slices;
+};
+
+// Solves per item of a table-mode batch: one per depth (parity) or one per receiver row (reciprocal).
+__host__ __device__ inline int eik_sources(const EikBatch& b) { return b.src_rows ? b.n_src_rows : b.nz; }
+
+// Floats of a per-warp window of the generic kernel (time field + refined grid, lane-interleaved): EikWork::window holds
+// EikWork::warps of them.  The other kernels need less per warp and take as many warps as fit (warps_fitting).
+static size_t eik_scratch_floats_per_warp(int nxmod, int nz)
 {
     return ((size_t)nxmod * nz + kFineNodes) * 32;
 }
@@ -59,14 +77,14 @@ __device__ __forceinline__ TableSolve table_solve(const EikBatch& b, int n_items
 // lane (node i of lane l at scratch[i*32 + l]) so that lanes that sweep the same node
 // -- the common case, all lanes of a warp share the source depth -- touch one 128-byte line.
 __global__ void __launch_bounds__(128)
-eik_generic_kernel(EikBatch b)
+eik_generic_kernel(EikBatch b, float* window)
 {
     const int lane = threadIdx.x & 31;
     const int warps_per_block = blockDim.x >> 5;
     const int warp = blockIdx.x * warps_per_block + (threadIdx.x >> 5);
     const int n_warps = gridDim.x * warps_per_block;
     const int nodes = b.nxmod * b.nz;
-    float* W = b.scratch + (size_t)warp * (((size_t)nodes + kFineNodes) * 32) + lane;
+    float* W = window + (size_t)warp * (((size_t)nodes + kFineNodes) * 32) + lane;
     float* WF = W + (size_t)nodes * 32;
     const int n_items = b.n_items_dev ? *b.n_items_dev : b.n_items;
     const int n_solves = b.src_iz ? b.n_solves : n_items * eik_sources(b);
@@ -98,15 +116,20 @@ eik_generic_kernel(EikBatch b)
     }
 }
 
-cudaError_t eik_launch_generic(const EikBatch& b, cudaStream_t stream)
+// Warps with windows of floats_per_warp floats that fit the work space's window.
+static long warps_fitting(const EikWork& w, size_t floats_per_warp)
 {
-    const int n_solves = b.src_iz ? b.n_solves : b.n_items * eik_sources(b);   // upper bound when n_items_dev is set
-    if (n_solves <= 0) return cudaSuccess;
+    return (long)((size_t)w.warps * eik_scratch_floats_per_warp(w.nxmod, w.nz) / floats_per_warp);
+}
+
+static cudaError_t eik_launch_generic(const EikBatch& b, const EikWork& w, const EikView& v, int n_solves, cudaStream_t stream)
+{
     const int n_tasks = (n_solves + 31) / 32;
-    const int warps = n_tasks < b.max_warps ? n_tasks : b.max_warps;
+    const long fit = warps_fitting(w, eik_scratch_floats_per_warp(b.nxmod, b.nz));
+    const int warps = n_tasks < fit ? n_tasks : (int)fit;
     const int wpb = 4;
     const int blocks = (warps + wpb - 1) / wpb;
-    eik_generic_kernel<<<blocks, wpb * 32, 0, stream>>>(b);
+    eik_generic_kernel<<<blocks, wpb * 32, 0, stream>>>(b, v.window);
     count_launch();
     return cudaGetLastError();
 }
@@ -127,7 +150,7 @@ static eikf::Dims fast_dims(int nxmod, int nz)
 static size_t fast_smem_floats_per_warp(const eikf::Dims& D) { return (size_t)eikf::smem_floats_per_lane(D) * 32; }
 static size_t fast_scratch_floats_per_warp(const eikf::Dims& D) { return ((size_t)D.wx * D.nz + kFineNodes) * 32; }
 
-bool eik_fast_supported(int nxmod, int nz)
+static bool eik_fast_supported(int nxmod, int nz)
 {
     if (nxmod < 2 || nz < 2) return false;
     const eikf::Dims D = fast_dims(nxmod, nz);
@@ -140,14 +163,14 @@ bool eik_fast_supported(int nxmod, int nz)
 // shared-memory slice, so that the lock-step sweeps (rows, the march) touch one 128-byte line per access.  Same code,
 // same results; what hides the memory latency is the number of resident warps.
 template <bool GLOBAL_SLICE>
-__device__ __forceinline__ void eik_fast_body(const EikBatch& b, const eikf::Dims& D, float* slice, int lpt)
+__device__ __forceinline__ void eik_fast_body(const EikBatch& b, const EikView& wk, const eikf::Dims& D, float* slice, int lpt)
 {
     const int lane = threadIdx.x;
     const int nodes = b.nxmod * b.nz;
     eikf::Lane L;
     if (GLOBAL_SLICE) eikf::carve_global(slice + lane, D, &L);
     else eikf::carve_shared(slice + lane, D, &L);
-    L.W = b.scratch + (size_t)blockIdx.x * (((size_t)D.wx * D.nz + kFineNodes) * 32) + lane;
+    L.W = wk.window + (size_t)blockIdx.x * (((size_t)D.wx * D.nz + kFineNodes) * 32) + lane;
     L.WF = L.W + (size_t)D.wx * D.nz * 32;
     const int n_items = b.n_items_dev ? *b.n_items_dev : b.n_items;
     const int n_solves = b.src_iz ? b.n_solves : n_items * eik_sources(b);
@@ -156,7 +179,7 @@ __device__ __forceinline__ void eik_fast_body(const EikBatch& b, const eikf::Dim
     for (int task = blockIdx.x; task < n_tasks; task += gridDim.x) {
         int g = task * lpt + lane;
         if (lane >= lpt) g = -1;
-        else if (b.order) g = b.order[g];
+        else if (wk.order) g = wk.order[g];
         eikf::LaneTask t;
         t.valid = g >= 0 && g < n_solves;
         t.iz = 0; t.slow = nullptr; t.out = nullptr; t.out_rstride = 0; t.full = nullptr; t.hand_col = nullptr; t.hand_x1 = nullptr;
@@ -182,15 +205,15 @@ __device__ __forceinline__ void eik_fast_body(const EikBatch& b, const eikf::Dim
 }
 
 // lanes_per_task: lanes of a warp that carry a solve (32, 16, 8 or 4)
-__global__ void __launch_bounds__(32, 9) eik_fast_kernel(EikBatch b, eikf::Dims D, int lanes_per_task)
+__global__ void __launch_bounds__(32, 9) eik_fast_kernel(EikBatch b, EikView wk, eikf::Dims D, int lanes_per_task)
 {
     extern __shared__ float smem[];
-    eik_fast_body<false>(b, D, smem, lanes_per_task);
+    eik_fast_body<false>(b, wk, D, smem, lanes_per_task);
 }
 
-__global__ void __launch_bounds__(32, 8) eik_fine_kernel(EikBatch b, eikf::Dims D, int lanes_per_task)
+__global__ void __launch_bounds__(32, 8) eik_fine_kernel(EikBatch b, EikView wk, eikf::Dims D, int lanes_per_task)
 {
-    eik_fast_body<true>(b, D, b.slice_scratch + (size_t)blockIdx.x * ((size_t)eikf::gmem_floats_per_lane(D) * 32), lanes_per_task);
+    eik_fast_body<true>(b, wk, D, wk.slices + (size_t)blockIdx.x * ((size_t)eikf::gmem_floats_per_lane(D) * 32), lanes_per_task);
 }
 
 // ---- regrouping of solves --------------------------------------------------------------------------------------
@@ -240,7 +263,8 @@ __global__ void eik_key_kernel(EikBatch b, int max_solves, uint64_t* keys, int32
     vals[g] = g;
 }
 
-size_t eik_order_bytes(int max_solves)
+// Bytes of the sort buffers (EikWork::sort) for up to max_solves solves.
+static size_t eik_order_bytes(int max_solves)
 {
     const size_t n = ((size_t)max_solves + 31) / 32 * 32;
     size_t tmp = 0;
@@ -249,23 +273,25 @@ size_t eik_order_bytes(int max_solves)
     return 2 * n * sizeof(uint64_t) + n * sizeof(int32_t) + ((tmp + 255) / 256 * 256) + 1024;
 }
 
-cudaError_t eik_order_tasks(const EikBatch& b, int32_t* order, void* work, size_t work_bytes, cudaStream_t stream)
+// Fills wk.order[0 .. round_up(max_solves, 32)): order[j] = the solve g (source * n_items + item) that lane j % 32 of warp
+// task j / 32 runs, or -1.
+static cudaError_t eik_order_tasks(const EikBatch& b, const EikWork& wk, cudaStream_t stream)
 {
     const int max_solves = b.n_items * eik_sources(b);
     if (max_solves <= 0) return cudaSuccess;
     const size_t n = ((size_t)max_solves + 31) / 32 * 32;
-    char* w = (char*)work;
+    char* w = (char*)wk.sort;
     uint64_t* k_in = (uint64_t*)w;               w += n * sizeof(uint64_t);
     uint64_t* k_out = (uint64_t*)w;              w += n * sizeof(uint64_t);
     int32_t* v_in = (int32_t*)w;                 w += n * sizeof(int32_t);
     w = (char*)(((uintptr_t)w + 255) / 256 * 256);
-    size_t tmp = work_bytes - (size_t)(w - (char*)work);
+    size_t tmp = wk.sort_bytes - (size_t)(w - (char*)wk.sort);
     eik_key_kernel<<<(unsigned)((n + 127) / 128), 128, 0, stream>>>(b, (int)n, k_in, v_in);
     count_launch();
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     // source depth needs at most 12 bits above bit 32 (nz <= 4096)
-    e = cub::DeviceRadixSort::SortPairs(w, tmp, k_in, k_out, v_in, order, (int)n, 0, 44, stream);
+    e = cub::DeviceRadixSort::SortPairs(w, tmp, k_in, k_out, v_in, wk.order, (int)n, 0, 44, stream);
     count_launch(3);
     return e;
 }
@@ -355,7 +381,7 @@ __device__ __forceinline__ void pipe_release(unsigned* mask, int bit, int lane)
 // CA: nodes -1 .. CA-2 per TMEM column array (nz <= CA - 2); WARPS: warps per CTA; RECIP: reciprocal tables
 // (EikBatch::src_rows, with rows = 0 .. nz-1): every row of each column is output.
 template <int CA, int WARPS, bool RECIP>
-__device__ __forceinline__ void eik_pipe_body(const EikBatch& b, const eikf::Dims& D, int n_slices, int* task_counter)
+__device__ __forceinline__ void eik_pipe_body(const EikBatch& b, const EikView& wk, const eikf::Dims& D)
 {
     constexpr int NB = CA / 4;
     constexpr int kSets = 512 / (3 * CA);        // TMEM sets per lane quarter: 2 at CA = 64, 1 at CA = 128
@@ -364,7 +390,7 @@ __device__ __forceinline__ void eik_pipe_body(const EikBatch& b, const eikf::Dim
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, quarter = warp & 3;
     if (warp == 0) eikm::tmem_alloc<512>(&ctl.tmem);
     if (threadIdx.x == 0) {
-        ctl.slice_free = (1u << n_slices) - 1u;
+        ctl.slice_free = (1u << wk.pipe_slices) - 1u;
         for (int q = 0; q < 4; q++) ctl.tset_free[q] = (1u << kSets) - 1u;
         ctl.tie_lock = 0;
     }
@@ -373,7 +399,7 @@ __device__ __forceinline__ void eik_pipe_body(const EikBatch& b, const eikf::Dim
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const size_t slice_floats = (size_t)eikf::smem_floats_per_lane(D) * 32;
     // scratch of the literal walk for a column with an exact tie (4 in 100 000): global memory, one per CTA, under a lock
-    float* tieP = b.tie_scratch + (size_t)blockIdx.x * kPipeTieFloats<CA> + 32 + lane;   // node k at tieP[k*32], k = -1 .. CA-2
+    float* tieP = wk.tie + (size_t)blockIdx.x * kPipeTieFloats<CA> + 32 + lane;   // node k at tieP[k*32], k = -1 .. CA-2
     float* tieC = tieP + (size_t)CA * 32;
     float* tieS = tieC + (size_t)CA * 32 + 32;                             // cell k at tieS[k*32], k = -2 .. CA-1
     const int nz = b.nz, ke = nz - 1, mx = b.nxmod - 1;
@@ -381,15 +407,15 @@ __device__ __forceinline__ void eik_pipe_body(const EikBatch& b, const eikf::Dim
     const int n_solves = n_items * (RECIP ? b.n_src_rows : nz);
     const int n_tasks = (n_solves + 31) >> 5;
     const size_t wfloats = ((size_t)D.wx * D.nz + kFineNodes) * 32;
-    float* Wbase = b.scratch + (size_t)(blockIdx.x * WARPS + warp) * wfloats + lane;
+    float* Wbase = wk.window + (size_t)(blockIdx.x * WARPS + warp) * wfloats + lane;
 
     for (;;) {
         int task = 0;
-        if (lane == 0) task = atomicAdd(task_counter, 1);
+        if (lane == 0) task = atomicAdd(wk.task_counter, 1);
         task = __shfl_sync(0xffffffffu, task, 0);
         if (task >= n_tasks) break;
         int g = task * 32 + lane;
-        if (b.order) g = b.order[g];
+        if (wk.order) g = wk.order[g];
         // ---- box phase on a shared-memory slice
         const int sl = pipe_acquire(&ctl.slice_free, lane);
         eikf::Lane L;
@@ -524,110 +550,63 @@ __device__ __forceinline__ void eik_pipe_body(const EikBatch& b, const eikf::Dim
 }
 
 template <int CA, int WARPS>
-__global__ void __launch_bounds__(WARPS * 32, 1) eik_pipe_kernel(EikBatch b, eikf::Dims D, int n_slices, int* task_counter)
+__global__ void __launch_bounds__(WARPS * 32, 1) eik_pipe_kernel(EikBatch b, EikView wk, eikf::Dims D)
 {
-    eik_pipe_body<CA, WARPS, false>(b, D, n_slices, task_counter);
+    eik_pipe_body<CA, WARPS, false>(b, wk, D);
 }
 // The reciprocal-table instantiation (a kernel of its own name: the parity kernel's code stays as it is)
 template <int CA, int WARPS>
-__global__ void __launch_bounds__(WARPS * 32, 1) eik_pipe_recip_kernel(EikBatch b, eikf::Dims D, int n_slices, int* task_counter)
+__global__ void __launch_bounds__(WARPS * 32, 1) eik_pipe_recip_kernel(EikBatch b, EikView wk, eikf::Dims D)
 {
-    eik_pipe_body<CA, WARPS, true>(b, D, n_slices, task_counter);
+    eik_pipe_body<CA, WARPS, true>(b, wk, D);
 }
 
-bool eik_pipe_supported(int nxmod, int nz)
+static bool eik_pipe_enabled()
 {
     static int enabled = -1;
     if (enabled < 0) {
         const char* e = getenv("MCMCEQ_EIKONAL_PIPE");
         enabled = (e && e[0] == '0') ? 0 : 1;     // on unless MCMCEQ_EIKONAL_PIPE=0
     }
-    return enabled && eik_fast_supported(nxmod, nz) && pipe_shape(nz).ca > 0;
+    return enabled;
 }
 
-cudaError_t eik_launch_pipe(const EikBatch& b, int* task_counter, cudaStream_t stream)
+static eikf::Dims pipe_dims(int nxmod, int nz)
 {
-    if (b.src_iz || b.full_out || !task_counter || !b.tie_scratch) return cudaErrorInvalidValue;
-    if (b.src_rows && b.n_rows != b.nz) return cudaErrorInvalidValue;   // the reciprocal march stores every row
-    const PipeShape sh = pipe_shape(b.nz);
-    if (!sh.ca) return cudaErrorInvalidValue;
-    void (*const kernel)(EikBatch, eikf::Dims, int, int*) =
-        b.src_rows ? (sh.ca == 64 ? eik_pipe_recip_kernel<64, kPipeWarps> : eik_pipe_recip_kernel<128, kPipeWarpsDeep>)
-                     : (sh.ca == 64 ? eik_pipe_kernel<64, kPipeWarps> : eik_pipe_kernel<128, kPipeWarpsDeep>);
-    eikf::Dims D = fast_dims(b.nxmod, b.nz);
+    eikf::Dims D = fast_dims(nxmod, nz);
     // Lock-step columns in the box phase (a second column buffer per slice: 7 slices instead of 9 on the Example plane).
     // Kernel ms per launch at 1024 / 2048 / 4096 / 8192 chains with the box phase inlined: 7.70 / 13.99 / 26.42 / 51.07
     // against 8.03 / 14.24 / 26.66 / 51.07 with the per-lane in-place walk (profiles/README.md r2c).
     D.lock_cols = 1;
-    const size_t slice = fast_smem_floats_per_warp(D) * sizeof(float);
-    int dev = 0, sms = 148, smem_max = 232448;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-    int n_slices = (int)(((size_t)smem_max - 256) / slice);
-    if (n_slices > sh.warps) n_slices = sh.warps;
-    if (n_slices < 2) return cudaErrorInvalidValue;
-    const size_t smem = (size_t)n_slices * slice;
-    // per instantiation and device: largest dynamic shared-memory size the kernel has been opted in for
-    static size_t configured[4][64] = {};
-    size_t* conf = (dev >= 0 && dev < 64) ? &configured[(sh.ca == 128) * 2 + (b.src_rows ? 1 : 0)][dev] : nullptr;
-    if (!conf || smem > *conf) {
-        cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-        if (conf) *conf = smem;
-    }
-    const int n_tasks = (b.n_items * eik_sources(b) + 31) / 32;
-    // per-warp global window: the scratch was sized for max_warps warps of the generic kernel
-    const size_t have = (size_t)b.max_warps * eik_scratch_floats_per_warp(b.nxmod, b.nz);
-    const long warps_by_scratch = (long)(have / fast_scratch_floats_per_warp(D));
-    int blocks = (n_tasks + sh.warps - 1) / sh.warps;
-    if (blocks > sms) blocks = sms;
-    if ((long)blocks * sh.warps > warps_by_scratch) blocks = (int)(warps_by_scratch / sh.warps);
-    if (blocks < 1) return cudaErrorInvalidValue;
-    cudaError_t e = cudaMemsetAsync(task_counter, 0, sizeof(int), stream);
-    if (e != cudaSuccess) return e;
-    kernel<<<blocks, sh.warps * 32, smem, stream>>>(b, D, n_slices, task_counter);
-    count_launch();
-    return cudaGetLastError();
+    return D;
 }
 
-size_t eik_pipe_tie_floats(int nz)
+static size_t eik_pipe_tie_floats(int nz)
 {
     return (size_t)kPipeMaxCtas * (pipe_shape(nz).ca == 128 ? kPipeTieFloats<128> : kPipeTieFloats<64>);
 }
 
-int eik_fast_max_warps(int nxmod, int nz, int device)
+static cudaError_t eik_launch_pipe(const EikBatch& b, const EikWork& w, const EikView& v, long fit, int n_solves, cudaStream_t stream)
 {
-    const eikf::Dims D = fast_dims(nxmod, nz);
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
-    int per_sm = 0;
-    const size_t smem = fast_smem_floats_per_warp(D) * sizeof(float);
-    cudaFuncSetAttribute(eik_fast_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    cudaFuncSetAttribute(eik_fast_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, eik_fast_kernel, 32, smem);
-    if (per_sm < 1) per_sm = 1;
-    return sms * per_sm;
+    void (*const kernel)(EikBatch, EikView, eikf::Dims) =
+        b.src_rows ? (w.pipe_ca == 64 ? eik_pipe_recip_kernel<64, kPipeWarps> : eik_pipe_recip_kernel<128, kPipeWarpsDeep>)
+                   : (w.pipe_ca == 64 ? eik_pipe_kernel<64, kPipeWarps> : eik_pipe_kernel<128, kPipeWarpsDeep>);
+    const int n_tasks = (n_solves + 31) / 32;
+    int blocks = (n_tasks + w.pipe_warps - 1) / w.pipe_warps;
+    if (blocks > w.sms) blocks = w.sms;
+    if ((long)blocks * w.pipe_warps > fit) blocks = (int)(fit / w.pipe_warps);
+    cudaError_t e = cudaMemsetAsync(w.task_counter, 0, sizeof(int), stream);
+    if (e != cudaSuccess) return e;
+    kernel<<<blocks, w.pipe_warps * 32, w.pipe_smem, stream>>>(b, v, pipe_dims(b.nxmod, b.nz));
+    count_launch();
+    return cudaGetLastError();
 }
 
-cudaError_t eik_launch_fast(const EikBatch& b, cudaStream_t stream)
+static cudaError_t eik_launch_fast(const EikBatch& b, const EikWork& w, const EikView& v, long fit, int n_solves, cudaStream_t stream)
 {
-    const int n_solves = b.src_iz ? b.n_solves : b.n_items * eik_sources(b);
-    if (n_solves <= 0) return cudaSuccess;
     const eikf::Dims D = fast_dims(b.nxmod, b.nz);
     const size_t smem = fast_smem_floats_per_warp(D) * sizeof(float);
-    static int configured_for = -1;
-    int dev = 0;
-    cudaGetDevice(&dev);
-    static int resident = 0;
-    if (configured_for != dev * 100000 + b.nz) {
-        resident = eik_fast_max_warps(b.nxmod, b.nz, dev);
-        configured_for = dev * 100000 + b.nz;
-    }
-    // scratch was sized for max_warps warps of the generic kernel, which is never less per warp
-    const size_t have = (size_t)b.max_warps * eik_scratch_floats_per_warp(b.nxmod, b.nz);
-    long warps = (long)(have / fast_scratch_floats_per_warp(D));
-    if (warps > resident) warps = resident;
+    long warps = fit < w.fast_resident ? fit : w.fast_resident;
     // A launch with fewer warp-tasks than warps that can be resident lasts as long as one task, and a task is the shorter
     // the fewer lanes have to wait for each other in the box phase: spread it over the idle warps.
     int lpt = 32;
@@ -635,7 +614,7 @@ cudaError_t eik_launch_fast(const EikBatch& b, cudaStream_t stream)
     const int n_tasks = (n_solves + lpt - 1) / lpt;
     if (warps > n_tasks) warps = n_tasks;
     if (warps < 1) warps = 1;
-    eik_fast_kernel<<<(unsigned)warps, 32, smem, stream>>>(b, D, lpt);
+    eik_fast_kernel<<<(unsigned)warps, 32, smem, stream>>>(b, v, D, lpt);
     count_launch();
     return cudaGetLastError();
 }
@@ -646,58 +625,142 @@ const char* eik_kernel_name(int which)
     return (which >= 0 && which < kEikKernels) ? names[which] : "?";
 }
 
-size_t eik_fine_slice_floats_per_warp(int nxmod, int nz)
+static size_t eik_fine_slice_floats_per_warp(int nxmod, int nz)
 {
     return (size_t)eikf::gmem_floats_per_lane(fast_dims(nxmod, nz)) * 32;
 }
 
-cudaError_t eik_launch_fine(const EikBatch& b, cudaStream_t stream)
+static cudaError_t eik_launch_fine(const EikBatch& b, const EikWork& w, const EikView& v, long fit, int n_solves, cudaStream_t stream)
 {
-    const int n_solves = b.src_iz ? b.n_solves : b.n_items * eik_sources(b);
-    if (n_solves <= 0) return cudaSuccess;
-    if (!b.slice_scratch) return cudaErrorInvalidValue;
-    const eikf::Dims D = fast_dims(b.nxmod, b.nz);
     const int n_tasks = (n_solves + 31) / 32;
-    // one warp per CTA; the window (b.scratch) and the slice were sized for max_warps warps
-    const size_t have = (size_t)b.max_warps * eik_scratch_floats_per_warp(b.nxmod, b.nz);
-    long warps = (long)(have / fast_scratch_floats_per_warp(D));
-    if (warps > b.max_warps) warps = b.max_warps;
+    // one warp per CTA; the slices exist for w.warps warps
+    long warps = fit < w.warps ? fit : w.warps;
     if (warps > n_tasks) warps = n_tasks;
     if (warps < 1) warps = 1;
-    eik_fine_kernel<<<(unsigned)warps, 32, 0, stream>>>(b, D, 32);
+    eik_fine_kernel<<<(unsigned)warps, 32, 0, stream>>>(b, v, fast_dims(b.nxmod, b.nz), 32);
     count_launch();
     return cudaGetLastError();
 }
 
-cudaError_t eik_launch(const EikBatch& b, cudaStream_t stream, int* which)
+cudaError_t eik_launch(const EikBatch& b, const EikWork& w, cudaStream_t stream, int* which)
 {
     int dummy;
     if (!which) which = &dummy;
+    if (b.nxmod != w.nxmod || b.nz != w.nz) return cudaErrorInvalidValue;   // the windows are laid out for the work's plane
     static int force_generic = -1;
     if (force_generic < 0) {
         const char* e = getenv("MCMCEQ_EIKONAL");
         force_generic = (e && strcmp(e, "generic") == 0) ? 1 : 0;
     }
-    if (!force_generic && b.task_counter && b.tie_scratch && !b.src_iz && !b.full_out && (!b.src_rows || b.n_rows == b.nz) &&
-        eik_pipe_supported(b.nxmod, b.nz)) {
-        // worth it (and the per-warp scratch windows suffice) only when there is work for every warp of every SM
-        const eikf::Dims D = fast_dims(b.nxmod, b.nz);
-        const size_t have = (size_t)b.max_warps * eik_scratch_floats_per_warp(b.nxmod, b.nz);
-        const long n_tasks = ((long)b.n_items * eik_sources(b) + 31) / 32;
-        int dev = 0, sms = 148;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        const int warps = pipe_shape(b.nz).warps;
-        if ((long)(have / fast_scratch_floats_per_warp(D)) >= (long)sms * warps && n_tasks >= (long)sms * warps &&
-            sms <= kPipeMaxCtas) {
+    EikView v = {w.window, w.slices, nullptr, w.task_counter, w.tie, w.pipe_slices};
+    if (b.regroup && w.order) {
+        const cudaError_t e = eik_order_tasks(b, w, stream);
+        if (e != cudaSuccess) return e;
+        v.order = w.order;
+    }
+    const int n_solves = b.src_iz ? b.n_solves : b.n_items * eik_sources(b);   // upper bound when n_items_dev is set
+    // warps of the fused, fine and pipelined kernels whose windows fit the work space
+    const long fit = warps_fitting(w, fast_scratch_floats_per_warp(fast_dims(b.nxmod, b.nz)));
+    if (!force_generic && w.pipe_ca && !b.src_iz && !b.full_out && (!b.src_rows || b.n_rows == b.nz)) {
+        // worth it (and the per-warp windows suffice) only when there is work for every warp of every SM
+        const long full = (long)w.sms * w.pipe_warps;
+        if (fit >= full && (n_solves + 31) / 32 >= full) {
             *which = kEikPipe;
-            return eik_launch_pipe(b, b.task_counter, stream);
+            return eik_launch_pipe(b, w, v, fit, n_solves, stream);
         }
     }
-    if (!force_generic && eik_fast_supported(b.nxmod, b.nz)) { *which = kEikFast; return eik_launch_fast(b, stream); }
-    if (!force_generic && b.slice_scratch && b.nxmod >= 2 && b.nz >= 2) { *which = kEikFine; return eik_launch_fine(b, stream); }
-    *which = kEikGeneric;
-    return eik_launch_generic(b, stream);
+    *which = force_generic ? kEikGeneric : w.fast_resident ? kEikFast : (w.slices && b.nxmod >= 2 && b.nz >= 2) ? kEikFine : kEikGeneric;
+    if (n_solves <= 0) return cudaSuccess;
+    if (*which == kEikFast) return eik_launch_fast(b, w, v, fit, n_solves, stream);
+    if (*which == kEikFine) return eik_launch_fine(b, w, v, fit, n_solves, stream);
+    return eik_launch_generic(b, w, v, n_solves, stream);
+}
+
+// Dynamic shared memory: the kernels that take it may use all a block can opt in to on the device, with the largest
+// carveout.  Set on every allocation (it is the same each time), so a kernel's limit is never lowered under a launch
+// that relies on it, whatever plane another work space on the device has.
+static cudaError_t opt_in_shared(int smem_optin)
+{
+    const void* kernels[] = {(const void*)eik_fast_kernel,
+                             (const void*)eik_pipe_kernel<64, kPipeWarps>, (const void*)eik_pipe_kernel<128, kPipeWarpsDeep>,
+                             (const void*)eik_pipe_recip_kernel<64, kPipeWarps>, (const void*)eik_pipe_recip_kernel<128, kPipeWarpsDeep>};
+    for (const void* kernel : kernels) {
+        cudaFuncAttributes a;
+        cudaError_t e = cudaFuncGetAttributes(&a, kernel);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_optin - (int)a.sharedSizeBytes);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
+}
+
+cudaError_t eik_work_alloc(EikWork* w, int nxmod, int nz, int max_solves, bool tables, int device)
+{
+    *w = EikWork{};
+    w->nxmod = nxmod;
+    w->nz = nz;
+    int smem_optin = 0;
+    cudaError_t e = cudaDeviceGetAttribute(&w->sms, cudaDevAttrMultiProcessorCount, device);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device);
+    if (e == cudaSuccess) e = opt_in_shared(smem_optin);
+    if (e != cudaSuccess) return e;
+    const bool fast = eik_fast_supported(nxmod, nz);
+    if (fast) {
+        int per_sm = 0;
+        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, eik_fast_kernel, 32,
+                                                          fast_smem_floats_per_warp(fast_dims(nxmod, nz)) * sizeof(float));
+        if (e != cudaSuccess) return e;
+        w->fast_resident = w->sms * (per_sm < 1 ? 1 : per_sm);
+    }
+    const PipeShape sh = pipe_shape(nz);
+    if (tables && fast && sh.ca && eik_pipe_enabled() && w->sms <= kPipeMaxCtas) {
+        const size_t slice = fast_smem_floats_per_warp(pipe_dims(nxmod, nz)) * sizeof(float);
+        const int n_slices = std::min<int>((int)(((size_t)smem_optin - 256) / slice), sh.warps);
+        if (n_slices >= 2) {
+            w->pipe_ca = sh.ca;
+            w->pipe_warps = sh.warps;
+            w->pipe_slices = n_slices;
+            w->pipe_smem = (size_t)n_slices * slice;
+        }
+    }
+
+    // Windows for one full wave of the solves, never more (the fine kernel: 12 warps per SM, the others 16).  Large planes
+    // (the 0.1 km fine-grid case: 565 x 2001 nodes = 145 MB of window + 0.8 MB of slice per warp): never more than 70 %
+    // of the device memory that is still free (25 % for planes that fit a shared-memory slice); the kernels loop over the
+    // tasks with however many warps they are given.  MCMCEQ_SCRATCH_FRACTION overrides the fraction.
+    long warps = std::min<long>(((long)max_solves + 31) / 32, (long)w->sms * (fast ? 16 : 12));
+    size_t free_b = 0, total_b = 0;
+    if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess) {
+        double frac = fast ? 0.25 : 0.7;
+        if (const char* s = getenv("MCMCEQ_SCRATCH_FRACTION")) { const double f = atof(s); if (f > 0.0 && f < 0.95) frac = f; }
+        const size_t per_warp = (eik_scratch_floats_per_warp(nxmod, nz) + (fast ? 0 : eik_fine_slice_floats_per_warp(nxmod, nz))) * sizeof(float);
+        const long by_mem = (long)(((double)free_b * frac) / (double)per_warp);
+        warps = std::min<long>(warps, std::max<long>(by_mem, 4));
+    }
+    w->warps = (int)((warps + 3) / 4 * 4);
+    e = cudaMalloc(&w->window, (size_t)w->warps * eik_scratch_floats_per_warp(nxmod, nz) * sizeof(float));
+    if (e == cudaSuccess && !fast) e = cudaMalloc(&w->slices, (size_t)w->warps * eik_fine_slice_floats_per_warp(nxmod, nz) * sizeof(float));
+    // regrouping (planes that do not fit a shared-memory slice keep the natural order: a chain's P and S solves of one
+    // source depth are neighbours there, which is the grouping their long box phases want; measured, tools/fine_probe2.py)
+    if (e == cudaSuccess && tables && fast) {
+        w->sort_bytes = eik_order_bytes(max_solves);
+        e = cudaMalloc(&w->sort, w->sort_bytes);
+        if (e == cudaSuccess) e = cudaMalloc((void**)&w->order, (((size_t)max_solves + 31) / 32 * 32) * sizeof(int32_t));
+    }
+    if (e == cudaSuccess && w->pipe_ca) {
+        e = cudaMalloc((void**)&w->task_counter, sizeof(int32_t));
+        if (e == cudaSuccess) e = cudaMemset(w->task_counter, 0, sizeof(int32_t));
+        if (e == cudaSuccess) e = cudaMalloc((void**)&w->tie, eik_pipe_tie_floats(nz) * sizeof(float));
+        if (e == cudaSuccess) e = cudaMemset(w->tie, 0, eik_pipe_tie_floats(nz) * sizeof(float));
+    }
+    if (e != cudaSuccess) eik_work_free(w);
+    return e;
+}
+
+void eik_work_free(EikWork* w)
+{
+    cudaFree(w->window); cudaFree(w->slices); cudaFree(w->sort); cudaFree(w->order); cudaFree(w->task_counter); cudaFree(w->tie);
+    *w = EikWork{};
 }
 
 }  // namespace mq

@@ -186,14 +186,8 @@ cudaError_t launch_tables(Handle* h, int max_items)
         b.rows = h->d_all_rows; b.n_rows = h->nz;
     }
     b.status_min = h->solve_status;
-    b.scratch = h->scratch; b.max_warps = h->scratch_warps; b.slice_scratch = h->eik_slice_scratch;
-    if (h->eik_order) {
-        const cudaError_t e = eik_order_tasks(b, h->eik_order, h->eik_order_work, h->eik_order_bytes, h->stream);
-        if (e != cudaSuccess) return e;
-        b.order = h->eik_order;
-    }
-    b.task_counter = h->eik_task_counter; b.tie_scratch = h->eik_tie_scratch;
-    return eik_launch(b, h->stream, &which);
+    b.regroup = true;
+    return eik_launch(b, h->eik, h->stream, &which);
 }
 
 // ---- travel-time lookup -------------------------------------------------------------------

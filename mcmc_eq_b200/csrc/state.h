@@ -19,6 +19,7 @@
 #include <stdint.h>
 
 #include "../../include/mcmceq_b200.h"
+#include "eikonal.cuh"
 
 namespace mq {
 
@@ -120,7 +121,6 @@ struct Handle {
     cudaEvent_t flags_ev; // ... valid once this event has completed
     bool flags_pending;
     cudaEvent_t timer_ev[2][16];   // mq_timer
-    int eik_pipe_smem;   // dynamic shared memory eik_pipe_kernel has been opted in for on this handle's device
 
     // evaluation plumbing
     EvalView cur_view;   // view of the current state
@@ -138,14 +138,7 @@ struct Handle {
     float* slow;         // [2n][nz]
     float** item_tab;    // [2n] destination table of each item
     int32_t* solve_status; // [1] min over solves
-    float* scratch;      // eikonal scratch
-    int scratch_warps;
-    float* eik_slice_scratch;    // per-warp global-memory slices of the fine-grid kernel (eikonal.cuh), or nullptr
-    int32_t* eik_task_counter;   // work counter and tie scratch of the pipelined eikonal kernel (eikonal.cuh), or nullptr
-    float* eik_tie_scratch;
-    int32_t* eik_order;  // [round_up(2n*nz, 32)] execution order of the solves of a table rebuild (eikonal.cuh), or nullptr
-    void* eik_order_work;
-    size_t eik_order_bytes;
+    EikWork eik;         // work space of the table rebuilds (eikonal.cuh), for 2n*nz solves
 
     // sampler (chain.cu)
     void* sampler;
