@@ -420,7 +420,7 @@ __global__ void propose_kernel(SamplerParams p, Handle hd, SamplerDev s, EvalVie
         }
     }
     if (p.cfg.aflag == 1) v.ev_only[c] = -2;   // prior sampling: no likelihood (src/misfit.c:61)
-    if (!ok) { s.not_valid[c] = 1; v.ev_only[c] = -2; }
+    if (!ok) { s.not_valid[c] = 2; v.ev_only[c] = -2; }   // a retry loop gave up: rejected whatever aflag (accept_kernel)
     s.draws[c] = rng.draws;
     if (s.hold) {
         if (s.hold[c] == 2) atomicAdd(&s.pass_stat[0], 1);
@@ -523,7 +523,7 @@ __global__ void accept_kernel(SamplerParams p, Handle hd, SamplerDev s, EvalView
     float alpha;
     double new_misfit = 0, new_rms = 0, new_ll = 0;
     if (not_valid) {
-        alpha = 0.f;   // ineligible move: still consumes a uniform and counts as a rejection (quirk Q5)
+        alpha = 0.f;   // ineligible move (1) or a retry loop that gave up (2): still consumes a uniform (quirk Q5)
     } else {
         for (int k = 0; k < 8; k++) mf[k] = (g.aflag == 1) ? 0.f : hd.mf_eval[8 * (size_t)c + k];
         new_misfit = chain_misfit(mf, noise);
@@ -538,6 +538,9 @@ __global__ void accept_kernel(SamplerParams p, Handle hd, SamplerDev s, EvalView
     }
     if (g.aflag == 1) alpha = 1.f;
     if (not_valid && g.aflag == 0) alpha = 0.f;
+    // a retry loop that gave up leaves its last rejected try in the proposal buffers: never installed, not even when
+    // sampling the prior (the reference would loop for ever there)
+    if (not_valid == 2) alpha = 0.f;
 
     float u;
     if (s.u_inject) u = s.u_inject[c];   // replay: the reference's own deviate, no draw is consumed
