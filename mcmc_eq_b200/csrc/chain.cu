@@ -94,30 +94,6 @@ struct Philox {
     }
 };
 
-struct SamplerParams {
-    int n, md, ne, ns, nz;
-    mq_config cfg;
-    float xmin, xmax, ymin, ymax, zmin, zmax;
-    int lvz_flag, revert, sum_of_picks;
-    int n_class[8];
-    uint64_t seed;
-    size_t tab_stride;
-    long long chain_offset;
-};
-
-static SamplerParams make_params(const Handle* h)
-{
-    SamplerParams p;
-    p.n = h->n; p.md = h->md; p.ne = h->ne; p.ns = h->ns; p.nz = h->nz; p.cfg = h->cfg;
-    p.xmin = h->xmin; p.xmax = h->xmax; p.ymin = h->ymin; p.ymax = h->ymax; p.zmin = h->zmin; p.zmax = h->zmax;
-    p.lvz_flag = h->lvz_flag;
-    p.revert = (int)(h->cfg.j_max_start + h->cfg.j_max_main / 2);   // src/mcmc_eq.c:840
-    p.sum_of_picks = h->sum_of_picks;
-    for (int k = 0; k < 8; k++) p.n_class[k] = h->n_class[k];
-    p.seed = h->seed; p.tab_stride = h->tab_stride; p.chain_offset = h->chain_offset;
-    return p;
-}
-
 // ---- model_valid (src/mcmc_eq.c:180-229) on a model in global memory ---------------------
 // Work arrays wz/wp/ws hold the depth-sorted copy.  Returns 0 when valid, 1 otherwise.
 __device__ int model_valid_dev(int dim, const float* z, const float* vp, const float* vpvs, float* wz, float* wp,
@@ -170,60 +146,116 @@ __device__ int find_neighbor_dev(const float* z, int dim, int n)
 
 #define MQ_PI 3.141592653   // src/mc.h:50
 
+// Chain c's current model (buffer mcur[c]) and the origin times of its current event buffer (ecur[c]).
+struct CurModel {
+    int mc, ec, dim;
+    const float *z, *vp, *vpvs;
+    const float* origin;   // [ne]
+};
+__device__ __forceinline__ CurModel cur_model(const Handle& hd, int c)
+{
+    CurModel m;
+    m.mc = hd.mcur[c]; m.ec = hd.ecur[c];
+    m.dim = hd.dim[m.mc * hd.n + c];
+    const size_t mo = ((size_t)m.mc * hd.n + c) * hd.md;
+    m.z = hd.z + mo; m.vp = hd.vp + mo; m.vpvs = hd.vpvs + mo;
+    m.origin = hd.origin + ((size_t)m.ec * hd.n + c) * hd.ne;
+    return m;
+}
+
+// The view of a chain before its proposal is known: nothing to evaluate, the current buffers.
+__device__ __forceinline__ void view_defaults(const Handle& hd, const EvalView& v, int c, const CurModel& m)
+{
+    v.q_idx[c] = -1; v.r_idx[c] = -1; v.ev_only[c] = -2;
+    v.mbuf[c] = m.mc; v.tbuf[2 * c] = hd.tcur[2 * c]; v.tbuf[2 * c + 1] = hd.tcur[2 * c + 1]; v.ebuf[c] = m.ec;
+}
+
+// A velocity-model proposal of `newdim` nuclei, written into the other model buffer: every event is evaluated with it into
+// the other event buffer; calct (1 P, 2 S, 3 both) names the phases whose tables it needs.
+__device__ __forceinline__ void view_model_arm(const Handle& hd, const SamplerDev& s, const EvalView& v, int c, const CurModel& m,
+                                               int newdim, int calct)
+{
+    hd.dim[(1 - m.mc) * hd.n + c] = newdim;
+    v.mbuf[c] = 1 - m.mc; v.ev_only[c] = -1; v.ebuf[c] = 1 - m.ec;
+    s.rebuilt[c] = calct;
+}
+
+// ---- table rebuild queue: the phases in calct get the chain's other table buffer ...
+__device__ __forceinline__ void flip_tables(const Handle& hd, const EvalView& v, int c, int calct)
+{
+    for (int ph = 0; ph < 2; ph++)
+        if (calct & (1 << ph)) v.tbuf[2 * c + ph] = 1 - hd.tcur[2 * c + ph];
+}
+// ... and become work items of the eikonal launch.  The rebuilds of one chain sit next to each other in the work list: its
+// P and S solves of one source depth grow their boxes alike (same interfaces), which is what the lanes of a warp should
+// have in common.
+__device__ __forceinline__ void queue_tables(const Handle& hd, const EvalView& v, int c, int calct)
+{
+    int item = atomicAdd(hd.n_items, (calct == 3) ? 2 : 1);
+    for (int ph = 0; ph < 2; ph++) {
+        if (!(calct & (1 << ph))) continue;
+        if (item < 2 * hd.n) {                  // cannot fail (two items per chain at most); never write past the lists
+            hd.item_chain[item] = c; hd.item_phase[item] = ph;
+            hd.item_tab[item] = hd.tab + (((size_t)v.tbuf[2 * c + ph] * hd.n + c) * 2 + ph) * hd.tab_stride;
+        }
+        item++;
+    }
+}
+
 // ---- start models (src/mcmc_eq.c:549-630) ---------------------------------------------------
-__global__ void init_chains_kernel(SamplerParams p, Handle hd, SamplerDev s)
+__global__ void init_chains_kernel(Handle hd, SamplerDev s)
 {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= p.n) return;
-    const mq_config& g = p.cfg;
-    Philox rng(p.seed, (uint32_t)(p.chain_offset + c), 0);
+    if (c >= hd.n) return;
+    const mq_config& g = hd.cfg;
+    Philox rng(hd.seed, (uint32_t)(hd.chain_offset + c), 0);
     bool ok = true;
     const float inv = (g.inv_control > 0.f) ? -g.inv_control : g.inv_control;
     s.inv_control[c] = inv;
-    float* z = hd.z + (size_t)c * p.md;     // buffer 0
-    float* vp = hd.vp + (size_t)c * p.md;
-    float* vpvs = hd.vpvs + (size_t)c * p.md;
-    float* wz = s.wz + (size_t)c * p.md; float* wp = s.wvp + (size_t)c * p.md; float* ws = s.wvs + (size_t)c * p.md;
+    float* z = hd.z + (size_t)c * hd.md;     // buffer 0
+    float* vp = hd.vp + (size_t)c * hd.md;
+    float* vpvs = hd.vpvs + (size_t)c * hd.md;
+    float* wz = s.wz + (size_t)c * hd.md; float* wp = s.wvp + (size_t)c * hd.md; float* ws = s.wvs + (size_t)c * hd.md;
     int dim = 1;
     for (int attempt = 0; attempt < 100000; attempt++) {
         if (g.start_cell_number > 1)
             dim = g.start_cell_number + (int)rng.gauss_bounded((float)g.start_cell_number, (float)g.sdev_start_cell_number,
-                                                                1.0f, (float)p.nz, &ok);
+                                                                1.0f, (float)hd.nz, &ok);
         else dim = 1;
         if (dim < 1) dim = 1;
         int first = 0;
         if (g.tria == 1) {   // two fixed nuclei at the top and the bottom of the model (src/mcmc_eq.c:577-588)
             dim += 2; first = 2;
-            z[0] = p.zmin; z[1] = p.zmax;
+            z[0] = hd.zmin; z[1] = hd.zmax;
             for (int i = 0; i < 2; i++) {
                 const float value = g.start_vp + (z[i] - g.grid.z0) * g.start_vp_grad;
                 vp[i] = value + rng.gauss_bounded(value, g.sdev_start_vp, g.vpmin, g.vpmax, &ok);
                 vpvs[i] = g.start_vpvs + rng.gauss_bounded(g.start_vpvs, g.sdev_start_vpvs, g.vpvsmin, g.vpvsmax, &ok);
             }
         }
-        if (dim > p.md) dim = p.md;
-        for (int i = first; i < dim; i++) z[i] = rng.between(p.zmin, p.zmax);
+        if (dim > hd.md) dim = hd.md;
+        for (int i = first; i < dim; i++) z[i] = rng.between(hd.zmin, hd.zmax);
         for (int i = first; i < dim; i++) {
             const float value = g.start_vp + (z[i] - g.grid.z0) * g.start_vp_grad;
             vp[i] = value + rng.gauss_bounded(value, g.sdev_start_vp, g.vpmin, g.vpmax, &ok);
             vpvs[i] = g.start_vpvs + rng.gauss_bounded(g.start_vpvs, g.sdev_start_vpvs, g.vpvsmin, g.vpvsmax, &ok);
         }
-        if (model_valid_dev(dim, z, vp, vpvs, wz, wp, ws, g.grid.h, p.zmin, p.zmax, inv) == 0) break;
+        if (model_valid_dev(dim, z, vp, vpvs, wz, wp, ws, g.grid.h, hd.zmin, hd.zmax, inv) == 0) break;
     }
     hd.dim[c] = dim;
     hd.mcur[c] = 0; hd.tcur[2 * c] = 0; hd.tcur[2 * c + 1] = 0; hd.ecur[c] = 0;
-    float* eq = hd.eq + (size_t)c * p.ne * 3;
-    const float hx = (p.xmax - p.xmin) / 2.0f, hy = (p.ymax - p.ymin) / 2.0f;
-    for (int q = 0; q < p.ne; q++) eq[3 * q] = rng.between(p.xmin + hx * (1.0f - g.r_start_eqh), p.xmin + hx * (1.0f + g.r_start_eqh));
-    for (int q = 0; q < p.ne; q++) eq[3 * q + 1] = rng.between(p.ymin + hy * (1.0f - g.r_start_eqh), p.ymin + hy * (1.0f + g.r_start_eqh));
-    for (int q = 0; q < p.ne; q++) eq[3 * q + 2] = rng.between(p.zmin, p.zmax * g.r_start_eqv);
-    for (int q = 0; q < p.ne; q++)
+    float* eq = hd.eq + (size_t)c * hd.ne * 3;
+    const float hx = (hd.xmax - hd.xmin) / 2.0f, hy = (hd.ymax - hd.ymin) / 2.0f;
+    for (int q = 0; q < hd.ne; q++) eq[3 * q] = rng.between(hd.xmin + hx * (1.0f - g.r_start_eqh), hd.xmin + hx * (1.0f + g.r_start_eqh));
+    for (int q = 0; q < hd.ne; q++) eq[3 * q + 1] = rng.between(hd.ymin + hy * (1.0f - g.r_start_eqh), hd.ymin + hy * (1.0f + g.r_start_eqh));
+    for (int q = 0; q < hd.ne; q++) eq[3 * q + 2] = rng.between(hd.zmin, hd.zmax * g.r_start_eqv);
+    for (int q = 0; q < hd.ne; q++)
         for (int k = 0; k < 3; k++)
             if (hd.pk.fix[3 * q + k] != -9999.0) eq[3 * q + k] = (float)hd.pk.fix[3 * q + k];
-    float* pres = hd.pres + (size_t)c * p.ns;
-    float* sres = hd.sres + (size_t)c * p.ns;
-    for (int i = 0; i < p.ns; i++) pres[i] = g.start_delay + rng.gauss_bounded(g.start_delay, g.sdev_start_delay, g.residual_min, g.residual_max, &ok);
-    for (int i = 0; i < p.ns; i++) sres[i] = g.start_delay + rng.gauss_bounded(g.start_delay, g.sdev_start_delay, g.residual_min, g.residual_max, &ok);
+    float* pres = hd.pres + (size_t)c * hd.ns;
+    float* sres = hd.sres + (size_t)c * hd.ns;
+    for (int i = 0; i < hd.ns; i++) pres[i] = g.start_delay + rng.gauss_bounded(g.start_delay, g.sdev_start_delay, g.residual_min, g.residual_max, &ok);
+    for (int i = 0; i < hd.ns; i++) sres[i] = g.start_delay + rng.gauss_bounded(g.start_delay, g.sdev_start_delay, g.residual_min, g.residual_max, &ok);
     if (g.scor_flag == 1 || g.scor_flag == 2) pres[g.reference_station] = g.ref_statcor_P;
     if (g.scor_flag == 2) sres[g.reference_station] = g.ref_statcor_S;
     for (int k = 0; k < 8; k++) hd.noise[8 * (size_t)c + k] = g.start_noise;
@@ -234,29 +266,27 @@ __global__ void init_chains_kernel(SamplerParams p, Handle hd, SamplerDev s)
 }
 
 // ---- proposal (src/mcmc_eq.c:856-1130) --------------------------------------------------------
-__global__ void propose_kernel(SamplerParams p, Handle hd, SamplerDev s, EvalView v, int use_override)
+__global__ void propose_kernel(Handle hd, SamplerDev s, EvalView v, int use_override)
 {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= p.n) return;
-    const mq_config& g = p.cfg;
-    const int n = p.n;
+    if (c >= hd.n) return;
+    const mq_config& g = hd.cfg;
     if (s.hold) {   // desynchronised stepping: parked chains keep their pending proposal, finished ones idle
         if (s.hold[c] == 2) { atomicAdd(&s.pass_stat[0], 1); return; }
         if (s.todo[c] <= 0) { s.hold[c] = 1; return; }
         s.hold[c] = 0;
     }
-    // default: nothing to evaluate
-    v.q_idx[c] = -1; v.r_idx[c] = -1; v.ev_only[c] = -2;
-    const int mc = hd.mcur[c], ec = hd.ecur[c];
-    v.mbuf[c] = mc; v.tbuf[2 * c] = hd.tcur[2 * c]; v.tbuf[2 * c + 1] = hd.tcur[2 * c + 1]; v.ebuf[c] = ec;
+    const CurModel m = cur_model(hd, c);
+    view_defaults(hd, v, c, m);
     s.kind[c] = 0; s.not_valid[c] = 0; s.rebuilt[c] = 0; s.log_fac[c] = 0.0;
 
     const long j = (long)s.acce[c];
     if (j >= (long)g.j_max_start + (long)g.j_max_main) return;   // chain finished (src/mcmc_eq.c:845)
 
-    Philox rng(p.seed, (uint32_t)(p.chain_offset + c), s.draws[c]);
+    Philox rng(hd.seed, (uint32_t)(hd.chain_offset + c), s.draws[c]);
     float inv = s.inv_control[c];
-    if (j == p.revert && p.lvz_flag == 1) { inv = -inv; s.inv_control[c] = inv; }   // fires every iteration while acce == revert (:849-853)
+    const int revert = (int)(g.j_max_start + g.j_max_main / 2);   // src/mcmc_eq.c:840
+    if (j == revert && hd.lvz_flag == 1) { inv = -inv; s.inv_control[c] = inv; }   // fires every iteration while acce == revert (:849-853)
 
     char kind;
     float fac;
@@ -265,15 +295,13 @@ __global__ void propose_kernel(SamplerParams p, Handle hd, SamplerDev s, EvalVie
     else { kind = s.ps_main[rng.below(s.len_main)]; fac = 1.0f; }
     s.kind[c] = kind;
 
-    const int dim = hd.dim[mc * n + c];
-    const float* z = hd.z + ((size_t)mc * n + c) * p.md;
-    const float* vp = hd.vp + ((size_t)mc * n + c) * p.md;
-    const float* vpvs = hd.vpvs + ((size_t)mc * n + c) * p.md;
-    const int mo = 1 - mc;
-    float* nz_ = hd.z + ((size_t)mo * n + c) * p.md;
-    float* nvp = hd.vp + ((size_t)mo * n + c) * p.md;
-    float* nvpvs = hd.vpvs + ((size_t)mo * n + c) * p.md;
-    float* wz = s.wz + (size_t)c * p.md; float* wp = s.wvp + (size_t)c * p.md; float* ws = s.wvs + (size_t)c * p.md;
+    const int dim = m.dim;
+    const float *z = m.z, *vp = m.vp, *vpvs = m.vpvs;
+    const size_t po = ((size_t)(1 - m.mc) * hd.n + c) * hd.md;   // the proposal's model buffer
+    float* nz_ = hd.z + po;
+    float* nvp = hd.vp + po;
+    float* nvpvs = hd.vpvs + po;
+    float* wz = s.wz + (size_t)c * hd.md; float* wp = s.wvp + (size_t)c * hd.md; float* ws = s.wvs + (size_t)c * hd.md;
     bool ok = true;
     int calct = 0, newdim = dim;
     bool model_arm = false;
@@ -281,11 +309,11 @@ __global__ void propose_kernel(SamplerParams p, Handle hd, SamplerDev s, EvalVie
 
     switch (kind) {
     case 'Q': {
-        const int idx = rng.below(p.ne);
-        const float* q = hd.eq + ((size_t)c * p.ne + idx) * 3;
-        float dx = rng.gauss_bounded(q[0], g.sdevxs * fac, p.xmin, p.xmax, &ok);
-        float dy = rng.gauss_bounded(q[1], g.sdevys * fac, p.ymin, p.ymax, &ok);
-        float dz = rng.gauss_bounded(q[2], g.sdevzs * fac, p.zmin, p.zmax, &ok);
+        const int idx = rng.below(hd.ne);
+        const float* q = hd.eq + ((size_t)c * hd.ne + idx) * 3;
+        float dx = rng.gauss_bounded(q[0], g.sdevxs * fac, hd.xmin, hd.xmax, &ok);
+        float dy = rng.gauss_bounded(q[1], g.sdevys * fac, hd.ymin, hd.ymax, &ok);
+        float dz = rng.gauss_bounded(q[2], g.sdevzs * fac, hd.zmin, hd.zmax, &ok);
         if (hd.pk.fix[3 * idx] != -9999.0) dx = 0.f;
         if (hd.pk.fix[3 * idx + 1] != -9999.0) dy = 0.f;
         if (hd.pk.fix[3 * idx + 2] != -9999.0) dz = 0.f;
@@ -295,9 +323,9 @@ __global__ void propose_kernel(SamplerParams p, Handle hd, SamplerDev s, EvalVie
         break;
     }
     case 'R': {
-        const int idx = rng.below(p.ns);
-        float dx = rng.gauss_bounded(hd.pres[(size_t)c * p.ns + idx], g.sdevresidual, g.residual_min, g.residual_max, &ok);
-        float dy = rng.gauss_bounded(hd.sres[(size_t)c * p.ns + idx], g.sdevresidual, g.residual_min, g.residual_max, &ok);
+        const int idx = rng.below(hd.ns);
+        float dx = rng.gauss_bounded(hd.pres[(size_t)c * hd.ns + idx], g.sdevresidual, g.residual_min, g.residual_max, &ok);
+        float dy = rng.gauss_bounded(hd.sres[(size_t)c * hd.ns + idx], g.sdevresidual, g.residual_min, g.residual_max, &ok);
         if (g.scor_flag == -1) dy = 0.f;
         if (g.scor_flag == -2) dx = 0.f;
         float dx2 = 0.f, dy2 = 0.f;
@@ -310,7 +338,7 @@ __global__ void propose_kernel(SamplerParams p, Handle hd, SamplerDev s, EvalVie
         }
         v.r_idx[c] = idx;
         v.r_d[4 * c] = dx; v.r_d[4 * c + 1] = dy; v.r_d[4 * c + 2] = dx2; v.r_d[4 * c + 3] = dy2;
-        v.ev_only[c] = -1; v.ebuf[c] = 1 - ec;
+        v.ev_only[c] = -1; v.ebuf[c] = 1 - m.ec;
         break;
     }
     case 'P': case 'V': case 'M': {
@@ -323,8 +351,8 @@ __global__ void propose_kernel(SamplerParams p, Handle hd, SamplerDev s, EvalVie
             const int idx = (kind == 'M') ? fixed + rng.below(dim - fixed) : rng.below(dim);
             if (kind == 'P') nvp[idx] = vp[idx] + rng.gauss_bounded(vp[idx], g.sdevvp, g.vpmin, g.vpmax, &ok);
             else if (kind == 'V') nvpvs[idx] = vpvs[idx] + rng.gauss_bounded(vpvs[idx], g.sdevvpvs, g.vpvsmin, g.vpvsmax, &ok);
-            else nz_[idx] = z[idx] + rng.gauss_bounded(z[idx], g.sdevz, p.zmin, p.zmax, &ok);
-            if (model_valid_dev(dim, nz_, nvp, nvpvs, wz, wp, ws, g.grid.h, p.zmin, p.zmax, inv) == 0) break;
+            else nz_[idx] = z[idx] + rng.gauss_bounded(z[idx], g.sdevz, hd.zmin, hd.zmax, &ok);
+            if (model_valid_dev(dim, nz_, nvp, nvpvs, wz, wp, ws, g.grid.h, hd.zmin, hd.zmax, inv) == 0) break;
         }
         if (t == kMaxTries) ok = false;
         calct = (kind == 'V') ? 2 : 3;
@@ -332,16 +360,16 @@ __global__ void propose_kernel(SamplerParams p, Handle hd, SamplerDev s, EvalVie
         break;
     }
     case 'B': {
-        if (!((double)(dim + 1) < ((double)g.max_dim / (1.0 + sqrt((double)(inv * inv))))) || dim + 1 > p.md) { s.not_valid[c] = 1; break; }
+        if (!((double)(dim + 1) < ((double)g.max_dim / (1.0 + sqrt((double)(inv * inv))))) || dim + 1 > hd.md) { s.not_valid[c] = 1; break; }
         int t, idx = 0;
         for (t = 0; t < kMaxTries; t++) {
             for (int i = 0; i < dim; i++) { nz_[i] = z[i]; nvp[i] = vp[i]; nvpvs[i] = vpvs[i]; }
-            const float newz = rng.between(p.zmin, p.zmax);
+            const float newz = rng.between(hd.zmin, hd.zmax);
             idx = find_in_cell_dev(z, dim, newz);
             const float dvp = rng.gauss_bounded(vp[idx], g.sdevvp, g.vpmin, g.vpmax, &ok);
             const float dvs = rng.gauss_bounded(vpvs[idx], g.sdevvpvs, g.vpvsmin, g.vpvsmax, &ok);
             nvp[dim] = vp[idx] + dvp; nvpvs[dim] = vpvs[idx] + dvs; nz_[dim] = newz;
-            if (model_valid_dev(dim + 1, nz_, nvp, nvpvs, wz, wp, ws, g.grid.h, p.zmin, p.zmax, inv) == 0) break;
+            if (model_valid_dev(dim + 1, nz_, nvp, nvpvs, wz, wp, ws, g.grid.h, hd.zmin, hd.zmax, inv) == 0) break;
         }
         if (t == kMaxTries) ok = false;
         newdim = dim + 1;
@@ -372,7 +400,7 @@ __global__ void propose_kernel(SamplerParams p, Handle hd, SamplerDev s, EvalVie
                 lf = lf + log((double)((g.vpvsmax - g.vpvsmin) / g.sdevvpvs) / sqrt(2.0 * MQ_PI)) -
                      (double)(ds * ds) / 2.0 / (double)g.sdevvpvs / (double)g.sdevvpvs;
             for (int i = 0, k = 0; i < dim; i++) if (i != dead) { nz_[k] = z[i]; nvp[k] = vp[i]; nvpvs[k] = vpvs[i]; k++; }
-            if (model_valid_dev(dim - 1, nz_, nvp, nvpvs, wz, wp, ws, g.grid.h, p.zmin, p.zmax, inv) == 0) break;
+            if (model_valid_dev(dim - 1, nz_, nvp, nvpvs, wz, wp, ws, g.grid.h, hd.zmin, hd.zmax, inv) == 0) break;
         }
         if (t == kMaxTries) ok = false;
         newdim = dim - 1;
@@ -386,7 +414,7 @@ __global__ void propose_kernel(SamplerParams p, Handle hd, SamplerDev s, EvalVie
         double lf = 0.0;
         // draw order p0,s0,p1,s1,... == index order 2*class+phase (:1097-1112)
         for (int k = 0; k < 8; k++) nn[k] = o[k] + rng.gauss_bounded(o[k], g.sdevn, g.noise_min, g.noise_max, &ok);
-        for (int k = 0; k < 8; k++) lf = lf + (double)p.n_class[k] * log((double)(o[k] / nn[k]));
+        for (int k = 0; k < 8; k++) lf = lf + (double)hd.n_class[k] * log((double)(o[k] / nn[k]));
         s.log_fac[c] = lf;
         v.ev_only[c] = -2;
         break;
@@ -395,31 +423,15 @@ __global__ void propose_kernel(SamplerParams p, Handle hd, SamplerDev s, EvalVie
     }
 
     if (model_arm) {
-        hd.dim[mo * n + c] = newdim;
-        v.mbuf[c] = mo;
-        v.ev_only[c] = -1; v.ebuf[c] = 1 - ec;
-        s.rebuilt[c] = calct;
+        view_model_arm(hd, s, v, c, m, newdim, calct);
         // a proposal whose retry loop gave up (!ok) is rejected without being evaluated: it queues no table rebuild
-        if (p.cfg.eikonal == 1 && p.cfg.aflag != 1 && ok) {
-            const bool park = s.hold != nullptr;      // the tables are built later, together with those of other parked chains
-            // the rebuilds of one chain sit next to each other in the work list: its P and S solves of one source depth
-            // grow their boxes alike (same interfaces), which is what the lanes of a warp should have in common
-            int item = park ? 0 : atomicAdd(hd.n_items, (calct == 3) ? 2 : 1);
-            for (int ph = 0; ph < 2; ph++) {
-                if (!(calct & (1 << ph))) continue;
-                const int tb = 1 - hd.tcur[2 * c + ph];
-                v.tbuf[2 * c + ph] = tb;
-                if (park) continue;
-                if (item < 2 * n) {                  // cannot fail (two items per chain at most); never write past the lists
-                    hd.item_chain[item] = c; hd.item_phase[item] = ph;
-                    hd.item_tab[item] = hd.tab + (((size_t)tb * n + c) * 2 + ph) * p.tab_stride;
-                }
-                item++;
-            }
-            if (park && calct) s.hold[c] = 2;
+        if (g.eikonal == 1 && g.aflag != 1 && ok) {
+            flip_tables(hd, v, c, calct);
+            if (s.hold) s.hold[c] = 2;   // the tables are built later, together with those of other parked chains
+            else queue_tables(hd, v, c, calct);
         }
     }
-    if (p.cfg.aflag == 1) v.ev_only[c] = -2;   // prior sampling: no likelihood (src/misfit.c:61)
+    if (g.aflag == 1) v.ev_only[c] = -2;   // prior sampling: no likelihood (src/misfit.c:61)
     if (!ok) { s.not_valid[c] = 2; v.ev_only[c] = -2; }   // a retry loop gave up: rejected whatever aflag (accept_kernel)
     s.draws[c] = rng.draws;
     if (s.hold) {
@@ -430,90 +442,69 @@ __global__ void propose_kernel(SamplerParams p, Handle hd, SamplerDev s, EvalVie
 
 // Desynchronised stepping, the pass that builds tables: every parked chain queues its table rebuilds and is evaluated
 // and decided in this pass, every other chain idles.
-__global__ void flush_parked_kernel(SamplerParams p, Handle hd, SamplerDev s, EvalView v)
+__global__ void flush_parked_kernel(Handle hd, SamplerDev s, EvalView v)
 {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= p.n) return;
+    if (c >= hd.n) return;
     if (s.hold[c] != 2) {
         s.hold[c] = 1;
         if (s.todo[c] > 0) atomicAdd(&s.pass_stat[1], 1);
         return;
     }
     s.hold[c] = 0;
-    const int calct = s.rebuilt[c];
-    int item = calct ? atomicAdd(hd.n_items, (calct == 3) ? 2 : 1) : 0;
-    for (int ph = 0; ph < 2; ph++) {
-        if (!(calct & (1 << ph))) continue;
-        hd.item_chain[item] = c; hd.item_phase[item] = ph;
-        hd.item_tab[item] = hd.tab + (((size_t)v.tbuf[2 * c + ph] * p.n + c) * 2 + ph) * p.tab_stride;
-        item++;
-    }
+    queue_tables(hd, v, c, s.rebuilt[c]);   // propose_kernel chose the table buffers when the chain parked
     if (s.todo[c] > 1) atomicAdd(&s.pass_stat[1], 1);
 }
 
 // ---- replay: the proposal comes from a recorded stream instead of the RNG ------------------------------
 // Fills exactly what propose_kernel fills, from injected data: s.kind[c] the arm, the proposed model in the work
-// arrays s.wz/wvp/wvs (+ dim_in), the proposed event in v.q_xyz (+ s.r_qidx), the proposed station corrections in
+// arrays s.wz/wvp/wvs (+ s.r_dim), the proposed event in v.q_xyz (+ s.r_qidx), the proposed station corrections in
 // v.pres_over/sres_over, the proposed sigmas in s.noise_new, the proposal ratio in s.log_fac.  No validity test and no
 // eligibility test: the recorded proposals passed the reference's own (src/mcmc_eq.c:945-951,1021,1059).
-__global__ void replay_setup_kernel(SamplerParams p, Handle hd, SamplerDev s, EvalView v, const int32_t* dim_in)
+__global__ void replay_setup_kernel(Handle hd, SamplerDev s, EvalView v)
 {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= p.n) return;
-    const int n = p.n;
-    const int d_in = dim_in[c];   // may alias s.rebuilt: read before that is reset
-    v.q_idx[c] = -1; v.r_idx[c] = -1; v.ev_only[c] = -2;
-    const int mc = hd.mcur[c], ec = hd.ecur[c];
-    v.mbuf[c] = mc; v.tbuf[2 * c] = hd.tcur[2 * c]; v.tbuf[2 * c + 1] = hd.tcur[2 * c + 1]; v.ebuf[c] = ec;
+    if (c >= hd.n) return;
+    const CurModel m = cur_model(hd, c);
+    view_defaults(hd, v, c, m);
     s.not_valid[c] = 0; s.rebuilt[c] = 0;
     const char kind = (char)s.kind[c];
     if (kind == 0) return;
     int calct = 0;
     switch (kind) {
     case 'Q': v.q_idx[c] = s.r_qidx[c]; v.ev_only[c] = s.r_qidx[c]; break;      // v.q_xyz was uploaded
-    case 'R': v.r_idx[c] = -2; v.ev_only[c] = -1; v.ebuf[c] = 1 - ec; break;
+    case 'R': v.r_idx[c] = -2; v.ev_only[c] = -1; v.ebuf[c] = 1 - m.ec; break;
     case 'N': v.ev_only[c] = -2; break;
     case 'V': calct = 2; break;
     case 'P': case 'M': case 'B': case 'D': calct = 3; break;
     default: s.not_valid[c] = 1; break;
     }
     if (calct) {
-        const int mo = 1 - mc, d = d_in;
-        float* nz_ = hd.z + ((size_t)mo * n + c) * p.md;
-        float* nvp = hd.vp + ((size_t)mo * n + c) * p.md;
-        float* nvpvs = hd.vpvs + ((size_t)mo * n + c) * p.md;
-        for (int i = 0; i < d; i++) { nz_[i] = s.wz[(size_t)c * p.md + i]; nvp[i] = s.wvp[(size_t)c * p.md + i]; nvpvs[i] = s.wvs[(size_t)c * p.md + i]; }
-        hd.dim[mo * n + c] = d;
-        v.mbuf[c] = mo; v.ev_only[c] = -1; v.ebuf[c] = 1 - ec;
-        s.rebuilt[c] = calct;
-        if (p.cfg.eikonal == 1 && p.cfg.aflag != 1) {
-            int item = atomicAdd(hd.n_items, (calct == 3) ? 2 : 1);
-            for (int ph = 0; ph < 2; ph++) {
-                if (!(calct & (1 << ph))) continue;
-                const int tb = 1 - hd.tcur[2 * c + ph];
-                v.tbuf[2 * c + ph] = tb;
-                hd.item_chain[item] = c; hd.item_phase[item] = ph;
-                hd.item_tab[item] = hd.tab + (((size_t)tb * n + c) * 2 + ph) * p.tab_stride;
-                item++;
-            }
+        const int d = s.r_dim[c];
+        const size_t po = ((size_t)(1 - m.mc) * hd.n + c) * hd.md, wo = (size_t)c * hd.md;
+        for (int i = 0; i < d; i++) { hd.z[po + i] = s.wz[wo + i]; hd.vp[po + i] = s.wvp[wo + i]; hd.vpvs[po + i] = s.wvs[wo + i]; }
+        view_model_arm(hd, s, v, c, m, d, calct);
+        if (hd.cfg.eikonal == 1 && hd.cfg.aflag != 1) {
+            flip_tables(hd, v, c, calct);
+            queue_tables(hd, v, c, calct);
         }
     }
-    if (p.cfg.aflag == 1) v.ev_only[c] = -2;
+    if (hd.cfg.aflag == 1) v.ev_only[c] = -2;
 }
 
 // ---- accept / reject (src/mcmc_eq.c:1135-1191) -------------------------------------------------
-__global__ void accept_kernel(SamplerParams p, Handle hd, SamplerDev s, EvalView v)
+__global__ void accept_kernel(Handle hd, SamplerDev s, EvalView v)
 {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= p.n) return;
+    if (c >= hd.n) return;
     if (s.hold) {   // desynchronised stepping: only chains evaluated in this pass are decided; an iteration is used up
         if (s.hold[c] != 0) return;
         s.todo[c]--;
     }
     const char kind = (char)s.kind[c];
     if (kind == 0) return;   // finished chain
-    const mq_config& g = p.cfg;
-    const int n = p.n;
+    const mq_config& g = hd.cfg;
+    const int n = hd.n;
     int64_t* cnt = s.counts + 20 * (size_t)c;
     const int slot = (kind == 'N') ? 0 : (kind == 'P') ? 1 : (kind == 'V') ? 2 : (kind == 'Q') ? 3 : (kind == 'R') ? 4
                    : (kind == 'M') ? 5 : (kind == 'B') ? 6 : 7;
@@ -527,7 +518,7 @@ __global__ void accept_kernel(SamplerParams p, Handle hd, SamplerDev s, EvalView
     } else {
         for (int k = 0; k < 8; k++) mf[k] = (g.aflag == 1) ? 0.f : hd.mf_eval[8 * (size_t)c + k];
         new_misfit = chain_misfit(mf, noise);
-        new_rms = chain_rms(mf, p.sum_of_picks);
+        new_rms = chain_rms(mf, hd.sum_of_picks);
         new_ll = -new_misfit / 2.0;
         // parallel tempering (comm.cu): the likelihood enters with the chain's inverse temperature; for the noise arm
         // log_fac is the likelihood's normalisation term (src/mcmc_eq.c:1114-1117) and is tempered with it.  beta == 1
@@ -545,7 +536,7 @@ __global__ void accept_kernel(SamplerParams p, Handle hd, SamplerDev s, EvalView
     float u;
     if (s.u_inject) u = s.u_inject[c];   // replay: the reference's own deviate, no draw is consumed
     else {
-        Philox rng(p.seed, (uint32_t)(p.chain_offset + c), s.draws[c]);
+        Philox rng(hd.seed, (uint32_t)(hd.chain_offset + c), s.draws[c]);
         u = rng.uniform();
         s.draws[c] = rng.draws;
     }
@@ -559,24 +550,24 @@ __global__ void accept_kernel(SamplerParams p, Handle hd, SamplerDev s, EvalView
         // apply the proposal
         if (kind == 'Q') {
             const int idx = v.q_idx[c];
-            float* q = hd.eq + ((size_t)c * p.ne + idx) * 3;
+            float* q = hd.eq + ((size_t)c * hd.ne + idx) * 3;
             q[0] = v.q_xyz[3 * c]; q[1] = v.q_xyz[3 * c + 1]; q[2] = v.q_xyz[3 * c + 2];
             if (g.aflag != 1) {
                 const int ec = hd.ecur[c];
-                float* es = hd.evsum + (((size_t)ec * n + c) * p.ne + idx) * 8;
+                float* es = hd.evsum + (((size_t)ec * n + c) * hd.ne + idx) * 8;
                 for (int k = 0; k < 8; k++) es[k] = hd.evq[8 * (size_t)c + k];
-                hd.origin[((size_t)ec * n + c) * p.ne + idx] = hd.oq[c];
+                hd.origin[((size_t)ec * n + c) * hd.ne + idx] = hd.oq[c];
             }
         } else if (kind == 'R') {
             const int idx = v.r_idx[c];
             const float dx = v.r_d[4 * c], dy = v.r_d[4 * c + 1], dx2 = v.r_d[4 * c + 2], dy2 = v.r_d[4 * c + 3];
-            float* pres = hd.pres + (size_t)c * p.ns;
-            float* sres = hd.sres + (size_t)c * p.ns;
-            const float nsm1 = (float)(p.ns - 1);
+            float* pres = hd.pres + (size_t)c * hd.ns;
+            float* sres = hd.sres + (size_t)c * hd.ns;
+            const float nsm1 = (float)(hd.ns - 1);
             if (idx == -2) {   // replay: the proposed corrections were given in full
-                for (int k = 0; k < p.ns; k++) { pres[k] = v.pres_over[(size_t)c * p.ns + k]; sres[k] = v.sres_over[(size_t)c * p.ns + k]; }
+                for (int k = 0; k < hd.ns; k++) { pres[k] = v.pres_over[(size_t)c * hd.ns + k]; sres[k] = v.sres_over[(size_t)c * hd.ns + k]; }
             } else if (g.scor_flag <= 0)
-                for (int k = 0; k < p.ns; k++) {
+                for (int k = 0; k < hd.ns; k++) {
                     pres[k] = (k == idx) ? __fadd_rn(pres[k], dx) : __fsub_rn(pres[k], __fdiv_rn(dx, nsm1));
                     sres[k] = (k == idx) ? __fadd_rn(sres[k], dy) : __fsub_rn(sres[k], __fdiv_rn(dy, nsm1));
                 }
@@ -611,43 +602,41 @@ __global__ void accept_kernel(SamplerParams p, Handle hd, SamplerDev s, EvalView
 }
 
 // ---- snapshots: one block per chain copies the current state when asked to ----------------------
-__device__ void snapshot_copy(const SamplerParams& p, const Handle& hd, const Snapshot& d, int c)
+__device__ void snapshot_copy(const Handle& hd, const Snapshot& d, int c)
 {
-    const int n = p.n, mc = hd.mcur[c], ec = hd.ecur[c];
-    const int dim = hd.dim[mc * n + c];
-    const size_t mo = ((size_t)mc * n + c) * p.md;
-    for (int i = threadIdx.x; i < dim; i += blockDim.x) {
-        d.z[(size_t)c * p.md + i] = hd.z[mo + i]; d.vp[(size_t)c * p.md + i] = hd.vp[mo + i]; d.vpvs[(size_t)c * p.md + i] = hd.vpvs[mo + i];
+    const CurModel m = cur_model(hd, c);
+    const int md = hd.md, ne = hd.ne, ns = hd.ns;
+    for (int i = threadIdx.x; i < m.dim; i += blockDim.x) {
+        d.z[(size_t)c * md + i] = m.z[i]; d.vp[(size_t)c * md + i] = m.vp[i]; d.vpvs[(size_t)c * md + i] = m.vpvs[i];
     }
-    for (int i = threadIdx.x; i < 3 * p.ne; i += blockDim.x) d.eq[(size_t)c * p.ne * 3 + i] = hd.eq[(size_t)c * p.ne * 3 + i];
-    for (int i = threadIdx.x; i < p.ne; i += blockDim.x) d.origin[(size_t)c * p.ne + i] = hd.origin[((size_t)ec * n + c) * p.ne + i];
-    for (int i = threadIdx.x; i < p.ns; i += blockDim.x) { d.pres[(size_t)c * p.ns + i] = hd.pres[(size_t)c * p.ns + i]; d.sres[(size_t)c * p.ns + i] = hd.sres[(size_t)c * p.ns + i]; }
+    for (int i = threadIdx.x; i < 3 * ne; i += blockDim.x) d.eq[(size_t)c * ne * 3 + i] = hd.eq[(size_t)c * ne * 3 + i];
+    for (int i = threadIdx.x; i < ne; i += blockDim.x) d.origin[(size_t)c * ne + i] = m.origin[i];
+    for (int i = threadIdx.x; i < ns; i += blockDim.x) { d.pres[(size_t)c * ns + i] = hd.pres[(size_t)c * ns + i]; d.sres[(size_t)c * ns + i] = hd.sres[(size_t)c * ns + i]; }
     if (threadIdx.x < 8) d.noise[8 * (size_t)c + threadIdx.x] = hd.noise[8 * (size_t)c + threadIdx.x];
-    if (threadIdx.x == 0) d.dim[c] = dim;
+    if (threadIdx.x == 0) d.dim[c] = m.dim;
 }
 
 // The chain's current state as one packed record (layout: struct Ring).
-__device__ void record_write(const SamplerParams& p, const Handle& hd, const Ring& R, int c, float* rec)
+__device__ void record_write(const Handle& hd, const Ring& R, int c, float* rec)
 {
-    const int n = p.n, mc = hd.mcur[c], ec = hd.ecur[c];
-    const int dim = hd.dim[mc * n + c];
-    const size_t mo = ((size_t)mc * n + c) * p.md;
+    const CurModel m = cur_model(hd, c);
+    const int md = hd.md, ne = hd.ne, ns = hd.ns;
     if (threadIdx.x == 0) {
         int32_t* hi = (int32_t*)rec;
-        hi[0] = c; hi[1] = R.code[c]; hi[2] = dim; hi[3] = 0;
+        hi[0] = c; hi[1] = R.code[c]; hi[2] = m.dim; hi[3] = 0;
         *(int64_t*)(rec + 4) = R.number[c];
         *(double*)(rec + 6) = R.rms[c];
     }
     float* o = rec + kRecHead;
     if (threadIdx.x < 8) o[threadIdx.x] = hd.noise[8 * (size_t)c + threadIdx.x];
     o += 8;
-    for (int i = threadIdx.x; i < dim; i += blockDim.x) { o[i] = hd.z[mo + i]; o[p.md + i] = hd.vp[mo + i]; o[2 * p.md + i] = hd.vpvs[mo + i]; }
-    o += 3 * p.md;
-    for (int i = threadIdx.x; i < 3 * p.ne; i += blockDim.x) o[i] = hd.eq[(size_t)c * p.ne * 3 + i];
-    o += 3 * p.ne;
-    for (int i = threadIdx.x; i < p.ne; i += blockDim.x) o[i] = hd.origin[((size_t)ec * n + c) * p.ne + i];
-    o += p.ne;
-    for (int i = threadIdx.x; i < p.ns; i += blockDim.x) { o[i] = hd.pres[(size_t)c * p.ns + i]; o[p.ns + i] = hd.sres[(size_t)c * p.ns + i]; }
+    for (int i = threadIdx.x; i < m.dim; i += blockDim.x) { o[i] = m.z[i]; o[md + i] = m.vp[i]; o[2 * md + i] = m.vpvs[i]; }
+    o += 3 * md;
+    for (int i = threadIdx.x; i < 3 * ne; i += blockDim.x) o[i] = hd.eq[(size_t)c * ne * 3 + i];
+    o += 3 * ne;
+    for (int i = threadIdx.x; i < ne; i += blockDim.x) o[i] = m.origin[i];
+    o += ne;
+    for (int i = threadIdx.x; i < ns; i += blockDim.x) { o[i] = hd.pres[(size_t)c * ns + i]; o[ns + i] = hd.sres[(size_t)c * ns + i]; }
 }
 
 // Drain, device side (copy stream): the published records [rd, wr) of every chain move to the staging buffer, one
@@ -712,22 +701,21 @@ __device__ void node_velocity(const mq_config& g, const float* z, const float* v
 // analyse_eq pass 1 for one decimated model (src/analyse_eq.c:564-640): per depth node the velocity of the nearest
 // nucleus, clipped to the prior range, goes into the Vp and Vp/Vs histograms; hypocentres, origin times, station
 // corrections and sigmas into running sums.
-__device__ void posterior_accumulate(const SamplerParams& p, const Handle& hd, int c)
+__device__ void posterior_accumulate(const Handle& hd, int c)
 {
     const Posterior& P = hd.post;
-    const int n = p.n, mc = hd.mcur[c], ec = hd.ecur[c];
-    const int dim = hd.dim[mc * n + c];
-    const size_t mo = ((size_t)mc * n + c) * p.md;
-    const float* z = hd.z + mo; const float* vp = hd.vp + mo; const float* vpvs = hd.vpvs + mo;
+    const CurModel m = cur_model(hd, c);
+    const int dim = m.dim, nz = hd.nz, ne = hd.ne, ns = hd.ns;
+    const float *z = m.z, *vp = m.vp, *vpvs = m.vpvs;
     int32_t* hist_vp = P.iblock;
-    int32_t* hist_vs = hist_vp + (size_t)P.ndv * p.nz;
-    int32_t* boundary = hist_vs + (size_t)P.ndvpvs * p.nz;
+    int32_t* hist_vs = hist_vp + (size_t)P.ndv * nz;
+    int32_t* boundary = hist_vs + (size_t)P.ndvpvs * nz;
     double* vsum = P.dblock;
-    double* eqsum = vsum + 4 * (size_t)p.nz;
-    double* ressum = eqsum + 8 * (size_t)p.ne;
-    double* noisesum = ressum + 4 * (size_t)p.ns;
-    const mq_config& g = p.cfg;
-    for (int i = threadIdx.x; i < p.nz; i += blockDim.x) {
+    double* eqsum = vsum + 4 * (size_t)nz;
+    double* ressum = eqsum + 8 * (size_t)ne;
+    double* noisesum = ressum + 4 * (size_t)ns;
+    const mq_config& g = hd.cfg;
+    for (int i = threadIdx.x; i < nz; i += blockDim.x) {
         float vv, rr;
         int k;
         node_velocity(g, z, vp, vpvs, dim, i, &vv, &rr, &k);
@@ -737,20 +725,20 @@ __device__ void posterior_accumulate(const SamplerParams& p, const Handle& hd, i
         }
         int j = (int)__fdiv_rn(__fsub_rn(vv, g.vpmin), P.dv);
         if (j > P.ndv - 1) j = P.ndv - 1;
-        atomicAdd(&hist_vp[(size_t)j * p.nz + i], 1);
+        atomicAdd(&hist_vp[(size_t)j * nz + i], 1);
         j = (int)__fdiv_rn(__fsub_rn(rr, g.vpvsmin), P.dvpvs);
         if (j > P.ndvpvs - 1) j = P.ndvpvs - 1;
-        atomicAdd(&hist_vs[(size_t)j * p.nz + i], 1);
+        atomicAdd(&hist_vs[(size_t)j * nz + i], 1);
         atomicAdd(&vsum[4 * i], (double)vv); atomicAdd(&vsum[4 * i + 1], (double)vv * vv);
         atomicAdd(&vsum[4 * i + 2], (double)rr); atomicAdd(&vsum[4 * i + 3], (double)rr * rr);
     }
-    for (int e = threadIdx.x; e < p.ne; e += blockDim.x) {
-        const float* q = hd.eq + ((size_t)c * p.ne + e) * 3;
-        const double v[4] = {q[0], q[1], q[2], hd.origin[((size_t)ec * n + c) * p.ne + e]};
+    for (int e = threadIdx.x; e < ne; e += blockDim.x) {
+        const float* q = hd.eq + ((size_t)c * ne + e) * 3;
+        const double v[4] = {q[0], q[1], q[2], m.origin[e]};
         for (int k = 0; k < 4; k++) { atomicAdd(&eqsum[8 * e + k], v[k]); atomicAdd(&eqsum[8 * e + 4 + k], v[k] * v[k]); }
     }
-    for (int i = threadIdx.x; i < p.ns; i += blockDim.x) {
-        const double a = hd.pres[(size_t)c * p.ns + i], b = hd.sres[(size_t)c * p.ns + i];
+    for (int i = threadIdx.x; i < ns; i += blockDim.x) {
+        const double a = hd.pres[(size_t)c * ns + i], b = hd.sres[(size_t)c * ns + i];
         atomicAdd(&ressum[4 * i], a); atomicAdd(&ressum[4 * i + 1], b);
         atomicAdd(&ressum[4 * i + 2], a * a); atomicAdd(&ressum[4 * i + 3], b * b);
     }
@@ -765,14 +753,11 @@ __device__ void posterior_accumulate(const SamplerParams& p, const Handle& hd, i
 // sigmas, then Vp and Vp/Vs per depth node, x y z t per event, P and S correction per station) goes into the chain's open
 // batch slot as d = x - ref.  Threads over quantities; each (chain, quantity) is summed in the same order whatever the
 // stepping, so the accumulators are a function of the chain's records alone.
-__device__ void diag_accumulate(const SamplerParams& p, const Handle& hd, const Ring& R, int c)
+__device__ void diag_accumulate(const Handle& hd, const Ring& R, int c)
 {
     const Diag& D = hd.diag;
-    const int n = p.n, mc = hd.mcur[c], ec = hd.ecur[c];
-    const int dim = hd.dim[mc * n + c];
-    const size_t mo = ((size_t)mc * n + c) * p.md;
-    const float* z = hd.z + mo; const float* vp = hd.vp + mo; const float* vpvs = hd.vpvs + mo;
-    const int Q = D.Q, K = D.K, nz = p.nz, ne = p.ne;
+    const CurModel cm = cur_model(hd, c);
+    const int Q = D.Q, K = D.K, nz = hd.nz, ne = hd.ne;
     const int64_t m = D.n_models[c];
     const int k = D.full_batches[c], L = D.batch_len[c];
     const bool fills = m + 1 - (int64_t)k * L == L;          // this model fills the open slot
@@ -782,20 +767,20 @@ __device__ void diag_accumulate(const SamplerParams& p, const Handle& hd, const 
     for (int q = threadIdx.x; q < Q; q += blockDim.x) {
         double x;
         if (q == 0) x = R.rms[c];
-        else if (q == 1) x = (double)dim;
+        else if (q == 1) x = (double)cm.dim;
         else if (q < 10) x = (double)hd.noise[8 * (size_t)c + q - 2];
         else if (q < 10 + 2 * nz) {
             const int i = (q - 10) % nz;
             float vv, rr;
             int near;
-            node_velocity(p.cfg, z, vp, vpvs, dim, i, &vv, &rr, &near);
+            node_velocity(hd.cfg, cm.z, cm.vp, cm.vpvs, cm.dim, i, &vv, &rr, &near);
             x = (double)(q < 10 + nz ? vv : rr);
         } else if (q < 10 + 2 * nz + 4 * ne) {
             const int e = (q - 10 - 2 * nz) >> 2, j = (q - 10 - 2 * nz) & 3;
-            x = (double)(j < 3 ? hd.eq[((size_t)c * ne + e) * 3 + j] : hd.origin[((size_t)ec * n + c) * ne + e]);
+            x = (double)(j < 3 ? hd.eq[((size_t)c * ne + e) * 3 + j] : cm.origin[e]);
         } else {
             const int st = (q - 10 - 2 * nz - 4 * ne) >> 1;
-            x = (double)((q & 1) == 0 ? hd.pres[(size_t)c * p.ns + st] : hd.sres[(size_t)c * p.ns + st]);
+            x = (double)((q & 1) == 0 ? hd.pres[(size_t)c * hd.ns + st] : hd.sres[(size_t)c * hd.ns + st]);
         }
         if (m == 0) ref[q] = x;
         const double d = __dsub_rn(x, ref[q]);
@@ -819,16 +804,16 @@ __device__ void diag_accumulate(const SamplerParams& p, const Handle& hd, const 
     }
 }
 
-__global__ void snapshot_kernel(SamplerParams p, Handle hd, SamplerDev s)
+__global__ void snapshot_kernel(Handle hd, SamplerDev s)
 {
     const int c = blockIdx.x;
     const int pend = s.ring.pend[c];
     if (pend) {
-        if (hd.post.on && (long long)s.ring.number[c] > hd.post.burn_in) posterior_accumulate(p, hd, c);
-        if (hd.diag.on && (long long)s.ring.number[c] > hd.diag.burn_in) diag_accumulate(p, hd, s.ring, c);
+        if (hd.post.on && (long long)s.ring.number[c] > hd.post.burn_in) posterior_accumulate(hd, c);
+        if (hd.diag.on && (long long)s.ring.number[c] > hd.diag.burn_in) diag_accumulate(hd, s.ring, c);
         if (pend == 1) {
             const int wr = s.ring.wr[c];
-            record_write(p, hd, s.ring, c, s.ring.data + ((size_t)c * s.ring.slots + wr % s.ring.slots) * s.ring.rec_floats);
+            record_write(hd, s.ring, c, s.ring.data + ((size_t)c * s.ring.slots + wr % s.ring.slots) * s.ring.rec_floats);
             __threadfence();
             __syncthreads();
             if (threadIdx.x == 0) *(volatile int32_t*)&s.ring.wr[c] = wr + 1;   // published: a drain may take it
@@ -837,7 +822,7 @@ __global__ void snapshot_kernel(SamplerParams p, Handle hd, SamplerDev s)
         if (threadIdx.x == 0) s.ring.pend[c] = 0;
     }
     if (s.best.flag[c] >= 2) {
-        snapshot_copy(p, hd, s.best, c);
+        snapshot_copy(hd, s.best, c);
         __syncthreads();
         if (threadIdx.x == 0) s.best.flag[c] = 1;
     }
@@ -937,7 +922,8 @@ int sampler_get(Handle* h, Sampler** out)
         TRY(cudaEventCreateWithFlags(&s->ev_main, cudaEventDisableTiming));
         memset(s->batch, 0, sizeof s->batch);
     }
-    TRY(dz(&s->r_alpha, n)); TRY(dz(&s->r_accept, n)); TRY(dz(&s->r_newll, n)); TRY(dz(&s->r_qidx, n));
+    TRY(dz(&s->u_buf, n)); TRY(dz(&s->r_alpha, n)); TRY(dz(&s->r_accept, n)); TRY(dz(&s->r_newll, n)); TRY(dz(&s->r_qidx, n));
+    TRY(dz(&s->r_dim, n));
     TRY(dz(&s->todo_buf, n)); TRY(dz(&s->hold_buf, n)); TRY(dz(&s->stat_buf, 2));
     const std::string a = balance(h->cfg.dstring_start, h->ne, h->ns, 10), b = balance(h->cfg.dstring_main, h->ne, h->ns, 20);
     s->len_start = (int)a.size(); s->len_main = (int)b.size();
@@ -976,7 +962,7 @@ void sampler_destroy(Handle* h)
     if (s->ev_main) cudaEventDestroy(s->ev_main);
     if (s->copy_stream) cudaStreamDestroy(s->copy_stream);
     cudaFree(s->ps_start); cudaFree(s->ps_main); cudaFree(s->ps_over);
-    cudaFree(s->u_inject); cudaFree(s->r_alpha); cudaFree(s->r_accept); cudaFree(s->r_newll); cudaFree(s->r_qidx);
+    cudaFree(s->u_buf); cudaFree(s->r_alpha); cudaFree(s->r_accept); cudaFree(s->r_newll); cudaFree(s->r_qidx); cudaFree(s->r_dim);
     cudaFree(s->todo_buf); cudaFree(s->hold_buf); cudaFree(s->stat_buf);
     cudaFree(h->prop_view.pres_over); cudaFree(h->prop_view.sres_over);
     h->prop_view.pres_over = nullptr; h->prop_view.sres_over = nullptr;
@@ -996,12 +982,19 @@ static int start_sampler_state(Handle* h, Sampler* s)
     init_best_kernel<<<(h->n + 127) / 128, 128, 0, h->stream>>>(h->n, h->rms, s->dev());
     count_launch();
     MQ_CUDA(cudaGetLastError());
-    const SamplerParams p = make_params(h);
-    snapshot_kernel<<<h->n, 128, 0, h->stream>>>(p, *h, s->dev());
+    snapshot_kernel<<<h->n, 128, 0, h->stream>>>(*h, s->dev());
     count_launch();
     MQ_CUDA(cudaGetLastError());
     s->started = true;
     return check_device_errors(h);   // synchronises: solver status, invalid station correction, start values out of bounds
+}
+
+// The handle's sampler, its chains scored once before their first step (chains supplied through mq_set_models included).
+static int started_sampler(Handle* h, Sampler** out)
+{
+    int rc = sampler_get(h, out);
+    if (rc == MQ_OK && (!(*out)->started || !h->forward_done)) rc = start_sampler_state(h, *out);
+    return rc;
 }
 
 extern "C" int mq_init_chains(mq_handle* hh)
@@ -1012,9 +1005,8 @@ extern "C" int mq_init_chains(mq_handle* hh)
     Sampler* s;
     int rc = sampler_get(h, &s);
     if (rc != MQ_OK) return rc;
-    const SamplerParams p = make_params(h);
     if (s->len_start < 1 || s->len_main < 1) { set_error("mq_init_chains: empty proposal string (config line 33)"); return MQ_ERR_ARG; }
-    init_chains_kernel<<<(h->n + 63) / 64, 64, 0, h->stream>>>(p, *h, s->dev());
+    init_chains_kernel<<<(h->n + 63) / 64, 64, 0, h->stream>>>(*h, s->dev());
     count_launch();
     MQ_CUDA(cudaGetLastError());
     h->models_set = true;
@@ -1050,26 +1042,30 @@ static bool desync_wanted(const Handle* h, int n_iters, const char* override_str
     return enabled && n_iters >= 4 && h->cfg.eikonal == 1 && h->cfg.aflag != 1;
 }
 
-static int finish_pass(Handle* h, Sampler* s, const SamplerParams& p, const EvalView& pv, const SamplerDev& d, int32_t stat[2])
+// The evaluate-and-decide part of every pass, behind the kernel that set up the proposal view `pv`: the table rebuilds
+// that kernel queued (at most `items`; 0: it queued none), the misfit of every chain the view selects, the accept test and
+// the records.
+static int evaluate_and_decide(Handle* h, const EvalView& pv, const SamplerDev& d, int items)
 {
     cudaStream_t st = h->stream;
-    const int grid = (h->n + 63) / 64;
-    MQ_CUDA(launch_misfit(h, pv));
-    MQ_CUDA(launch_totals(h, pv));
-    SamplerDev free_running = d;
-    free_running.u_inject = nullptr;
-    accept_kernel<<<grid, 64, 0, st>>>(p, *h, free_running, pv);
+    if (h->cfg.aflag != 1) {
+        if (h->cfg.eikonal == 1 && items > 0) {
+            MQ_CUDA(launch_rasterise(h, pv, items));
+            MQ_CUDA(launch_tables(h, items));
+        }
+        MQ_CUDA(launch_misfit(h, pv));
+        MQ_CUDA(launch_totals(h, pv));
+    }
+    accept_kernel<<<(h->n + 63) / 64, 64, 0, st>>>(*h, d, pv);
     count_launch();
     MQ_CUDA(cudaGetLastError());
-    snapshot_kernel<<<h->n, 128, 0, st>>>(p, *h, s->dev());
+    snapshot_kernel<<<h->n, 128, 0, st>>>(*h, d);
     count_launch();
     MQ_CUDA(cudaGetLastError());
-    MQ_CUDA(cudaMemcpyAsync(stat, s->stat_buf, 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    MQ_CUDA(cudaStreamSynchronize(st));
     return MQ_OK;
 }
 
-static int step_desync(Handle* h, Sampler* s, const SamplerParams& p, int n_iters, int use_override)
+static int step_desync(Handle* h, Sampler* s, int n_iters, int use_override)
 {
     cudaStream_t st = h->stream;
     const int grid = (h->n + 63) / 64;
@@ -1091,18 +1087,16 @@ static int step_desync(Handle* h, Sampler* s, const SamplerParams& p, int n_iter
         MQ_CUDA(cudaMemsetAsync(s->stat_buf, 0, 2 * sizeof(int32_t), st));
         if (flush) {
             MQ_CUDA(cudaMemsetAsync(h->n_items, 0, sizeof(int32_t), st));
-            flush_parked_kernel<<<grid, 64, 0, st>>>(p, *h, d, pv);
-            count_launch();
-            MQ_CUDA(cudaGetLastError());
-            MQ_CUDA(launch_rasterise(h, pv, 2 * parked));
-            MQ_CUDA(launch_tables(h, 2 * parked));
+            flush_parked_kernel<<<grid, 64, 0, st>>>(*h, d, pv);
         } else {
-            propose_kernel<<<grid, 64, 0, st>>>(p, *h, d, pv, use_override);
-            count_launch();
-            MQ_CUDA(cudaGetLastError());
+            propose_kernel<<<grid, 64, 0, st>>>(*h, d, pv, use_override);   // parks the chains that need tables
         }
-        const int rc = finish_pass(h, s, p, pv, d, stat);
+        count_launch();
+        MQ_CUDA(cudaGetLastError());
+        const int rc = evaluate_and_decide(h, pv, d, flush ? 2 * parked : 0);
         if (rc != MQ_OK) return rc;
+        MQ_CUDA(cudaMemcpyAsync(stat, s->stat_buf, 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+        MQ_CUDA(cudaStreamSynchronize(st));
     }
     return check_device_errors(h);
 }
@@ -1113,15 +1107,11 @@ extern "C" int mq_step(mq_handle* hh, int n_iters, const char* proposal_override
     Handle* h = &hh->h;
     if (!h->models_set) { set_error("mq_step: no models (mq_init_chains or mq_set_models first)"); return MQ_ERR_STATE; }
     MQ_CUDA(cudaSetDevice(h->device));
+    int rc = flags_poll(h, false);     // an error raised by the kernels of an earlier, asynchronous call
+    if (rc != MQ_OK) return rc;
     Sampler* s;
-    int rc = sampler_get(h, &s);
+    rc = started_sampler(h, &s);
     if (rc != MQ_OK) return rc;
-    rc = flags_poll(h, false);     // an error raised by the kernels of an earlier, asynchronous call
-    if (rc != MQ_OK) return rc;
-    if (!s->started || !h->forward_done) {   // chains supplied through mq_set_models
-        rc = start_sampler_state(h, s);
-        if (rc != MQ_OK) return rc;
-    }
     int use_override = 0;
     if (proposal_override && *proposal_override) {
         for (const char* q = proposal_override; *q; q++)
@@ -1133,31 +1123,15 @@ extern "C" int mq_step(mq_handle* hh, int n_iters, const char* proposal_override
         }
         use_override = 1;
     }
-    const SamplerParams p = make_params(h);
+    if (desync_wanted(h, n_iters, use_override ? proposal_override : nullptr)) return step_desync(h, s, n_iters, use_override);
     cudaStream_t st = h->stream;
-    const int grid = (h->n + 63) / 64;
-    if (desync_wanted(h, n_iters, use_override ? proposal_override : nullptr)) return step_desync(h, s, p, n_iters, use_override);
     for (int it = 0; it < n_iters; it++) {
         MQ_CUDA(cudaMemsetAsync(h->n_items, 0, sizeof(int32_t), st));
-        propose_kernel<<<grid, 64, 0, st>>>(p, *h, s->dev(), h->prop_view, use_override);
+        propose_kernel<<<(h->n + 63) / 64, 64, 0, st>>>(*h, s->dev(), h->prop_view, use_override);
         count_launch();
         MQ_CUDA(cudaGetLastError());
-        if (h->cfg.aflag != 1) {
-            if (h->cfg.eikonal == 1) {
-                MQ_CUDA(launch_rasterise(h, h->prop_view, 2 * h->n));
-                MQ_CUDA(launch_tables(h, 2 * h->n));
-            }
-            MQ_CUDA(launch_misfit(h, h->prop_view));
-            MQ_CUDA(launch_totals(h, h->prop_view));
-        }
-        SamplerDev free_running = s->dev();
-        free_running.u_inject = nullptr;     // the accept test draws from the chain's own stream
-        accept_kernel<<<grid, 64, 0, st>>>(p, *h, free_running, h->prop_view);
-        count_launch();
-        MQ_CUDA(cudaGetLastError());
-        snapshot_kernel<<<h->n, 128, 0, st>>>(p, *h, s->dev());
-        count_launch();
-        MQ_CUDA(cudaGetLastError());
+        rc = evaluate_and_decide(h, h->prop_view, s->dev(), 2 * h->n);
+        if (rc != MQ_OK) return rc;
     }
     return n_iters > 0 ? flags_enqueue(h) : MQ_OK;   // stays asynchronous: reported by the next synchronising call
 }
@@ -1174,15 +1148,10 @@ extern "C" int mq_replay_step(mq_handle* hh, const mq_replay* r)
     if (!h->models_set) { set_error("mq_replay_step: no models (mq_set_models or mq_init_chains first)"); return MQ_ERR_STATE; }
     MQ_CUDA(cudaSetDevice(h->device));
     Sampler* s;
-    int rc = sampler_get(h, &s);
+    int rc = started_sampler(h, &s);
     if (rc != MQ_OK) return rc;
-    if (!s->started || !h->forward_done) {
-        rc = start_sampler_state(h, s);
-        if (rc != MQ_OK) return rc;
-    }
     const size_t n = h->n, md = h->md, ne = h->ne, ns = h->ns;
     cudaStream_t st = h->stream;
-    if (!s->u_inject) MQ_CUDA(dz(&s->u_inject, n));
     if (!h->prop_view.pres_over) { MQ_CUDA(dz(&h->prop_view.pres_over, n * ns)); MQ_CUDA(dz(&h->prop_view.sres_over, n * ns)); }
     // stage the injected proposal
     std::vector<int32_t> kind(n), dim(n), qidx(n, 0);
@@ -1204,7 +1173,7 @@ extern "C" int mq_replay_step(mq_handle* hh, const mq_replay* r)
     }
     MQ_CUDA(cudaMemcpyAsync(s->kind, kind.data(), n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
     MQ_CUDA(cudaMemcpyAsync(s->r_qidx, qidx.data(), n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    MQ_CUDA(cudaMemcpyAsync(s->rebuilt, dim.data(), n * sizeof(int32_t), cudaMemcpyHostToDevice, st));   // staging for dim_in
+    MQ_CUDA(cudaMemcpyAsync(s->r_dim, dim.data(), n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
     MQ_CUDA(cudaMemcpyAsync(s->wz, wz.data(), n * md * sizeof(float), cudaMemcpyHostToDevice, st));
     MQ_CUDA(cudaMemcpyAsync(s->wvp, wvp.data(), n * md * sizeof(float), cudaMemcpyHostToDevice, st));
     MQ_CUDA(cudaMemcpyAsync(s->wvs, wvs.data(), n * md * sizeof(float), cudaMemcpyHostToDevice, st));
@@ -1213,30 +1182,16 @@ extern "C" int mq_replay_step(mq_handle* hh, const mq_replay* r)
     MQ_CUDA(cudaMemcpyAsync(h->prop_view.sres_over, m->sres, n * ns * sizeof(float), cudaMemcpyHostToDevice, st));
     MQ_CUDA(cudaMemcpyAsync(s->noise_new, m->noise, n * 8 * sizeof(float), cudaMemcpyHostToDevice, st));
     MQ_CUDA(cudaMemcpyAsync(s->log_fac, r->log_fac, n * sizeof(double), cudaMemcpyHostToDevice, st));
-    MQ_CUDA(cudaMemcpyAsync(s->u_inject, r->u, n * sizeof(float), cudaMemcpyHostToDevice, st));
+    MQ_CUDA(cudaMemcpyAsync(s->u_buf, r->u, n * sizeof(float), cudaMemcpyHostToDevice, st));
     MQ_CUDA(cudaStreamSynchronize(st));   // the staging vectors go out of scope below
 
-    const SamplerParams p = make_params(h);
-    const int grid = (h->n + 63) / 64;
     MQ_CUDA(cudaMemsetAsync(h->n_items, 0, sizeof(int32_t), st));
-    // dim_in lives in s->rebuilt until the setup kernel overwrites it per chain (read before written by the same thread)
-    replay_setup_kernel<<<grid, 64, 0, st>>>(p, *h, s->dev(), h->prop_view, s->rebuilt);
+    const SamplerDev d = s->dev_replay();
+    replay_setup_kernel<<<(h->n + 63) / 64, 64, 0, st>>>(*h, d, h->prop_view);
     count_launch();
     MQ_CUDA(cudaGetLastError());
-    if (h->cfg.aflag != 1) {
-        if (h->cfg.eikonal == 1) {
-            MQ_CUDA(launch_rasterise(h, h->prop_view, 2 * h->n));
-            MQ_CUDA(launch_tables(h, 2 * h->n));
-        }
-        MQ_CUDA(launch_misfit(h, h->prop_view));
-        MQ_CUDA(launch_totals(h, h->prop_view));
-    }
-    accept_kernel<<<grid, 64, 0, st>>>(p, *h, s->dev(), h->prop_view);
-    count_launch();
-    MQ_CUDA(cudaGetLastError());
-    snapshot_kernel<<<h->n, 128, 0, st>>>(p, *h, s->dev());
-    count_launch();
-    MQ_CUDA(cudaGetLastError());
+    rc = evaluate_and_decide(h, h->prop_view, d, 2 * h->n);
+    if (rc != MQ_OK) return rc;
     if (r->accepted) MQ_CUDA(cudaMemcpyAsync(r->accepted, s->r_accept, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     if (r->alpha) MQ_CUDA(cudaMemcpyAsync(r->alpha, s->r_alpha, n * sizeof(float), cudaMemcpyDeviceToHost, st));
     if (r->new_ll) MQ_CUDA(cudaMemcpyAsync(r->new_ll, s->r_newll, n * sizeof(double), cudaMemcpyDeviceToHost, st));
@@ -1406,10 +1361,7 @@ extern "C" int mq_drain(mq_handle* hh, mq_record_fn fn, void* user, int* n_lost)
 }
 
 // Copies of whole SoA arrays, then one callback per chain: 13 transfers whatever the number of chains.
-static int deliver_soa(Handle* h, int first, int count, int kind, char code, const int32_t* d_dim, const int32_t* d_code,
-                       const int64_t* d_number, const double* d_rms, const float* d_z, const float* d_vp, const float* d_vpvs,
-                       const float* d_eq, const float* d_origin, const float* d_pres, const float* d_sres, const float* d_noise,
-                       mq_record_fn fn, void* user)
+static int deliver_soa(Handle* h, int first, int count, int kind, char code, const Snapshot& d, mq_record_fn fn, void* user)
 {
     const size_t md = h->md, ne = h->ne, ns = h->ns, k = (size_t)count, c0 = (size_t)first;
     std::vector<int32_t> dim(k), cd(k);
@@ -1418,10 +1370,10 @@ static int deliver_soa(Handle* h, int first, int count, int kind, char code, con
     std::vector<float> z(k * md), vp(k * md), vpvs(k * md), eq(k * ne * 3), origin(k * ne), pres(k * ns), sres(k * ns), noise(k * 8);
     cudaStream_t st = h->stream;
 #define D2H(dst, src, off, cnt) MQ_CUDA(cudaMemcpyAsync((dst).data(), (src) + (off), (cnt) * sizeof((dst)[0]), cudaMemcpyDeviceToHost, st))
-    D2H(dim, d_dim, c0, k); D2H(cd, d_code, c0, k); D2H(number, d_number, c0, k); D2H(rms, d_rms, c0, k);
-    D2H(z, d_z, c0 * md, k * md); D2H(vp, d_vp, c0 * md, k * md); D2H(vpvs, d_vpvs, c0 * md, k * md);
-    D2H(eq, d_eq, c0 * ne * 3, k * ne * 3); D2H(origin, d_origin, c0 * ne, k * ne);
-    D2H(pres, d_pres, c0 * ns, k * ns); D2H(sres, d_sres, c0 * ns, k * ns); D2H(noise, d_noise, c0 * 8, k * 8);
+    D2H(dim, d.dim, c0, k); D2H(cd, d.code, c0, k); D2H(number, d.number, c0, k); D2H(rms, d.rms, c0, k);
+    D2H(z, d.z, c0 * md, k * md); D2H(vp, d.vp, c0 * md, k * md); D2H(vpvs, d.vpvs, c0 * md, k * md);
+    D2H(eq, d.eq, c0 * ne * 3, k * ne * 3); D2H(origin, d.origin, c0 * ne, k * ne);
+    D2H(pres, d.pres, c0 * ns, k * ns); D2H(sres, d.sres, c0 * ns, k * ns); D2H(noise, d.noise, c0 * 8, k * 8);
 #undef D2H
     MQ_CUDA(cudaStreamSynchronize(st));
     for (size_t i = 0; i < k; i++) {
@@ -1436,10 +1388,10 @@ static int deliver_soa(Handle* h, int first, int count, int kind, char code, con
 }
 
 // gathers the current state of every chain (current model / origin buffers) into the layout of a Snapshot
-__global__ void gather_current_kernel(SamplerParams p, Handle hd, SamplerDev s, Snapshot d)
+__global__ void gather_current_kernel(Handle hd, SamplerDev s, Snapshot d)
 {
     const int c = blockIdx.x;
-    snapshot_copy(p, hd, d, c);
+    snapshot_copy(hd, d, c);
     if (threadIdx.x == 0) {
         const int64_t acce = s.acce[c];
         d.number[c] = acce > 0 ? acce - 1 : 0;
@@ -1455,20 +1407,13 @@ static int snapshot_range(mq_handle* hh, int first, int count, int which, mq_rec
     Sampler* s;
     int rc = sampler_get(h, &s);
     if (rc != MQ_OK) return rc;
-    if (which == 1) {
-        const Snapshot& d = s->best;
-        return deliver_soa(h, first, count, MQ_REC_BEST, 'F', d.dim, d.code, d.number, d.rms, d.z, d.vp, d.vpvs, d.eq, d.origin,
-                           d.pres, d.sres, d.noise, fn, user);
-    }
+    if (which == 1) return deliver_soa(h, first, count, MQ_REC_BEST, 'F', s->best, fn, user);
     // current state: gathered on the device into a scratch snapshot, then the same bulk copies
     if (!s->cur.dim) MQ_CUDA(alloc_snapshot(&s->cur, h));
-    const SamplerParams p = make_params(h);
-    gather_current_kernel<<<h->n, 128, 0, h->stream>>>(p, *h, s->dev(), s->cur);
+    gather_current_kernel<<<h->n, 128, 0, h->stream>>>(*h, s->dev(), s->cur);
     count_launch();
     MQ_CUDA(cudaGetLastError());
-    const Snapshot& d = s->cur;
-    return deliver_soa(h, first, count, MQ_REC_CURRENT, 'S', d.dim, d.code, d.number, d.rms, d.z, d.vp, d.vpvs, d.eq, d.origin,
-                       d.pres, d.sres, d.noise, fn, user);
+    return deliver_soa(h, first, count, MQ_REC_CURRENT, 'S', s->cur, fn, user);
 }
 
 extern "C" int mq_snapshot(mq_handle* hh, int chain, int which, mq_record_fn fn, void* user)

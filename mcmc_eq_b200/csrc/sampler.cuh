@@ -48,11 +48,12 @@ struct SamplerDev {
     char *ps_start, *ps_main, *ps_over;
     int len_start, len_main, len_over;
     // replay mode (mq_replay_step): injected uniform deviates and per-chain results of the last decision
-    float* u_inject;     // [n] or nullptr
+    float* u_inject;     // [n] or nullptr (every pass but a replayed one: the accept test draws from the chain's stream)
     float* r_alpha;      // [n]
     int32_t* r_accept;   // [n]
     double* r_newll;     // [n]
     int32_t* r_qidx;     // [n] injected event index of a Q proposal
+    int32_t* r_dim;      // [n] injected number of nuclei of the proposed model
     // desynchronised stepping (mq_step): iterations a chain still owes to the current call, and what it does in the
     // current pass: 0 = evaluated and decided, 1 = idle, 2 = parked with a proposal that waits for its travel-time tables
     int32_t* todo;       // [n] or nullptr (lock-step passes)
@@ -81,8 +82,10 @@ struct Sampler : SamplerDev {
     mq_batch batch[2];
     Snapshot cur;                 // scratch of mq_snapshot(which = 0)
     int32_t *todo_buf, *hold_buf, *stat_buf;   // storage of todo / hold / pass_stat, handed to the kernels by dev_desync() only
+    float* u_buf;                              // storage of u_inject, handed to the kernels by dev_replay() only
     SamplerDev dev() const { return *this; }
     SamplerDev dev_desync() const { SamplerDev d = *this; d.todo = todo_buf; d.hold = hold_buf; d.pass_stat = stat_buf; return d; }
+    SamplerDev dev_replay() const { SamplerDev d = *this; d.u_inject = u_buf; return d; }
 };
 
 // the handle's sampler, allocated on first use
