@@ -37,7 +37,14 @@ constexpr int kInitMin = 10;         // reference INIT_MIN,    src/time_2d.c:238
 constexpr int kFineMax = 4 * kInitMin + 3;
 constexpr float kSqrt2 = 1.41421356237309504880f;
 constexpr float kRsqrt2 = 0.70710678118654752440f;
+// Frames of the head-wave reverse-propagation stack (sweep_line).  The library is always built with 12; the CPU tests
+// build host variants with a lower bound (-DEIK_MAX_REVERSE_DEPTH=B) so that every frame of the stack and its overflow
+// run on columns that nest only a few frames deep (tests/test_reverse_depth_cpu.py).
+#ifdef EIK_MAX_REVERSE_DEPTH
+constexpr int kMaxReverseDepth = EIK_MAX_REVERSE_DEPTH;
+#else
 constexpr int kMaxReverseDepth = 12;
+#endif
 
 enum Status : int {
     kOk = 0,

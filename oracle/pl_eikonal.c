@@ -190,6 +190,7 @@ static int sweep_line(grid_t *g, int axis, int line, int future, int kb, int ke)
         int l;
         if (g->st) g->st->headwaves += longhead;
         g->rev_depth++;
+        if (g->st && g->rev_depth > g->st->max_rev_depth) g->st->max_rev_depth = g->rev_depth;
         for (l = past; l != g->side_limit; l -= future) {
             if (l < 0 || l > across) break;
             if (sweep_line(g, axis, l, -future, kb, ke) == 0) break;

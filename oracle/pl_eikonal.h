@@ -37,6 +37,7 @@ typedef struct {
     long recursive_init;  /* half-spacing re-discretised initialisations */
     long nearest_init;    /* minimal (<=4 cell) initialisations */
     long box_init;        /* analytic homogeneous-box initialisations */
+    long max_rev_depth;   /* deepest nesting of head-wave reverse propagation (frames open at once) */
 } pl_stats;
 
 /* Same contract as the reference time_2d(): hs and t are [nx][ny] arrays,

@@ -19,7 +19,8 @@ ip = C.POINTER(C.c_int)
 
 class PlStats(C.Structure):
     _fields_ = [(n, C.c_long) for n in
-                ("col_sweeps", "row_sweeps", "reverse_sweeps", "headwaves", "recursive_init", "nearest_init", "box_init")]
+                ("col_sweeps", "row_sweeps", "reverse_sweeps", "headwaves", "recursive_init", "nearest_init", "box_init",
+                 "max_rev_depth")]
 
 
 class FmGrid(C.Structure):
