@@ -338,6 +338,46 @@ int mq_diag_chains(mq_handle* h, double* ref, double* sum, double* sumsq, int32_
 int mq_diag_summary(mq_handle* h, int collective, double* mean, double* sd, double* rhat, double* ess, int64_t* n_models,
                     int32_t* chains_used);
 
+/* Hypocentre uncertainty on the device: per event the mean, the 4 x 4 covariance of (x, y, z, t), quantiles and mode of
+ * x, y and z, and the error ellipsoid of (x, y, z), from the same used models as mq_posterior_* and mq_diag_* (decimated,
+ * number > burn_in; a model dropped from a full ring counts; every chain whatever its beta).  t is the model's origin time.
+ * These are this library's own statistics, not analyse_eq's EZ / EM.
+ *
+ * Per chain c and event e, v = (x, y, z, t) of each used model: ref[c][k][e] = the chain's first used value, d = (double)v -
+ * ref, sum[c][k][e] += d_k, cross[c][p][e] += d_i d_j over the pairs p = xx xy xz xt yy yz yt zz zt tt (round to nearest, no
+ * contraction), n_models[c] += 1.  Each (chain, event) is summed in record order: the accumulators are a function of the
+ * chain's records.  Histograms of x, y and z over the box the sampler keeps hypocentres in (lo = grid x0 / y0 / z0, hi =
+ * lo + (n - 1) h), bin width w = bin_km: n_bins[a] = (int)((hi - lo) / w) + 1, a value goes to bin (int)((v - lo) / w)
+ * (float arithmetic) clamped to [0, n_bins[a] - 1]; a value outside [lo, hi] is also counted in outside[e][a].
+ * Layout: hist [n_events][n_bins[0] + n_bins[1] + n_bins[2]] (int32, x bins then y then z), outside [n_events][3] (int32),
+ * ref and sum [n_chains][4][n_events], cross [n_chains][10][n_events] (double), n_models [n_chains] (int64).  Memory:
+ * 18 doubles per (chain, event) + 8 bytes per chain + 4 (sum n_bins + 3) bytes per event.
+ *
+ * Summary: N = sum_c n_c; mean = sum_c (n_c ref_c + S_c) / N; with m_c = ref_c + S_c / n_c and W_c[ij] = C_c[ij] -
+ * S_c[i] S_c[j] / n_c, cov = (sum_c W_c + sum_c n_c (m_c - mean)(m_c - mean)^T) / (N - 1) (chains with n_c = 0 add
+ * nothing).  Quantiles of x, y, z at p = 0.025 0.16 0.5 0.84 0.975: target = p N, j = the smallest bin whose cumulative
+ * count cum_j >= target, value = lo + w (j + (target - cum_{j-1}) / count_j).  Mode: the centre lo + (j + 0.5) w of the
+ * fullest bin (the lowest index on a tie).  Error ellipsoid from the 3 x 3 (x, y, z) block: cyclic Jacobi in double,
+ * axes = sqrt(eigenvalue) in descending order (1 sigma; a negative rounding residue gives 0), axis_dir[e][k] = the unit
+ * vector (x, y, z) of axis k, signed so that v_z >= 0, or v_y >= 0 when v_z == 0, or v_x >= 0 when both are 0.  For a
+ * confidence level P multiply the axes by sqrt(chi2_3(P)) (e.g. 2.796 for 95 %).  N = 0: everything NaN; N = 1: cov,
+ * axes and axis_dir NaN.
+ *
+ * mq_hypo_begin allocates and zeroes the accumulators (again = restart), before or after mq_init_chains; MQ_ERR_ARG for
+ * bin_km <= 0, more than 2^20 bins on an axis or a negative burn_in.  mq_hypo_chains copies the accumulators out.
+ * mq_hypo_summary computes the summary on the device (fixed-order reductions, no floating-point atomics: the same
+ * accumulators give the same bits): mean [n_events][4], cov [n_events][4][4], quant [n_events][3][5], mode [n_events][3],
+ * axes [n_events][3], axis_dir [n_events][3][3], *n_models = N.  Any output pointer may be NULL.  With collective != 0 and
+ * a communicator (mq_comm_init) the sums are all-reduced over the ranks in two rounds and the histograms as int32, and
+ * every rank gets the job-wide numbers; without one, collective is ignored (outside stays per handle: mq_hypo_chains).
+ * It first reports a pending error of an earlier asynchronous call.  Both return MQ_ERR_STATE before mq_hypo_begin.  The
+ * accumulators are part of a saved state (MQ_STATE_HYPO). */
+typedef struct mq_hypo_dims { int32_t n_events, n_bins[3]; float bin_km, lo[3]; } mq_hypo_dims;
+int mq_hypo_begin(mq_handle* h, float bin_km, int64_t burn_in, mq_hypo_dims* dims);
+int mq_hypo_chains(mq_handle* h, int32_t* hist, int32_t* outside, double* ref, double* sum, double* cross, int64_t* n_models);
+int mq_hypo_summary(mq_handle* h, int collective, double* mean, double* cov, double* quant, double* mode, double* axes,
+                    double* axis_dir, int64_t* n_models);
+
 /* NCCL communicator of the job (one rank per handle).  Rank 0 calls mq_comm_unique_id and hands the 128 bytes to the
  * other ranks by whatever means the host has (torch.distributed broadcast, a file, MPI); every rank then calls
  * mq_comm_init.  libnccl is bound at run time; MQ_ERR_UNSUPPORTED when it is absent. */
@@ -392,7 +432,10 @@ int mq_temper_swap(mq_handle* h, int64_t round, int32_t* n_swapped);
  * n_batches, int32 n_quantities), then ref, sum, sumsq (double), n_models (int64), batch_len and full_batches (int32) as
  * mq_diag_chains lays them out.  A state without diagnostics has no such flag or section: its layout does not depend on
  * whether the library knows them.  Loading replaces the handle's diagnostics, or frees them when the state has none; a
- * diagnostics section of another quantity count or a bad n_batches is refused with MQ_ERR_ARG. */
+ * diagnostics section of another quantity count or a bad n_batches is refused with MQ_ERR_ARG.  MQ_STATE_SEC_HYPO =
+ * the hypocentre accumulators' own parameters (int64 burn_in, float bin_km, int32 n_bins[3]), then hist and outside
+ * (int32), zero padding to 8 bytes, ref, sum, cross (double) and n_models (int64) as mq_hypo_chains lays them out; the
+ * same rules hold (flag MQ_STATE_HYPO, none: freed, a section whose bin width or bin counts do not fit: MQ_ERR_ARG). */
 #define MQ_STATE_MAGIC "MQSTATE"
 #define MQ_STATE_FORMAT 1
 #define MQ_STATE_POSTERIOR 1u    /* flags */
@@ -400,11 +443,13 @@ int mq_temper_swap(mq_handle* h, int64_t round, int32_t* n_swapped);
 #define MQ_STATE_TABLES 4u       /* table hashes present (no tables exist with eikonal == 0 or aflag == 1) */
 #define MQ_STATE_DIAG 8u         /* diagnostics accumulators present (mq_diag_begin) */
 #define MQ_STATE_RECIPROCAL 16u  /* saved from a handle with reciprocal tables (mq_set_tables); set only with MQ_STATE_TABLES */
+#define MQ_STATE_HYPO 32u        /* hypocentre accumulators present (mq_hypo_begin) */
 #define MQ_STATE_SEC_CHAINS 1u
 #define MQ_STATE_SEC_TABLES 2u
 #define MQ_STATE_SEC_POSTERIOR 3u
 #define MQ_STATE_SEC_BETA 4u
 #define MQ_STATE_SEC_DIAG 5u
+#define MQ_STATE_SEC_HYPO 6u
 typedef struct mq_state_header {
     char magic[8];             /* MQ_STATE_MAGIC */
     uint32_t format;           /* MQ_STATE_FORMAT */
@@ -413,7 +458,7 @@ typedef struct mq_state_header {
     int32_t n_chains, max_dim, n_events, n_stations, n_picks, nz, nxmod, n_rows;
     uint64_t seed;
     int64_t chain_offset;
-    uint32_t flags;            /* MQ_STATE_POSTERIOR | MQ_STATE_BETA | MQ_STATE_TABLES | MQ_STATE_DIAG | MQ_STATE_RECIPROCAL */
+    uint32_t flags;            /* MQ_STATE_POSTERIOR | MQ_STATE_BETA | MQ_STATE_TABLES | MQ_STATE_DIAG | MQ_STATE_RECIPROCAL | MQ_STATE_HYPO */
     uint32_t n_sections;
     float post_dv, post_dvpvs; /* mq_posterior_begin's arguments and the histogram sizes (0 when off) */
     int32_t post_ndv, post_ndvpvs;

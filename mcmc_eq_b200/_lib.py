@@ -86,6 +86,10 @@ class MqDiagDims(C.Structure):
                 ("n_batches", C.c_int32)]
 
 
+class MqHypoDims(C.Structure):
+    _fields_ = [("n_events", C.c_int32), ("n_bins", C.c_int32 * 3), ("bin_km", C.c_float), ("lo", C.c_float * 3)]
+
+
 class MqStateHeader(C.Structure):
     """Start of a saved sampler state (include/mcmceq_b200.h: mq_state_header)."""
     _fields_ = [("magic", C.c_char * 8), ("format", C.c_uint32), ("header_bytes", C.c_uint32), ("version", C.c_char * 48),
@@ -100,9 +104,9 @@ class MqStateSection(C.Structure):
     _fields_ = [("id", C.c_uint32), ("reserved", C.c_uint32), ("offset", C.c_uint64), ("bytes", C.c_uint64)]
 
 
-STATE_POSTERIOR, STATE_BETA, STATE_TABLES, STATE_DIAG, STATE_RECIPROCAL = 1, 2, 4, 8, 16
+STATE_POSTERIOR, STATE_BETA, STATE_TABLES, STATE_DIAG, STATE_RECIPROCAL, STATE_HYPO = 1, 2, 4, 8, 16, 32
 TABLES_PARITY, TABLES_RECIPROCAL = 0, 1     # mq_set_tables
-STATE_SEC_DIAG = 5
+STATE_SEC_DIAG, STATE_SEC_HYPO = 5, 6
 
 
 RECORD_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.POINTER(MqRecord))
@@ -135,6 +139,9 @@ def lib() -> C.CDLL:
         L.mq_diag_begin.argtypes = [C.c_void_p, C.c_int64, C.c_int, C.POINTER(MqDiagDims)]
         L.mq_diag_chains.argtypes = [C.c_void_p, dp, dp, dp, ip, ip, lp]
         L.mq_diag_summary.argtypes = [C.c_void_p, C.c_int, dp, dp, dp, dp, lp, ip]
+        L.mq_hypo_begin.argtypes = [C.c_void_p, C.c_float, C.c_int64, C.POINTER(MqHypoDims)]
+        L.mq_hypo_chains.argtypes = [C.c_void_p, ip, ip, dp, dp, dp, lp]
+        L.mq_hypo_summary.argtypes = [C.c_void_p, C.c_int, dp, dp, dp, dp, dp, dp, lp]
         L.mq_comm_unique_id.argtypes = [u8p]
         L.mq_comm_init.argtypes = [C.c_void_p, u8p, C.c_int, C.c_int]
         L.mq_comm_destroy.argtypes = [C.c_void_p]
@@ -441,6 +448,36 @@ class Sampler:
         out["names"] = quantity_names(self.nz, self.picks.n_events, self.picks.n_stations)
         return out
 
+    # ---- hypocentre uncertainty (mq_hypo_*, mcmc_eq_b200/hypo.py) -------------------------------------------------
+    def hypo_begin(self, bin_km: float, burn_in: int = 0) -> MqHypoDims:
+        """Per-event covariance, quantiles, mode and error ellipsoid of the hypocentres of the decimated models with
+        number > burn_in; histograms of x, y and z with bins of bin_km."""
+        d = MqHypoDims()
+        check(lib().mq_hypo_begin(self.h, bin_km, burn_in, C.byref(d)))
+        self._hbins = tuple(d.n_bins)
+        return d
+
+    def hypo_chains(self) -> dict:
+        """Raw accumulators: hist [ne, Bx + By + Bz], outside [ne, 3], ref / sum [n, 4, ne], cross [n, 10, ne], n_models [n]."""
+        ne = self.picks.n_events
+        out = dict(hist=np.zeros((ne, sum(self._hbins)), np.int32), outside=np.zeros((ne, 3), np.int32),
+                   ref=np.zeros((self.n, 4, ne)), sum=np.zeros((self.n, 4, ne)), cross=np.zeros((self.n, 10, ne)),
+                   n_models=np.zeros(self.n, np.int64))
+        check(lib().mq_hypo_chains(self.h, _p(out["hist"], ip), _p(out["outside"], ip), _p(out["ref"], dp), _p(out["sum"], dp),
+                                   _p(out["cross"], dp), _p(out["n_models"], lp)))
+        return out
+
+    def hypo_summary(self, collective: bool = False) -> dict:
+        """mean [ne, 4], cov [ne, 4, 4], quant [ne, 3, 5], mode [ne, 3], axes [ne, 3], axis_dir [ne, 3, 3], n_models (N)."""
+        ne = self.picks.n_events
+        out = dict(mean=np.zeros((ne, 4)), cov=np.zeros((ne, 4, 4)), quant=np.zeros((ne, 3, 5)), mode=np.zeros((ne, 3)),
+                   axes=np.zeros((ne, 3)), axis_dir=np.zeros((ne, 3, 3)))
+        n = C.c_int64(0)
+        check(lib().mq_hypo_summary(self.h, int(collective), *[_p(out[k], dp) for k in ("mean", "cov", "quant", "mode", "axes", "axis_dir")],
+                                    C.byref(n)))
+        out["n_models"] = n.value
+        return out
+
     def comm_init(self, unique_id: bytes, rank: int, world: int):
         buf = (C.c_uint8 * 128).from_buffer_copy(unique_id)
         check(lib().mq_comm_init(self.h, buf, rank, world))
@@ -486,6 +523,11 @@ class Sampler:
                 if sec.id == STATE_SEC_DIAG:
                     K, Q = np.frombuffer(blob, np.int32, 2, sec.offset + 8)
                     self._ddims = (int(Q), int(K))
+        if head.flags & STATE_HYPO:   # the section starts with int64 burn_in, float bin_km, int32 n_bins[3]
+            for k in range(head.n_sections):
+                sec = MqStateSection.from_buffer_copy(blob, C.sizeof(MqStateHeader) + k * C.sizeof(MqStateSection))
+                if sec.id == STATE_SEC_HYPO:
+                    self._hbins = tuple(int(b) for b in np.frombuffer(blob, np.int32, 3, sec.offset + 12))
 
     def sync(self):
         check(lib().mq_sync(self.h))

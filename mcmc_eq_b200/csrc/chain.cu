@@ -804,6 +804,44 @@ __device__ void diag_accumulate(const Handle& hd, const Ring& R, int c)
     }
 }
 
+// Hypocentre uncertainty for one used model (DESIGN.md section 4e): per event, v = (x, y, z, t) goes into the chain's
+// sums of d = v - ref and of the ten products d_i d_j, and x, y, z into the event's histograms.  Threads over events; each
+// (chain, event) is summed in record order whatever the stepping, and integer atomics give the same counts in any order.
+__device__ void hypo_accumulate(const Handle& hd, int c)
+{
+    const Hypo& H = hd.hypo;
+    const CurModel cm = cur_model(hd, c);
+    const int ne = hd.ne, nbt = H.nb[0] + H.nb[1] + H.nb[2];
+    const int64_t m = H.n_models[c];
+    const float lo[3] = {hd.xmin, hd.ymin, hd.zmin}, hi[3] = {hd.xmax, hd.ymax, hd.zmax};
+    double* ref = H.ref + (size_t)c * 4 * ne;
+    double* S = H.sum + (size_t)c * 4 * ne;
+    double* C = H.cross + (size_t)c * 10 * ne;
+    for (int e = threadIdx.x; e < ne; e += blockDim.x) {
+        const float* q = hd.eq + ((size_t)c * ne + e) * 3;
+        const float v[4] = {q[0], q[1], q[2], cm.origin[e]};
+        double d[4];
+        for (int k = 0; k < 4; k++) {
+            if (m == 0) ref[(size_t)k * ne + e] = (double)v[k];
+            d[k] = __dsub_rn((double)v[k], ref[(size_t)k * ne + e]);
+            S[(size_t)k * ne + e] = __dadd_rn(S[(size_t)k * ne + e], d[k]);
+        }
+        int p = 0;
+        for (int i = 0; i < 4; i++)
+            for (int j = i; j < 4; j++, p++) C[(size_t)p * ne + e] = __dadd_rn(C[(size_t)p * ne + e], __dmul_rn(d[i], d[j]));
+        int32_t* row = H.hist + (size_t)e * nbt;
+        for (int a = 0; a < 3; a++) {
+            int j = (int)__fdiv_rn(__fsub_rn(v[a], lo[a]), H.bin);
+            j = min(max(j, 0), H.nb[a] - 1);
+            if (!(v[a] >= lo[a] && v[a] <= hi[a])) atomicAdd(&H.outside[3 * e + a], 1);
+            atomicAdd(&row[j], 1);
+            row += H.nb[a];
+        }
+    }
+    __syncthreads();   // every thread has read m
+    if (threadIdx.x == 0) H.n_models[c] = m + 1;
+}
+
 __global__ void snapshot_kernel(Handle hd, SamplerDev s)
 {
     const int c = blockIdx.x;
@@ -811,6 +849,7 @@ __global__ void snapshot_kernel(Handle hd, SamplerDev s)
     if (pend) {
         if (hd.post.on && (long long)s.ring.number[c] > hd.post.burn_in) posterior_accumulate(hd, c);
         if (hd.diag.on && (long long)s.ring.number[c] > hd.diag.burn_in) diag_accumulate(hd, s.ring, c);
+        if (hd.hypo.on && (long long)s.ring.number[c] > hd.hypo.burn_in) hypo_accumulate(hd, c);
         if (pend == 1) {
             const int wr = s.ring.wr[c];
             record_write(hd, s.ring, c, s.ring.data + ((size_t)c * s.ring.slots + wr % s.ring.slots) * s.ring.rec_floats);

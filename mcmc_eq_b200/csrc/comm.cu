@@ -317,6 +317,14 @@ int comm_allreduce_sum(Handle* h, double* buf, size_t count)
     return MQ_OK;
 }
 
+int comm_allreduce_sum(Handle* h, int32_t* buf, size_t count)
+{
+    Comm* c = (Comm*)h->comm;
+    if (!c || c->world < 2) return MQ_OK;
+    MQ_NCCL(nccl()->AllReduce(buf, buf, count, ncclInt32, ncclSum, c->comm, h->stream));
+    return MQ_OK;
+}
+
 void comm_destroy(Handle* h)
 {
     mq_handle* hh = reinterpret_cast<mq_handle*>(h);   // Handle is the first and only member of mq_handle

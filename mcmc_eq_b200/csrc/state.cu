@@ -218,10 +218,10 @@ namespace {
 struct Plan {   // sizes and places of everything in a blob of this handle
     mq_state_header head;
     int n_sections;
-    mq_state_section sec[5];
+    mq_state_section sec[6];
     size_t payload_off, payload_bytes, total_bytes;
     size_t rec_bytes;
-    size_t chains_off, hash_off, post_off, post_int_bytes, beta_off, diag_off;   // offsets inside the payload (= the staging buffer)
+    size_t chains_off, hash_off, post_off, post_int_bytes, beta_off, diag_off, hypo_off;   // offsets inside the payload (= the staging buffer)
 };
 
 // The diagnostics section: DiagHead, then ref [n][Q], sum [n][K][Q], sumsq [n][K][Q] (double), n_models [n] (int64),
@@ -237,13 +237,26 @@ inline size_t diag_section_bytes(size_t n, size_t K, size_t Q)
 
 inline size_t up8(size_t x) { return (x + 7) / 8 * 8; }
 
+// The hypocentre section: HypoHead, then hist [ne][nb0 + nb1 + nb2] and outside [ne][3] (int32), zero padding to 8 bytes,
+// ref [n][4][ne], sum [n][4][ne], cross [n][10][ne] (double), n_models [n] (int64).
+struct HypoHead {
+    int64_t burn_in;
+    float bin_km;
+    int32_t n_bins[3];
+};
+inline size_t hypo_int_bytes(size_t ne, const int nb[3]) { return up8(ne * ((size_t)nb[0] + nb[1] + nb[2] + 3) * sizeof(int32_t)); }
+inline size_t hypo_section_bytes(size_t n, size_t ne, const int nb[3])
+{
+    return sizeof(HypoHead) + hypo_int_bytes(ne, nb) + n * ne * 18 * sizeof(double) + n * sizeof(int64_t);
+}
+
 bool has_tables(const Handle* h) { return h->cfg.eikonal == 1 && h->cfg.aflag != 1; }
 
 // reciprocal tables are part of a state's identity only where tables exist
 bool reciprocal_tables(const Handle* h) { return has_tables(h) && h->tables_mode == MQ_TABLES_RECIPROCAL; }
 
 // the sections of a blob with the given options; the header's identity fields from the handle
-void make_plan(const Handle* h, bool post, bool beta, bool tables, bool diag, Plan* P)
+void make_plan(const Handle* h, bool post, bool beta, bool tables, bool diag, bool hypo, Plan* P)
 {
     memset(P, 0, sizeof *P);
     mq_state_header& H = P->head;
@@ -256,7 +269,7 @@ void make_plan(const Handle* h, bool post, bool beta, bool tables, bool diag, Pl
     H.config_sum = config_checksum(&h->cfg);
     H.picks_sum = h->picks_sum;
     H.flags = (post ? MQ_STATE_POSTERIOR : 0) | (beta ? MQ_STATE_BETA : 0) | (tables ? MQ_STATE_TABLES : 0) | (diag ? MQ_STATE_DIAG : 0) |
-              (tables && reciprocal_tables(h) ? MQ_STATE_RECIPROCAL : 0);
+              (tables && reciprocal_tables(h) ? MQ_STATE_RECIPROCAL : 0) | (hypo ? MQ_STATE_HYPO : 0);
     const size_t n = h->n;
     P->rec_bytes = chain_bytes(h->md, h->ne, h->ns);
     size_t off = 0;
@@ -276,6 +289,7 @@ void make_plan(const Handle* h, bool post, bool beta, bool tables, bool diag, Pl
     }
     if (beta) P->beta_off = add(MQ_STATE_SEC_BETA, n * sizeof(float));
     if (diag) P->diag_off = add(MQ_STATE_SEC_DIAG, diag_section_bytes(n, h->diag.K, h->diag.Q));
+    if (hypo) P->hypo_off = add(MQ_STATE_SEC_HYPO, hypo_section_bytes(n, h->ne, h->hypo.nb));
     H.n_sections = P->n_sections;
     P->payload_off = sizeof(mq_state_header) + P->n_sections * sizeof(mq_state_section);
     P->payload_bytes = off;
@@ -286,7 +300,7 @@ void make_plan(const Handle* h, bool post, bool beta, bool tables, bool diag, Pl
 
 void plan_of_handle(const Handle* h, Plan* P)
 {
-    make_plan(h, h->post.on != 0, h->beta != nullptr, has_tables(h), h->diag.on != 0, P);
+    make_plan(h, h->post.on != 0, h->beta != nullptr, has_tables(h), h->diag.on != 0, h->hypo.on != 0, P);
     mq_state_header& H = P->head;
     H.seed = h->seed;
     H.chain_offset = h->chain_offset;
@@ -395,6 +409,21 @@ extern "C" int mq_state_save(mq_handle* hh, void* buf, uint64_t cap, uint64_t* b
         MQ_CUDA(cudaMemcpyAsync(o, D.full_batches, n * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
         MQ_CUDA(cudaStreamSynchronize(st));   // dh is on this stack frame
     }
+    if (P.head.flags & MQ_STATE_HYPO) {
+        const Hypo& Y = h->hypo;
+        const HypoHead yh = {(int64_t)Y.burn_in, Y.bin, {Y.nb[0], Y.nb[1], Y.nb[2]}};
+        const size_t ne = h->ne, nh = ne * ((size_t)Y.nb[0] + Y.nb[1] + Y.nb[2]), nd = n * ne;
+        char* o = d + P.hypo_off;
+        MQ_CUDA(cudaMemcpyAsync(o, &yh, sizeof yh, cudaMemcpyHostToDevice, st)); o += sizeof yh;
+        MQ_CUDA(cudaMemcpyAsync(o, Y.hist, nh * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
+        MQ_CUDA(cudaMemcpyAsync(o + nh * sizeof(int32_t), Y.outside, ne * 3 * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
+        o += hypo_int_bytes(ne, Y.nb);
+        MQ_CUDA(cudaMemcpyAsync(o, Y.ref, 4 * nd * sizeof(double), cudaMemcpyDeviceToDevice, st)); o += 4 * nd * sizeof(double);
+        MQ_CUDA(cudaMemcpyAsync(o, Y.sum, 4 * nd * sizeof(double), cudaMemcpyDeviceToDevice, st)); o += 4 * nd * sizeof(double);
+        MQ_CUDA(cudaMemcpyAsync(o, Y.cross, 10 * nd * sizeof(double), cudaMemcpyDeviceToDevice, st)); o += 10 * nd * sizeof(double);
+        MQ_CUDA(cudaMemcpyAsync(o, Y.n_models, n * sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
+        MQ_CUDA(cudaStreamSynchronize(st));   // yh is on this stack frame
+    }
     char* out = (char*)buf;
     memcpy(out, &P.head, sizeof P.head);
     memcpy(out + sizeof P.head, P.sec, P.n_sections * sizeof(mq_state_section));
@@ -434,8 +463,8 @@ extern "C" int mq_state_load(mq_handle* hh, const void* buf, uint64_t bytes)
     if (H.config_sum != config_checksum(&h->cfg)) { set_error("mq_state_load: the state was saved with another configuration"); return MQ_ERR_ARG; }
     if (H.picks_sum != h->picks_sum) { set_error("mq_state_load: the state was saved with other picks"); return MQ_ERR_ARG; }
     const bool post = (H.flags & MQ_STATE_POSTERIOR) != 0, beta = (H.flags & MQ_STATE_BETA) != 0, tables = (H.flags & MQ_STATE_TABLES) != 0;
-    const bool diag = (H.flags & MQ_STATE_DIAG) != 0;
-    if ((H.flags & ~(uint32_t)(MQ_STATE_POSTERIOR | MQ_STATE_BETA | MQ_STATE_TABLES | MQ_STATE_DIAG | MQ_STATE_RECIPROCAL)) ||
+    const bool diag = (H.flags & MQ_STATE_DIAG) != 0, hypo = (H.flags & MQ_STATE_HYPO) != 0;
+    if ((H.flags & ~(uint32_t)(MQ_STATE_POSTERIOR | MQ_STATE_BETA | MQ_STATE_TABLES | MQ_STATE_DIAG | MQ_STATE_RECIPROCAL | MQ_STATE_HYPO)) ||
         tables != has_tables(h)) {
         set_error("mq_state_load: flags 0x%x do not fit the handle", H.flags);
         return MQ_ERR_ARG;
@@ -452,15 +481,20 @@ extern "C" int mq_state_load(mq_handle* hh, const void* buf, uint64_t bytes)
         posterior_sizes(h, H.post_dv, H.post_dvpvs, &ndv, &ndvpvs, &n_int, &n_dbl);
         if (ndv != H.post_ndv || ndvpvs != H.post_ndvpvs) { set_error("mq_state_load: posterior histogram sizes do not fit"); return MQ_ERR_ARG; }
     }
-    // the diagnostics section starts with its own parameters: they must fit the handle
-    DiagHead dh = {0, 0, 0};
-    if (diag) {
+    // the diagnostics and hypocentre sections start with their own parameters, which must fit the handle (make_plan below
+    // checks the whole section table)
+    auto find_section = [&](uint32_t id) -> const mq_state_section* {
         const mq_state_section* sec = nullptr;
-        if (H.n_sections <= 5 && sizeof H + H.n_sections * sizeof(mq_state_section) <= bytes)
+        if (H.n_sections <= 6 && sizeof H + H.n_sections * sizeof(mq_state_section) <= bytes)
             for (uint32_t k = 0; k < H.n_sections; k++) {
                 const mq_state_section* e = (const mq_state_section*)(in + sizeof H + k * sizeof(mq_state_section));
-                if (e->id == MQ_STATE_SEC_DIAG) sec = e;
+                if (e->id == id) sec = e;
             }
+        return sec;
+    };
+    DiagHead dh = {0, 0, 0};
+    if (diag) {
+        const mq_state_section* sec = find_section(MQ_STATE_SEC_DIAG);
         if (!sec || sec->bytes < sizeof dh || sec->offset > bytes - sizeof(uint64_t) || sec->bytes > bytes - sizeof(uint64_t) - sec->offset) {
             set_error("mq_state_load: flags 0x%x without a diagnostics section", H.flags);
             return MQ_ERR_ARG;
@@ -473,13 +507,31 @@ extern "C" int mq_state_load(mq_handle* hh, const void* buf, uint64_t bytes)
             return MQ_ERR_ARG;
         }
     }
+    // the hypocentre bin counts must be what the bin width gives on this handle's box
+    HypoHead yh = {0, 0.f, {0, 0, 0}};
+    if (hypo) {
+        const mq_state_section* sec = find_section(MQ_STATE_SEC_HYPO);
+        if (!sec || sec->bytes < sizeof yh || sec->offset > bytes - sizeof(uint64_t) || sec->bytes > bytes - sizeof(uint64_t) - sec->offset) {
+            set_error("mq_state_load: flags 0x%x without a hypocentre section", H.flags);
+            return MQ_ERR_ARG;
+        }
+        memcpy(&yh, in + sec->offset, sizeof yh);
+        int nb[3] = {0, 0, 0};
+        if (yh.burn_in < 0 || !(yh.bin_km > 0.f) || hypo_bins(h, yh.bin_km, nb) != 0 || nb[0] != yh.n_bins[0] ||
+            nb[1] != yh.n_bins[1] || nb[2] != yh.n_bins[2]) {
+            set_error("mq_state_load: hypocentre accumulators of bin width %g km, %d x %d x %d bins (burn-in %lld) do not fit the handle",
+                      (double)yh.bin_km, yh.n_bins[0], yh.n_bins[1], yh.n_bins[2], (long long)yh.burn_in);
+            return MQ_ERR_ARG;
+        }
+    }
     // the layout these options give must be the blob's, section by section
     Plan P;
     {
-        Handle tmp = *h;                  // sizes of the posterior and diagnostics blocks as the state has them
+        Handle tmp = *h;                  // sizes of the posterior, diagnostics and hypocentre blocks as the state has them
         tmp.post.n_int = n_int; tmp.post.n_dbl = n_dbl;
         tmp.diag.K = dh.n_batches; tmp.diag.Q = dh.n_quantities;
-        make_plan(&tmp, post, beta, tables, diag, &P);
+        for (int a = 0; a < 3; a++) tmp.hypo.nb[a] = yh.n_bins[a];
+        make_plan(&tmp, post, beta, tables, diag, hypo, &P);
     }
     if (bytes != P.total_bytes || H.n_sections != (uint32_t)P.n_sections ||
         memcmp(in + sizeof H, P.sec, P.n_sections * sizeof(mq_state_section)) != 0) {
@@ -545,6 +597,26 @@ extern "C" int mq_state_load(mq_handle* hh, const void* buf, uint64_t bytes)
         MQ_CUDA(cudaMemcpyAsync(D.full_batches, o, n * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
     } else if (h->diag.on) {
         diag_destroy(h);
+    }
+    if (hypo) {
+        Hypo& Y = h->hypo;
+        if (!Y.on || Y.bin != yh.bin_km) {
+            MQ_CUDA(cudaStreamSynchronize(st));
+            rc = hypo_alloc(h, yh.bin_km, yh.burn_in);
+            if (rc != MQ_OK) return rc;
+        }
+        Y.burn_in = yh.burn_in;
+        const size_t ne = h->ne, nh = ne * ((size_t)Y.nb[0] + Y.nb[1] + Y.nb[2]), nd = n * ne;
+        const char* o = d + P.hypo_off + sizeof yh;
+        MQ_CUDA(cudaMemcpyAsync(Y.hist, o, nh * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
+        MQ_CUDA(cudaMemcpyAsync(Y.outside, o + nh * sizeof(int32_t), ne * 3 * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
+        o += hypo_int_bytes(ne, Y.nb);
+        MQ_CUDA(cudaMemcpyAsync(Y.ref, o, 4 * nd * sizeof(double), cudaMemcpyDeviceToDevice, st)); o += 4 * nd * sizeof(double);
+        MQ_CUDA(cudaMemcpyAsync(Y.sum, o, 4 * nd * sizeof(double), cudaMemcpyDeviceToDevice, st)); o += 4 * nd * sizeof(double);
+        MQ_CUDA(cudaMemcpyAsync(Y.cross, o, 10 * nd * sizeof(double), cudaMemcpyDeviceToDevice, st)); o += 10 * nd * sizeof(double);
+        MQ_CUDA(cudaMemcpyAsync(Y.n_models, o, n * sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
+    } else if (h->hypo.on) {
+        hypo_destroy(h);
     }
     h->seed = H.seed;
     h->chain_offset = H.chain_offset;

@@ -86,6 +86,24 @@ struct Diag {
     size_t scratch_bytes;
 };
 
+// On-device hypocentre uncertainty (hypo.cu, DESIGN.md section 4e): per chain and event, sums of d = v - ref and of the
+// ten products d_i d_j of v = (x, y, z, t) over the same decimated models the posterior takes, and per event histograms
+// of x, y and z over the hypocentre box.  Memory: 18 doubles per (chain, event).
+struct Hypo {
+    int on;
+    float bin;              // bin width (km)
+    int nb[3];              // bins of x, y, z
+    long long burn_in;      // models with number <= burn_in are skipped, as in the posterior
+    int32_t* hist;          // [ne][nb[0] + nb[1] + nb[2]]
+    int32_t* outside;       // [ne][3] values outside the box (clamped into the end bins)
+    double* ref;            // [n][4][ne] the chain's first used value
+    double* sum;            // [n][4][ne] sums of d
+    double* cross;          // [n][10][ne] sums of d_i d_j (xx xy xz xt yy yz yt zz zt tt)
+    int64_t* n_models;      // [n] used models so far
+    void* scratch;          // summary work space (hypo.cu), allocated on the first mq_hypo_summary
+    size_t scratch_bytes;
+};
+
 struct Handle {
     mq_config cfg;
     int device;
@@ -153,6 +171,7 @@ struct Handle {
     void* comm;
     Posterior post;
     Diag diag;
+    Hypo hypo;
 };
 
 // checksums a saved sampler state carries (state.cu)
@@ -163,8 +182,14 @@ uint64_t picks_checksum(const mq_picks* pk);
 inline int diag_quantities(int nz, int ne, int ns) { return 10 + 2 * nz + 4 * ne + 2 * ns; }
 int diag_alloc(Handle* h, int K, long long burn_in);
 void diag_destroy(Handle* h);
-// comm.cu: in-place sum of `count` doubles over the ranks of the handle's communicator; nothing without one
+// hypocentre accumulators (hypo.cu): bins per axis for a bin width (-1: more than 2^20 on some axis); allocate (zeroed) /
+// free them
+int hypo_bins(const Handle* h, float bin_km, int nb[3]);
+int hypo_alloc(Handle* h, float bin_km, long long burn_in);
+void hypo_destroy(Handle* h);
+// comm.cu: in-place sum of `count` doubles (int32s) over the ranks of the handle's communicator; nothing without one
 int comm_allreduce_sum(Handle* h, double* buf, size_t count);
+int comm_allreduce_sum(Handle* h, int32_t* buf, size_t count);
 
 }  // namespace mq
 

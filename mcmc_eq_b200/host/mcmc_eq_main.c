@@ -1,7 +1,7 @@
 /* mcmc_eq_main.c -- the reference's command line on top of the B200 library (plain C host code, C ABI only).
  *
  *     mcmc_eq <config_eqx.dat> <out> <picks> [-n chains] [-d device] [-s seed] [-r slots] [-q]
- *             [-k checkpoint [-K minutes]] [-R checkpoint] [-D diagnostics] [-x]
+ *             [-k checkpoint [-K minutes]] [-R checkpoint] [-D diagnostics] [-L locations] [-x]
  *
  * The first three arguments are the reference's (src/mcmc_eq.c:332-338; it ignores anything after them).
  * With one chain (the default) <out> is written exactly like the reference writes it: a "sta ST" record, a
@@ -38,6 +38,15 @@
  * one line per quantity "name index n_models mean sd rhat ess" (names rms dim noise vp vpvs x y z t pres sres), plus one
  * stderr line with the largest R-hat and the smallest ESS and where they occur.  The accumulators are part of the
  * checkpoint: under -R they continue, and -D with a checkpoint that has none fails before any chain file is touched.
+ *
+ * Hypocentre uncertainty: -L <file> accumulates every event's hypocentre and origin time on the device (mq_hypo_*) from
+ * the decimated models after the start phase (burn-in = j_max_start, histogram bins of grid h / 10), and writes <file>
+ * like -D's, at every checkpoint and at the end of the run: a "#" header line (events, models N, burn-in, bin width,
+ * iterations done), then one line per event "index N mean_x mean_y mean_z mean_t sd_x sd_y sd_z sd_t corr_zt", the
+ * quantiles 0.025 0.16 0.5 0.84 0.975 of x, of y and of z, "mode_x mode_y mode_z", three times "semi_axis azimuth
+ * plunge" (1-sigma error ellipsoid, longest axis first; azimuth in degrees clockwise from +y in [0, 360), plunge in
+ * degrees towards +z, down, in [0, 90]) and "outside_x outside_y outside_z" (models outside the hypocentre box on that
+ * axis).  Under -R the accumulators continue; -L with a checkpoint that has none fails before any chain file is touched.
  *
  * Reciprocal tables: -x builds the travel-time tables with the source at each receiver row instead of at each event depth
  * (mq_set_tables, MQ_TABLES_RECIPROCAL): n_rows solves per table instead of nz, at the price of the finite-difference
@@ -367,6 +376,79 @@ out:
     return ok ? 0 : 1;
 }
 
+/* ---- hypocentre uncertainty: the parameters a saved state holds, the report file ---------------------------------------- */
+static int state_hypo_params(const unsigned char* state, uint64_t bytes, int64_t* burn_in, float* bin_km)
+{
+    const mq_state_header* H = (const mq_state_header*)state;
+    uint32_t k;
+    if (!(H->flags & MQ_STATE_HYPO) || bytes < sizeof *H + H->n_sections * sizeof(mq_state_section)) return 1;
+    for (k = 0; k < H->n_sections; k++) {
+        mq_state_section sec;
+        memcpy(&sec, state + sizeof *H + k * sizeof sec, sizeof sec);
+        if (sec.id == MQ_STATE_SEC_HYPO && sec.bytes >= 24 && sec.offset + 24 <= bytes) {
+            memcpy(burn_in, state + sec.offset, sizeof *burn_in);
+            memcpy(bin_km, state + sec.offset + 8, sizeof *bin_km);
+            return 0;
+        }
+    }
+    return 1;
+}
+
+/* azimuth (degrees clockwise from +y, [0, 360)) and plunge (degrees towards +z) of a unit vector with v[2] >= 0 */
+static void azimuth_plunge(const double* v, double* az, double* pl)
+{
+    const double deg = 57.295779513082320876798;
+    double a = atan2(v[0], v[1]) * deg;
+    if (a < 0.0) a += 360.0;
+    if (a >= 360.0) a -= 360.0;
+    *az = a;
+    *pl = atan2(v[2], hypot(v[0], v[1])) * deg;
+}
+
+static int hypo_write(const char* path, mq_handle* h, int ne, int64_t burn_in, float bin_km, long iters_done)
+{
+    double* v = (double*)malloc(50 * (size_t)ne * sizeof(double));
+    int32_t* outside = (int32_t*)malloc(3 * (size_t)ne * sizeof(int32_t));
+    double *mean = v, *cov = v + 4 * ne, *quant = cov + 16 * ne, *mode = quant + 15 * ne, *axes = mode + 3 * ne, *dir = axes + 3 * ne;
+    int64_t n_models = 0;
+    int e, k, ok = 0;
+    char tmp[4200];
+    FILE* f = NULL;
+    if (!v || !outside) goto out;
+    if (mq_hypo_summary(h, 0, mean, cov, quant, mode, axes, dir, &n_models) != MQ_OK ||
+        mq_hypo_chains(h, NULL, outside, NULL, NULL, NULL, NULL) != MQ_OK) {
+        fprintf(stderr, "locations: mq_hypo_summary failed: %s\n", mq_last_error()); goto out;
+    }
+    snprintf(tmp, sizeof tmp, "%s.tmp", path);
+    if (!(f = fopen(tmp, "w"))) { fprintf(stderr, "locations: cannot write %s\n", tmp); goto out; }
+    fprintf(f, "# events %d n_models %lld burn_in %lld bin_km %.9g iterations %ld\n", ne, (long long)n_models, (long long)burn_in,
+            (double)bin_km, iters_done);
+    for (e = 0; e < ne; e++) {
+        const double* m = mean + 4 * e;
+        const double* c = cov + 16 * e;
+        fprintf(f, "%d %lld %.9g %.9g %.9g %.9g", e, (long long)n_models, m[0], m[1], m[2], m[3]);
+        for (k = 0; k < 4; k++) fprintf(f, " %.9g", sqrt(c[5 * k]));
+        fprintf(f, " %.9g", c[11] / sqrt(c[10] * c[15]));
+        for (k = 0; k < 15; k++) fprintf(f, " %.9g", quant[15 * e + k]);
+        for (k = 0; k < 3; k++) fprintf(f, " %.9g", mode[3 * e + k]);
+        for (k = 0; k < 3; k++) {
+            double az, pl;
+            azimuth_plunge(dir + 9 * e + 3 * k, &az, &pl);
+            fprintf(f, " %.9g %.6f %.6f", axes[3 * e + k], az, pl);
+        }
+        fprintf(f, " %d %d %d\n", outside[3 * e], outside[3 * e + 1], outside[3 * e + 2]);
+    }
+    if (fclose(f) != 0) { f = NULL; fprintf(stderr, "locations: cannot write %s\n", tmp); goto out; }
+    f = NULL;
+    if (rename(tmp, path) != 0) { fprintf(stderr, "locations: cannot rename %s to %s\n", tmp, path); goto out; }
+    ok = 1;
+out:
+    if (f) fclose(f);
+    free(v);
+    free(outside);
+    return ok ? 0 : 1;
+}
+
 static double now_s(void)
 {
     struct timespec t;
@@ -380,9 +462,10 @@ static double now_s(void)
 int main(int argc, char** argv)
 {
     int rc = 0, n_chains = 1, device = 0, quiet = 0, i, c, from_file = 0, ring = 0, writer_on = 0, n_given = 0, reciprocal = 0;
-    const char *ck_path = NULL, *resume_path = NULL, *diag_path = NULL;
-    int64_t diag_burn_in = 0;
+    const char *ck_path = NULL, *resume_path = NULL, *diag_path = NULL, *hypo_path = NULL;
+    int64_t diag_burn_in = 0, hypo_burn_in = 0;
     int32_t diag_batches = 16;
+    float hypo_bin = 0.f;
     double ck_minutes = 30.0, ck_last;
     ckpt_t ck;
     uint64_t seed_used = 0;
@@ -404,7 +487,7 @@ int main(int argc, char** argv)
     memset(&ck, 0, sizeof ck);
     if (argc < 4) {
         fprintf(stderr, "usage: %s config_eqx.dat outfile picks [-n chains] [-d device] [-s seed] [-r ring slots] [-q] "
-                        "[-k checkpoint [-K minutes]] [-R checkpoint] [-D diagnostics] [-x]\n", argv[0]);
+                        "[-k checkpoint [-K minutes]] [-R checkpoint] [-D diagnostics] [-L locations] [-x]\n", argv[0]);
         return 2;
     }
     if ((env = getenv("MCMCEQ_CHAINS")) != NULL) { n_chains = atoi(env); n_given = 1; }
@@ -415,6 +498,7 @@ int main(int argc, char** argv)
         else if (!strcmp(argv[i], "-K") && i + 1 < argc) ck_minutes = atof(argv[++i]);
         else if (!strcmp(argv[i], "-R") && i + 1 < argc) resume_path = argv[++i];
         else if (!strcmp(argv[i], "-D") && i + 1 < argc) diag_path = argv[++i];
+        else if (!strcmp(argv[i], "-L") && i + 1 < argc) hypo_path = argv[++i];
         else if (!strcmp(argv[i], "-d") && i + 1 < argc) device = atoi(argv[++i]);
         else if (!strcmp(argv[i], "-s") && i + 1 < argc) seed_arg = atol(argv[++i]);
         else if (!strcmp(argv[i], "-r") && i + 1 < argc) ring = atoi(argv[++i]);
@@ -431,6 +515,8 @@ int main(int argc, char** argv)
         n_chains = ck.head.n_chains;
         if (diag_path && state_diag_params(ck.state, ck.head.state_bytes, &diag_burn_in, &diag_batches))
             FAIL("-D: the checkpoint %s holds no diagnostics (the run was started without -D)", resume_path);
+        if (hypo_path && state_hypo_params(ck.state, ck.head.state_bytes, &hypo_burn_in, &hypo_bin))
+            FAIL("-L: the checkpoint %s holds no hypocentre accumulators (the run was started without -L)", resume_path);
         {   /* the table mode is the checkpoint's; a state without tables (eikonal == 0, aflag == 1) has none */
             const uint32_t flags = ((const mq_state_header*)ck.state)->flags;
             if (reciprocal && (flags & MQ_STATE_TABLES) && !(flags & MQ_STATE_RECIPROCAL))
@@ -457,9 +543,16 @@ int main(int argc, char** argv)
         }
         if (ring > 0) MQ(mq_set_ring(h, ring));
         if (resume_path) MQ(mq_state_load(h, ck.state, ck.head.state_bytes));
-        else if (diag_path) {   /* the models of the start phase are burn-in */
-            diag_burn_in = cfg.j_max_start;
-            MQ(mq_diag_begin(h, diag_burn_in, diag_batches, NULL));
+        else {   /* the models of the start phase are burn-in */
+            if (diag_path) {
+                diag_burn_in = cfg.j_max_start;
+                MQ(mq_diag_begin(h, diag_burn_in, diag_batches, NULL));
+            }
+            if (hypo_path) {
+                hypo_burn_in = cfg.j_max_start;
+                hypo_bin = cfg.grid.h / 10.0f;
+                MQ(mq_hypo_begin(h, hypo_bin, hypo_burn_in, NULL));
+            }
         }
     }
 
@@ -568,6 +661,8 @@ main_loop:
                 if (ckpt_write(ck_path, h, &sink, seed_used, iters_done, lost)) FAIL("could not write the checkpoint %s", ck_path);
                 if (diag_path && diag_write(diag_path, h, cfg.grid.nz, pk.view.n_events, pk.view.n_stations, diag_burn_in, diag_batches, iters_done))
                     FAIL("could not write the diagnostics %s", diag_path);
+                if (hypo_path && hypo_write(hypo_path, h, pk.view.n_events, hypo_burn_in, hypo_bin, iters_done))
+                    FAIL("could not write the locations %s", hypo_path);
                 ck_last = now_s();
             }
         }
@@ -580,6 +675,8 @@ main_loop:
     for (c = 0; c < n_chains; c++) mqio_write_counts(sink.out[c], counts + 20 * c);
     if (diag_path && diag_write(diag_path, h, cfg.grid.nz, pk.view.n_events, pk.view.n_stations, diag_burn_in, diag_batches, iters_done))
         FAIL("could not write the diagnostics %s", diag_path);
+    if (hypo_path && hypo_write(hypo_path, h, pk.view.n_events, hypo_burn_in, hypo_bin, iters_done))
+        FAIL("could not write the locations %s", hypo_path);
 
 done:
     if (writer_on) {
